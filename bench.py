@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the LineRefineNet forward hot path (BASELINE.json metric: segments/s & points/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- encoder forward (shared MLP, fusion, gate,
 max+mean pooling -> global_feat) over 4096 segments x 4096 context points per GPU, synthetic
@@ -16,6 +16,9 @@ own shard, no data-path collective (segments are independent) -> weak scaling.
   roofline   : fusion GEMM kernel (72.7 % of the FLOPs): algorithmic FLOP per launch / mean launch
                duration from CUDA events recorded around each launch (lrn_profile_*), against the
                sustained bf16 peak of MEASURED_PEAKS.json; `chain_kernel` is the same for the fused conv1..conv5 kernel
+  --dump-outputs DIR : after the timed steps, DIR/global_feat.npy holds the global_feat (float32) of the last timed step
+               on rank 0: (B, 2048), or a fixed sample of its rows (numpy default_rng(0)) when that exceeds 64 MB.  The
+               inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
   cpu_baseline / --impl reference : the reference's OWN module (oracle/_ref/src/model.py, staged by oracle/make_ref.py
                from /root/reference in the build container; kind "reference") on the host cores, bounded sample;
                the op-for-op port oracle/torch_port.py (kind "port") only if the staged copy is absent.
@@ -51,6 +54,18 @@ FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustain
 # profiles/r02u_train_gemm_shapes.jsonl: seven of the nine layers are HBM-bound at this batch), the BatchNorm / gate passes
 # (10.3 ms) and the attention K / V / dK / dV traffic (3.0 ms) at the measured copy bandwidth, ~3 ms of query-side work.
 TRAIN_BOUND_MS = {"burst": 16.2, "sustained": 19.3, "dataflow": 34.0}
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_global_feat(out_dir: str, gf) -> None:
+    """Write gf (B, 2048) as out_dir/global_feat.npy; above DUMP_LIMIT_BYTES, a seeded sample of its rows in index order."""
+    import numpy as np
+    arr = gf.float().cpu().numpy()
+    if arr.nbytes > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 4096) // arr[0].nbytes         # room for the .npy header
+        arr = arr[np.sort(np.random.default_rng(0).choice(len(arr), keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "global_feat.npy"), arr)
 
 
 def load_peaks():
@@ -170,7 +185,12 @@ def main():
     ap.add_argument("--cpu-sample-segments", type=int, default=16)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip full_model / config5 / config3_sample / train_step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's global_feat to DIR/global_feat.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native arm")
 
     # stdout carries exactly ONE line, the result: anything libraries print to fd 1 meanwhile (NCCL's version banner,
     # warnings) goes to stderr
@@ -195,7 +215,7 @@ def main():
         if rank != 0:
             return
         seg = args.cpu_sample_segments
-        steps, warm = max(5, min(args.steps, 8)), max(1, min(args.warmup, 2))
+        steps, warm = args.steps, args.warmup
         v, dt, threads, kind = cpu_reference_run(seg, args.points, steps, warm)
         vf, dtf, _, _ = cpu_reference_run(max(1, seg // 2), args.points, 3, 1, full_forward=True)
         sample = f"{seg} segments x {args.points} points per step, {warm} warm-up + {steps} timed ({kind_text(kind)}, encoder, fp32)"
@@ -266,13 +286,16 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            step()
+            gf_last = step()
         e1.record()
         barrier()
         launches = _lib.launch_counter - launches0
         clocks = sampler.stop() if rank == 0 else None
         ms_per_step = max_over_ranks(e0.elapsed_time(e1)) / args.steps
         value = world * B / (ms_per_step * 1e-3)
+        if args.dump_outputs and rank == 0:
+            dump_global_feat(args.dump_outputs, gf_last)
+        del gf_last
 
         # ---- per-kernel timing for the roofline (same workload, events around every launch)
         prof_steps = min(args.steps, 3)
@@ -331,7 +354,7 @@ def main():
         for _ in range(2):
             e2e_step()
         barrier()
-        e2e_steps = max(3, min(args.steps, 5))
+        e2e_steps = args.steps
         t0 = time.perf_counter()
         for _ in range(e2e_steps):
             e2e_step()
