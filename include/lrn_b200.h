@@ -30,8 +30,9 @@
 extern "C" {
 #endif
 
-/* 2: lrn_train_attention_forward / _backward take `seed_state`; lrn_adam_step_capturable added */
-#define LRN_ABI_VERSION 2
+/* 2: lrn_train_attention_forward / _backward take `seed_state`; lrn_adam_step_capturable added
+ * 3: lrn_launch_count added */
+#define LRN_ABI_VERSION 3
 
 typedef struct CUstream_st* lrn_stream_t; /* == cudaStream_t */
 
@@ -96,6 +97,9 @@ const char* lrn_status_string(int status);
 const char* lrn_last_error(void);
 /* LRN_OK iff the current CUDA device can run this library (compute capability 10.0). */
 int lrn_device_check(void);
+/* Number of kernels this library has enqueued in this process (counted at enqueue: a CUDA-graph capture counts its
+ * kernels once, replays of the graph count nothing). */
+size_t lrn_launch_count(void);
 
 /* ---- weight folding (eval-mode BatchNorm folded into the preceding 1x1 conv) ----
  * Replaces: the bn_k(conv_k(x)) pairs of MultiScalePointNetEncoder.forward in eval mode,

@@ -14,6 +14,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <utility>
 #include <vector>
 
 #include "gemm_common.cuh"
@@ -44,6 +45,35 @@ int fail(int status, const char* fmt, ...) {
     cudaError_t e_ = (expr);                                                                    \
     if (e_ != cudaSuccess) return fail(LRN_ERR_CUDA, "%s -> %s", #expr, cudaGetErrorString(e_)); \
   } while (0)
+
+// Returns the status of a call of this library (helper, launch) from the enclosing function unless it is LRN_OK.
+#define LRN_TRY(expr)                       \
+  do {                                      \
+    if (const int st_ = (expr)) return st_; \
+  } while (0)
+
+// Declares `dev` (current device ordinal, SM count); off compute capability 10.0 the enclosing call returns
+// LRN_ERR_UNSUPPORTED_ARCH.
+#define LRN_DEVICE(dev) \
+  DeviceInfo dev;       \
+  LRN_TRY(device_info(&dev))
+
+// Every kernel of this library is enqueued by launch(); lrn_launch_count() reports how many.
+std::atomic<uint64_t> g_launches{0};
+
+template <typename... P, typename... A>
+int launch(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, A&&... args) {
+  kernel<<<grid, block, smem, s>>>(std::forward<A>(args)...);
+  LRN_CUDA(cudaGetLastError());
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  return LRN_OK;
+}
+
+// True when any of the pointers is not `align`-byte aligned (align is a power of two; NULL is aligned).
+template <typename... T>
+bool misaligned(uintptr_t align, T*... p) {
+  return ((reinterpret_cast<uintptr_t>(p) & (align - 1)) | ...) != 0;
+}
 
 constexpr int kCat = 2048;          // operand row: feat1..feat5 (1984) + gate hidden (64)
 constexpr int kFusionK = 1984;
@@ -112,42 +142,49 @@ int get_encode_fn(EncodeTiledFn* out) {
   return LRN_OK;
 }
 
+// Every tensor map of the library: `rank` dimensions (innermost first), byte strides of dimensions 1.., box in elements,
+// dense element strides, 128B swizzle, 256-byte L2 promotion, no out-of-bounds fill value (zeros).
+int encode_tmap(CUtensorMap* m, CUtensorMapDataType dtype, cuuint32_t rank, const void* base, const cuuint64_t* dims,
+                const cuuint64_t* strides, const cuuint32_t* box) {
+  EncodeTiledFn enc;
+  LRN_TRY(get_encode_fn(&enc));
+  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult r = enc(m, dtype, rank, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(LRN_ERR_CUDA, "cuTensorMapEncodeTiled%s failed (%d)", rank == 4 ? " (4-D)" : "", int(r));
+  return LRN_OK;
+}
+
 // K-major 2-D operand: `rows` x `cols` elements, row pitch `ld` elements; box = 128 bytes x box_rows, 128B swizzle.
 int make_tmap(CUtensorMap* m, int precision, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-  EncodeTiledFn enc;
-  int st = get_encode_fn(&enc);
-  if (st) return st;
   const size_t es = elem_size(precision);
-  if ((reinterpret_cast<uintptr_t>(base) & 15) || (ld * es) % 16) return fail(LRN_ERR_MISALIGNED, "tensor map base/pitch");
-  cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
-  cuuint64_t strides[1] = {cuuint64_t(ld * es)};
-  cuuint32_t box[2] = {cuuint32_t(128 / es), cuuint32_t(box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, precision != LRN_PREC_BF16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
-                   const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(LRN_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", int(r));
-  return LRN_OK;
+  if (misaligned(16, base) || (ld * es) % 16) return fail(LRN_ERR_MISALIGNED, "tensor map base/pitch");
+  const cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
+  const cuuint64_t strides[1] = {cuuint64_t(ld * es)};
+  const cuuint32_t box[2] = {cuuint32_t(128 / es), cuuint32_t(box_rows)};
+  return encode_tmap(m, precision != LRN_PREC_BF16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
+                     base, dims, strides, box);
 }
 
 // Tiled operand matrix (bf16): [row tile of 128][column block of 64][128 rows][128 bytes] - every [128 x 64] box that the
 // kernels move is one contiguous 16 KB block in global memory (a row-major matrix scatters it as 128 pieces of 128 bytes
 // at the row pitch, which caps the write bandwidth of the chain kernel at about half of a streaming copy).
 int make_tmap_tiled(CUtensorMap* m, const void* base, int64_t rows, int64_t cols) {
-  EncodeTiledFn enc;
-  int st = get_encode_fn(&enc);
-  if (st) return st;
-  if ((reinterpret_cast<uintptr_t>(base) & 1023) || cols % 64) return fail(LRN_ERR_MISALIGNED, "tiled tensor map base / columns");
+  if (misaligned(1024, base) || cols % 64) return fail(LRN_ERR_MISALIGNED, "tiled tensor map base / columns");
   const cuuint64_t nb = cuuint64_t(cols / 64), nt = cuuint64_t((rows + 127) / 128);
-  cuuint64_t dims[4] = {64, 128, nb, nt};
-  cuuint64_t strides[3] = {128, 16384, nb * 16384};
-  cuuint32_t box[4] = {64, 128, 1, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(LRN_ERR_CUDA, "cuTensorMapEncodeTiled (4-D) failed (%d)", int(r));
-  return LRN_OK;
+  const cuuint64_t dims[4] = {64, 128, nb, nt};
+  const cuuint64_t strides[3] = {128, 16384, nb * 16384};
+  const cuuint32_t box[4] = {64, 128, 1, 1};
+  return encode_tmap(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box);
+}
+
+// MN-major sibling of make_tmap: matrix stored (K rows, C cols) row-major, box = 64 cols x 64 rows
+int make_tmap_mn(CUtensorMap* m, const void* base, int64_t k_rows, int64_t cols, int64_t ld) {
+  if (misaligned(16, base) || (ld * 2) % 16) return fail(LRN_ERR_MISALIGNED, "tensor map base/pitch");
+  const cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(k_rows)};
+  const cuuint64_t strides[1] = {cuuint64_t(ld * 2)};
+  const cuuint32_t box[2] = {64, 64};
+  return encode_tmap(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box);
 }
 
 struct DeviceInfo {
@@ -197,14 +234,11 @@ int launch_pair_t(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMa
   using L = PairSmem<BN, STAGES, EPI == EPI_FUSION, STAGED>;
   auto kern = gemm_pair_kernel<BN, TF32, EPI, STAGES, GENERAL, STAGED, MN>;
   static std::atomic<uint64_t> configured{0};  // per instantiation
-  int st = configure_smem(kern, L::kDynamic, configured);
-  if (st) return st;
+  LRN_TRY(configure_smem(kern, L::kDynamic, configured));
   const int tiles = p.m_tiles * p.n_tiles * std::max(p.k_splits, 1);
   if (tiles <= 0) return LRN_OK;
   const int grid = 2 * std::min(tiles, sms / 2);  // one CTA pair (cluster of 2) per work-item slot
-  kern<<<grid, kPairThreads, L::kDynamic, stream>>>(ta, tb, tout, p);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(kern, grid, kPairThreads, L::kDynamic, stream, ta, tb, tout, p);
 }
 
 // How one GEMM is tiled over CTA pairs (cta_group::2, 256-row tiles).
@@ -252,14 +286,11 @@ int fold_one(int precision, const float* w, const float* b, const float* g, cons
   const long long total = static_cast<long long>(cout) * cin;
   const int grid = static_cast<int>(std::min<long long>((total + 255) / 256, 4096));
   if (precision != LRN_PREC_BF16)
-    fold_linear_kernel<float><<<grid, 256, 0, stream>>>(w, b, g, beta, mean, var, eps, cout, cin,
-                                                        static_cast<float*>(out_w), ld, col0, out_b, operand ? 1 : 0,
-                                                        precision == LRN_PREC_FP32X3 && operand ? lo_off : 0);
-  else
-    fold_linear_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(w, b, g, beta, mean, var, eps, cout, cin,
-                                                                static_cast<__nv_bfloat16*>(out_w), ld, col0, out_b, 0);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+    return launch(fold_linear_kernel<float>, grid, 256, 0, stream, w, b, g, beta, mean, var, eps, cout, cin,
+                  static_cast<float*>(out_w), ld, col0, out_b, operand ? 1 : 0,
+                  precision == LRN_PREC_FP32X3 && operand ? lo_off : 0);
+  return launch(fold_linear_kernel<__nv_bfloat16>, grid, 256, 0, stream, w, b, g, beta, mean, var, eps, cout, cin,
+                static_cast<__nv_bfloat16*>(out_w), ld, col0, out_b, 0, 0);
 }
 
 // ------------------------------------------------------------------ optional per-stage timing
@@ -339,6 +370,8 @@ const char* lrn_status_string(int status) {
 
 const char* lrn_last_error(void) { return g_err; }
 
+size_t lrn_launch_count(void) { return size_t(g_launches.load(std::memory_order_relaxed)); }
+
 int lrn_device_check(void) {
   DeviceInfo d;
   return device_info(&d);
@@ -352,12 +385,10 @@ size_t lrn_encoder_packed_bytes(int precision) {
 int lrn_encoder_fold(const lrn_encoder_params* pr, int precision, void* packed, size_t packed_bytes,
                      lrn_stream_t stream) {
   if (!pr || !packed || bad_precision(precision)) return fail(LRN_ERR_BAD_ARG, "null params/packed or bad precision");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const PackedLayout L = packed_layout(precision);
   if (packed_bytes < L.total) return fail(LRN_ERR_WORKSPACE, "packed buffer %zu < %zu", packed_bytes, L.total);
-  if (reinterpret_cast<uintptr_t>(packed) & 1023) return fail(LRN_ERR_MISALIGNED, "packed buffer must be 1024-byte aligned");
+  if (misaligned(1024, packed)) return fail(LRN_ERR_MISALIGNED, "packed buffer must be 1024-byte aligned");
   for (int k = 0; k < 5; ++k)
     if (!pr->conv_w[k] || !pr->conv_b[k] || !pr->bn_w[k] || !pr->bn_b[k] || !pr->bn_mean[k] || !pr->bn_var[k])
       return fail(LRN_ERR_BAD_ARG, "null conv/bn parameter %d", k + 1);
@@ -365,32 +396,24 @@ int lrn_encoder_fold(const lrn_encoder_params* pr, int precision, void* packed, 
       !pr->fusion_bn_var || !pr->gate0_w || !pr->gate0_b || !pr->gate2_w || !pr->gate2_b)
     return fail(LRN_ERR_BAD_ARG, "null fusion/gate parameter");
   uint8_t* base = static_cast<uint8_t*>(packed);
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const int wm = op_mul(precision);
   // conv1 stays fp32 (FMA kernel); gate layer 1 is copied as is
-  st = fold_one(LRN_PREC_TF32, pr->conv_w[0], pr->conv_b[0], pr->bn_w[0], pr->bn_b[0], pr->bn_mean[0], pr->bn_var[0],
-                pr->bn_eps, 64, 4, base + L.w1, 4, 0, reinterpret_cast<float*>(base + L.b1), s, /*operand=*/false);
-  if (st) return st;
-  LRN_CUDA(cudaMemcpyAsync(base + L.wg1, pr->gate0_w, 64 * 4, cudaMemcpyDeviceToDevice, s));
-  LRN_CUDA(cudaMemcpyAsync(base + L.bg1, pr->gate0_b, 64 * 4, cudaMemcpyDeviceToDevice, s));
-  for (int k = 2; k <= 5; ++k) {
-    st = fold_one(precision, pr->conv_w[k - 1], pr->conv_b[k - 1], pr->bn_w[k - 1], pr->bn_b[k - 1], pr->bn_mean[k - 1],
-                  pr->bn_var[k - 1], pr->bn_eps, kChan[k], kChan[k - 1], base + L.w[k], kChan[k - 1] * wm, 0,
-                  reinterpret_cast<float*>(base + L.b[k]), s, true, kChan[k - 1]);
-    if (st) return st;
-  }
-  st = fold_one(precision, pr->fusion_w, pr->fusion_b, pr->fusion_bn_w, pr->fusion_bn_b, pr->fusion_bn_mean,
-                pr->fusion_bn_var, pr->bn_eps, 1024, kFusionK, base + L.wfg, kCat * wm, 0,
-                reinterpret_cast<float*>(base + L.bf), s, true, kCat);
-  if (st) return st;
-  st = fold_one(precision, pr->gate2_w, pr->gate2_b, nullptr, nullptr, nullptr, nullptr, 0.f, 1024, kGateK,
-                base + L.wfg, kCat * wm, kFusionK, reinterpret_cast<float*>(base + L.bg), s, true, kCat);
-  if (st) return st;
-  if (pr->proj_w && pr->proj_b) {
-    st = fold_one(precision, pr->proj_w, pr->proj_b, nullptr, nullptr, nullptr, nullptr, 0.f, 256, 1024, base + L.wp,
-                  1024 * wm, 0, reinterpret_cast<float*>(base + L.bp), s, true, 1024);
-    if (st) return st;
-  }
+  LRN_TRY(fold_one(LRN_PREC_TF32, pr->conv_w[0], pr->conv_b[0], pr->bn_w[0], pr->bn_b[0], pr->bn_mean[0], pr->bn_var[0],
+                   pr->bn_eps, 64, 4, base + L.w1, 4, 0, reinterpret_cast<float*>(base + L.b1), stream, /*operand=*/false));
+  LRN_CUDA(cudaMemcpyAsync(base + L.wg1, pr->gate0_w, 64 * 4, cudaMemcpyDeviceToDevice, stream));
+  LRN_CUDA(cudaMemcpyAsync(base + L.bg1, pr->gate0_b, 64 * 4, cudaMemcpyDeviceToDevice, stream));
+  for (int k = 2; k <= 5; ++k)
+    LRN_TRY(fold_one(precision, pr->conv_w[k - 1], pr->conv_b[k - 1], pr->bn_w[k - 1], pr->bn_b[k - 1], pr->bn_mean[k - 1],
+                     pr->bn_var[k - 1], pr->bn_eps, kChan[k], kChan[k - 1], base + L.w[k], kChan[k - 1] * wm, 0,
+                     reinterpret_cast<float*>(base + L.b[k]), stream, true, kChan[k - 1]));
+  LRN_TRY(fold_one(precision, pr->fusion_w, pr->fusion_b, pr->fusion_bn_w, pr->fusion_bn_b, pr->fusion_bn_mean,
+                   pr->fusion_bn_var, pr->bn_eps, 1024, kFusionK, base + L.wfg, kCat * wm, 0,
+                   reinterpret_cast<float*>(base + L.bf), stream, true, kCat));
+  LRN_TRY(fold_one(precision, pr->gate2_w, pr->gate2_b, nullptr, nullptr, nullptr, nullptr, 0.f, 1024, kGateK,
+                   base + L.wfg, kCat * wm, kFusionK, reinterpret_cast<float*>(base + L.bg), stream, true, kCat));
+  if (pr->proj_w && pr->proj_b)
+    LRN_TRY(fold_one(precision, pr->proj_w, pr->proj_b, nullptr, nullptr, nullptr, nullptr, 0.f, 256, 1024, base + L.wp,
+                     1024 * wm, 0, reinterpret_cast<float*>(base + L.bp), stream, true, 1024));
   return LRN_OK;
 }
 
@@ -414,13 +437,9 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
   if ((flags & LRN_OUT_ARGMAX) && !argmax) return fail(LRN_ERR_BAD_ARG, "argmax is null");
   if ((flags & LRN_OUT_FUSED) && !fused) return fail(LRN_ERR_BAD_ARG, "fused is null");
   if ((flags & LRN_OUT_MEMORY) && !memory) return fail(LRN_ERR_BAD_ARG, "memory is null");
-  if ((reinterpret_cast<uintptr_t>(context) & 15) || (reinterpret_cast<uintptr_t>(workspace) & 1023) ||
-      (reinterpret_cast<uintptr_t>(packed) & 1023) || (reinterpret_cast<uintptr_t>(memory) & 15) ||
-      (reinterpret_cast<uintptr_t>(global_feat) & 15))
+  if (misaligned(16, context, memory, global_feat) || misaligned(1024, workspace, packed))
     return fail(LRN_ERR_MISALIGNED, "context/memory/global_feat need 16-byte, packed/workspace 1024-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
 
   const bool tf32 = precision != LRN_PREC_BF16;      // fp32 operands on the kind::tf32 tensor-core path
   const bool x3 = precision == LRN_PREC_FP32X3;      // ... as hi / lo halves, three passes per k-block (fp32-class products)
@@ -430,7 +449,6 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
   const PackedLayout L = packed_layout(precision);
   const WorkspaceLayout W = workspace_layout(B, N, precision, flags, chunk_rows);
   if (workspace_bytes < W.total) return fail(LRN_ERR_WORKSPACE, "workspace %zu < %zu", workspace_bytes, W.total);
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const uint8_t* pk = static_cast<const uint8_t*>(packed);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   void* cat = ws + W.cat;
@@ -438,33 +456,27 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + W.keys);
   const int64_t P = B * N;
 
-  if (flags & (LRN_OUT_POOL | LRN_OUT_ARGMAX)) LRN_CUDA(cudaMemsetAsync(global_feat, 0, size_t(B) * 2048 * 4, s));
-  if (flags & LRN_OUT_ARGMAX) LRN_CUDA(cudaMemsetAsync(keys, 0, size_t(B) * 1024 * 8, s));
+  if (flags & (LRN_OUT_POOL | LRN_OUT_ARGMAX)) LRN_CUDA(cudaMemsetAsync(global_feat, 0, size_t(B) * 2048 * 4, stream));
+  if (flags & LRN_OUT_ARGMAX) LRN_CUDA(cudaMemsetAsync(keys, 0, size_t(B) * 1024 * 8, stream));
 
   // weight tensor maps (B operands)
   CUtensorMap tw[6], twfg, twp;
   GemmPlan plan[6];
   for (int k = 2; k <= 5; ++k) {
     plan[k] = plan_gemm(kChan[k], EPI_ACT);
-    st = make_tmap(&tw[k], precision, pk + L.w[k], kChan[k], kChan[k - 1] * wm, kChan[k - 1] * wm, plan[k].b_box_rows);
-    if (st) return st;
+    LRN_TRY(make_tmap(&tw[k], precision, pk + L.w[k], kChan[k], kChan[k - 1] * wm, kChan[k - 1] * wm, plan[k].b_box_rows));
   }
   const GemmPlan plan_f = plan_gemm(1024, EPI_FUSION), plan_p = plan_gemm(256, EPI_ACT);
   CUtensorMap tw_chain[4];
   if (!tf32) {
     for (int k = 2; k <= 5; ++k) {
       // TMA box = the weight rows ONE CTA of the pair stages per k-block: N / 2 (conv2 and conv5 run as N = 128 MMAs)
-      st = make_tmap(&tw_chain[k - 2], precision, pk + L.w[k], kChan[k], kChan[k - 1], kChan[k - 1],
-                     (k == 2 || k == 5) ? 64 : 128);
-      if (st) return st;
+      LRN_TRY(make_tmap(&tw_chain[k - 2], precision, pk + L.w[k], kChan[k], kChan[k - 1], kChan[k - 1],
+                        (k == 2 || k == 5) ? 64 : 128));
     }
   }
-  st = make_tmap(&twfg, precision, pk + L.wfg, 1024, kCat * wm, kCat * wm, plan_f.b_box_rows);
-  if (st) return st;
-  if (flags & LRN_OUT_MEMORY) {
-    st = make_tmap(&twp, precision, pk + L.wp, 256, 1024 * wm, 1024 * wm, plan_p.b_box_rows);
-    if (st) return st;
-  }
+  LRN_TRY(make_tmap(&twfg, precision, pk + L.wfg, 1024, kCat * wm, kCat * wm, plan_f.b_box_rows));
+  if (flags & LRN_OUT_MEMORY) LRN_TRY(make_tmap(&twp, precision, pk + L.wp, 256, 1024 * wm, 1024 * wm, plan_p.b_box_rows));
 
   EmbedWeights ew{reinterpret_cast<const float*>(pk + L.w1), reinterpret_cast<const float*>(pk + L.b1),
                   reinterpret_cast<const float*>(pk + L.wg1), reinterpret_cast<const float*>(pk + L.bg1)};
@@ -473,20 +485,16 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
     const int64_t rows = std::min<int64_t>(W.chunk, P - r0);
     auto m_tiles_of = [&](const GemmPlan& g) { return int((rows + g.m_rows - 1) / g.m_rows); };
     CUtensorMap ta, tpm;
-    st = make_tmap(&ta, precision, cat, rows, kCat * wm, kCat * wm, BM);
-    if (st) return st;
+    LRN_TRY(make_tmap(&ta, precision, cat, rows, kCat * wm, kCat * wm, BM));
 
     // bf16 tier: conv1..conv5 + gate layer 1 as ONE fused kernel (activations stay on the SM, the operand matrix is kept
     // in the tiled layout); the tf32 tier runs one kernel per layer on row-major operand rows.
     const bool fused_chain = !tf32;
     const bool tiled = fused_chain;
-    if (tiled) {
-      st = make_tmap_tiled(&ta, cat, rows, kCat);
-      if (st) return st;
-    }
+    if (tiled) LRN_TRY(make_tmap_tiled(&ta, cat, rows, kCat));
     if (fused_chain) {
       static std::atomic<uint64_t> configured{0};
-      if ((st = configure_smem(chain_pair_kernel, ChainSmem::kDynamic, configured))) return st;
+      LRN_TRY(configure_smem(chain_pair_kernel, ChainSmem::kDynamic, configured));
       ChainParams cp{};
       cp.M = int(rows);
       cp.num_tiles = int((rows + 2 * BM - 1) / (2 * BM));
@@ -501,22 +509,23 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
       static const int dbg_layer = [] { const char* e = getenv("LRN_DBG_LAYER"); return e ? atoi(e) : 0; }();
       cp.dbg = dbg_layer == 4 ? g_dbg : nullptr;
 #endif
-      StageTimer timer(LRN_STAGE_CONV5, s);  // reported as stage "conv5"; the other chain stages then read 0
+      StageTimer timer(LRN_STAGE_CONV5, stream);  // reported as stage "conv5"; the other chain stages then read 0
       const int grid = 2 * std::min(cp.num_tiles, dev.sms / 2);
 #ifdef LRN_TIMELINE   // tools/l2_ring_probe.py: fusion kernel alone on whatever the operand buffer holds
       const char* skip_chain = getenv("LRN_DBG_SKIP_CHAIN");
       if (!(skip_chain && atoi(skip_chain)))
 #endif
-      chain_pair_kernel<<<grid, kPairThreads, ChainSmem::kDynamic, s>>>(tw_chain[0], tw_chain[1], tw_chain[2], tw_chain[3], ta, cp);
-      LRN_CUDA(cudaGetLastError());
+      LRN_TRY(launch(chain_pair_kernel, grid, kPairThreads, ChainSmem::kDynamic, stream, tw_chain[0], tw_chain[1], tw_chain[2],
+                     tw_chain[3], ta, cp));
     } else {  // layer 1 (+ gate layer 1): raw points -> operand columns
-      StageTimer timer(LRN_STAGE_EMBED, s);
+      StageTimer timer(LRN_STAGE_EMBED, stream);
       const int grid = int(std::min<int64_t>((rows + 15) / 16, int64_t(dev.sms) * 16));
       if (tf32)
-        point_embed_kernel<true><<<grid, 256, 0, s>>>(reinterpret_cast<const float4*>(context) + r0, rows, ew, cat, kCat * wm, x3 ? kCat : 0);
+        LRN_TRY(launch(point_embed_kernel<true>, grid, 256, 0, stream, reinterpret_cast<const float4*>(context) + r0, rows, ew, cat,
+                       kCat * wm, x3 ? kCat : 0));
       else
-        point_embed_kernel<false><<<grid, 256, 0, s>>>(reinterpret_cast<const float4*>(context) + r0, rows, ew, cat, kCat);
-      LRN_CUDA(cudaGetLastError());
+        LRN_TRY(launch(point_embed_kernel<false>, grid, 256, 0, stream, reinterpret_cast<const float4*>(context) + r0, rows, ew,
+                       cat, kCat, 0));
     }
     for (int k = fused_chain ? 6 : 2; k <= 5; ++k) {  // tf32 tier: conv2..conv5, each writes its own column block of the operand row
       GemmParams p{};
@@ -541,9 +550,8 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
       static const int dbg_layer = [] { const char* e = getenv("LRN_DBG_LAYER"); return e ? atoi(e) : 0; }();
       p.dbg = (k == dbg_layer) ? g_dbg : nullptr;
 #endif
-      StageTimer timer(LRN_STAGE_CONV2 + (k - 2), s);
-      st = launch_gemm(precision, plan[k], EPI_ACT, ta, tw[k], p, dev.sms, s, &ta);
-      if (st) return st;
+      StageTimer timer(LRN_STAGE_CONV2 + (k - 2), stream);
+      LRN_TRY(launch_gemm(precision, plan[k], EPI_ACT, ta, tw[k], p, dev.sms, stream, &ta));
     }
     {  // fusion + gate + pooling
       GemmParams p{};
@@ -573,13 +581,11 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
       p.dbg = getenv("LRN_DBG_LAYER") ? nullptr : g_dbg;
       if (const char* ring = getenv("LRN_DBG_RING")) p.a_ring = atoi(ring);
 #endif
-      StageTimer timer(LRN_STAGE_FUSION, s);
-      st = launch_gemm(precision, plan_f, EPI_FUSION, ta, twfg, p, dev.sms, s);
-      if (st) return st;
+      StageTimer timer(LRN_STAGE_FUSION, stream);
+      LRN_TRY(launch_gemm(precision, plan_f, EPI_FUSION, ta, twfg, p, dev.sms, stream));
     }
     if (flags & LRN_OUT_MEMORY) {  // memory = fused * Wp^T + bp
-      st = make_tmap(&tpm, precision, fused_pm, rows, 1024 * wm, 1024 * wm, BM);
-      if (st) return st;
+      LRN_TRY(make_tmap(&tpm, precision, fused_pm, rows, 1024 * wm, 1024 * wm, BM));
       GemmParams p{};
       p.M = int(rows);
       p.m_tiles = m_tiles_of(plan_p);
@@ -597,40 +603,20 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
         p.out = reinterpret_cast<uint16_t*>(memory) + r0 * 512;
         p.ldo = 512;
         p.out_f32 = 0;
-        st = make_tmap(&tmem_out, precision, p.out, rows, 256, 512, BM);
-        if (st) return st;
+        LRN_TRY(make_tmap(&tmem_out, precision, p.out, rows, 256, 512, BM));
       } else {
         p.out = reinterpret_cast<float*>(memory) + r0 * 256;
         p.ldo = 256;
         p.out_f32 = 1;
       }
-      StageTimer timer(LRN_STAGE_PROJ, s);
-      st = launch_gemm(precision, plan_p, EPI_ACT, tpm, twp, p, dev.sms, s, mem_bf16 ? &tmem_out : nullptr);
-      if (st) return st;
+      StageTimer timer(LRN_STAGE_PROJ, stream);
+      LRN_TRY(launch_gemm(precision, plan_p, EPI_ACT, tpm, twp, p, dev.sms, stream, mem_bf16 ? &tmem_out : nullptr));
     }
   }
   if (flags & LRN_OUT_ARGMAX) {
     const int grid = int(std::min<int64_t>((B * 1024 + 255) / 256, 2048));
-    argmax_finalize_kernel<<<grid, 256, 0, s>>>(keys, B, global_feat, reinterpret_cast<long long*>(argmax));
-    LRN_CUDA(cudaGetLastError());
+    LRN_TRY(launch(argmax_finalize_kernel, grid, 256, 0, stream, keys, B, global_feat, reinterpret_cast<long long*>(argmax)));
   }
-  return LRN_OK;
-}
-
-// K-major tensor map helper's MN-major sibling: matrix stored (K rows, C cols) row-major, box = 64 cols x 64 rows
-static int make_tmap_mn(CUtensorMap* m, const void* base, int64_t k_rows, int64_t cols, int64_t ld) {
-  EncodeTiledFn enc;
-  int st = get_encode_fn(&enc);
-  if (st) return st;
-  if ((reinterpret_cast<uintptr_t>(base) & 15) || (ld * 2) % 16) return fail(LRN_ERR_MISALIGNED, "tensor map base/pitch");
-  cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(k_rows)};
-  cuuint64_t strides[1] = {cuuint64_t(ld * 2)};
-  cuuint32_t box[2] = {64, 64};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(LRN_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", int(r));
   return LRN_OK;
 }
 
@@ -638,13 +624,11 @@ int lrn_gemm_tn(const void* At, int64_t lda, const void* Bt, int64_t ldb, float*
                 int64_t K, lrn_stream_t stream) {
   if (!At || !Bt || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (M <= 0 || N <= 0 || K <= 0 || N % 128 || M % 64) return fail(LRN_ERR_BAD_SHAPE, "M=%lld N=%lld K=%lld", (long long)M, (long long)N, (long long)K);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const int bn = (N % 256 == 0) ? 256 : 128;
   CUtensorMap ta, tb;
-  if ((st = make_tmap_mn(&ta, At, K, M, lda))) return st;
-  if ((st = make_tmap_mn(&tb, Bt, K, N, ldb))) return st;
+  LRN_TRY(make_tmap_mn(&ta, At, K, M, lda));
+  LRN_TRY(make_tmap_mn(&tb, Bt, K, N, ldb));
   GemmParams p{};
   p.M = int(M);
   p.m_tiles = int((M + 2 * BM - 1) / (2 * BM));
@@ -672,12 +656,11 @@ int lrn_gemm_tn(const void* At, int64_t lda, const void* Bt, int64_t ldb, float*
     if (want > 1) {
       p.kb_per_split = (p.kb_main + want - 1) / want;
       p.k_splits = (p.kb_main + p.kb_per_split - 1) / p.kb_per_split;
-      LRN_CUDA(cudaMemset2DAsync(out, size_t(ldo) * 4, 0, size_t(N) * 4, size_t(M), reinterpret_cast<cudaStream_t>(stream)));
+      LRN_CUDA(cudaMemset2DAsync(out, size_t(ldo) * 4, 0, size_t(N) * 4, size_t(M), stream));
     }
   }
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  return bn == 256 ? launch_pair_t<256, false, EPI_ACT, 6, true, false, true>(ta, tb, ta, p, dev.sms, s)
-                   : launch_pair_t<128, false, EPI_ACT, 8, true, false, true>(ta, tb, ta, p, dev.sms, s);
+  return bn == 256 ? launch_pair_t<256, false, EPI_ACT, 6, true, false, true>(ta, tb, ta, p, dev.sms, stream)
+                   : launch_pair_t<128, false, EPI_ACT, 8, true, false, true>(ta, tb, ta, p, dev.sms, stream);
 }
 
 int lrn_ctx_attention_splits(int B, int N) {
@@ -699,13 +682,11 @@ int lrn_ctx_attention(const void* qfold, const void* kp, int64_t ld_kp, const vo
   if (splits < 1 || splits > total) return fail(LRN_ERR_BAD_ARG, "splits=%d (1..%d)", splits, total);
   const int per = (total + splits - 1) / splits;
   if ((splits - 1) * per >= total) return fail(LRN_ERR_BAD_ARG, "splits=%d leaves an empty split (use lrn_ctx_attention_splits)", splits);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   CUtensorMap tq, tk, tv;
-  if ((st = make_tmap(&tq, LRN_PREC_BF16, qfold, int64_t(B) * 256, 256, 256, 128))) return st;
-  if ((st = make_tmap(&tk, LRN_PREC_BF16, kp, int64_t(B) * N, 256, ld_kp, 64))) return st;
-  if ((st = make_tmap_mn(&tv, mem, int64_t(B) * N, 256, ld_mem))) return st;
+  LRN_TRY(make_tmap(&tq, LRN_PREC_BF16, qfold, int64_t(B) * 256, 256, 256, 128));
+  LRN_TRY(make_tmap(&tk, LRN_PREC_BF16, kp, int64_t(B) * N, 256, ld_kp, 64));
+  LRN_TRY(make_tmap_mn(&tv, mem, int64_t(B) * N, 256, ld_mem));
   AttnParams p{};
   p.items = B * splits;
   p.N = N;
@@ -715,47 +696,35 @@ int lrn_ctx_attention(const void* qfold, const void* kp, int64_t ld_kp, const vo
   p.out_bf16 = out_bf16 ? 1 : 0;
   p.lse = lse;
   static std::atomic<uint64_t> configured{0};
-  if ((st = configure_smem(ctx_attn_kernel, int(AttnSmem::kDynamic), configured))) return st;
+  LRN_TRY(configure_smem(ctx_attn_kernel, int(AttnSmem::kDynamic), configured));
   const int clusters = std::min(B * splits, dev.sms / 2);  // persistent: one cluster per SM pair walks the items
-  ctx_attn_kernel<<<2 * clusters, kAttnThreads, AttnSmem::kDynamic, reinterpret_cast<cudaStream_t>(stream)>>>(tq, tk, tv, p);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(ctx_attn_kernel, 2 * clusters, kAttnThreads, AttnSmem::kDynamic, stream, tq, tk, tv, p);
 }
 
 int lrn_pos_hidden(const float* w1, const float* b1, const float* context, int64_t P, void* out, int64_t ld_out,
                    lrn_stream_t stream) {
   if (!w1 || !b1 || !context || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (P <= 0) return fail(LRN_ERR_BAD_SHAPE, "P=%lld", (long long)P);
-  if ((reinterpret_cast<uintptr_t>(context) & 15) || (reinterpret_cast<uintptr_t>(out) & 15) || ld_out < 256 || (ld_out * 2) % 16)
+  if (misaligned(16, context, out) || ld_out < 256 || (ld_out * 2) % 16)
     return fail(LRN_ERR_MISALIGNED, "context / out need 16-byte alignment, ld_out >= 256 and a multiple of 8");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const int grid = int(std::min<int64_t>((P + 7) / 8, int64_t(dev.sms) * 8));
-  pos_hidden_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float4*>(context), P, w1, b1,
-                                                                              reinterpret_cast<uint16_t*>(out), ld_out);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(pos_hidden_kernel, grid, 256, 0, stream, reinterpret_cast<const float4*>(context), P, w1, b1,
+                reinterpret_cast<uint16_t*>(out), ld_out);
 }
 
 int lrn_pos_hidden_backward(const float* context, int64_t P, const void* hidden, int64_t ld_hidden, const void* d_hidden,
                             int64_t ld_d, float* d_w1, float* d_b1, lrn_stream_t stream) {
   if (!context || !hidden || !d_hidden || !d_w1 || !d_b1) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (P <= 0) return fail(LRN_ERR_BAD_SHAPE, "P=%lld", (long long)P);
-  if ((reinterpret_cast<uintptr_t>(context) | reinterpret_cast<uintptr_t>(hidden) | reinterpret_cast<uintptr_t>(d_hidden)) & 15 ||
-      ld_hidden % 8 || ld_d % 8 || ld_hidden < 256 || ld_d < 256)
+  if (misaligned(16, context, hidden, d_hidden) || ld_hidden % 8 || ld_d % 8 || ld_hidden < 256 || ld_d < 256)
     return fail(LRN_ERR_MISALIGNED, "16-byte alignment, row pitches >= 256 and multiples of 8");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  LRN_CUDA(cudaMemsetAsync(d_w1, 0, 256 * 3 * 4, s));
-  LRN_CUDA(cudaMemsetAsync(d_b1, 0, 256 * 4, s));
+  LRN_DEVICE(dev);
+  LRN_CUDA(cudaMemsetAsync(d_w1, 0, 256 * 3 * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(d_b1, 0, 256 * 4, stream));
   const int grid = int(std::min<int64_t>((P + 7) / 8, int64_t(dev.sms) * 4));
-  pos_hidden_bwd_kernel<<<grid, 256, 0, s>>>(reinterpret_cast<const float4*>(context), P, reinterpret_cast<const uint16_t*>(hidden),
-                                             ld_hidden, reinterpret_cast<const uint16_t*>(d_hidden), ld_d, d_w1, d_b1);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(pos_hidden_bwd_kernel, grid, 256, 0, stream, reinterpret_cast<const float4*>(context), P,
+                reinterpret_cast<const uint16_t*>(hidden), ld_hidden, reinterpret_cast<const uint16_t*>(d_hidden), ld_d, d_w1, d_b1);
 }
 
 // ---------------------------------------------------------------- scene preprocessing (section 8f row 3)
@@ -791,13 +760,9 @@ int lrn_scene_resample(const double* vertices, const int64_t* offsets, int L, in
   if (!vertices || !offsets || !line32 || !dense200 || !centers || !noisy_centered) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (L <= 0 || max_vertices < 0 || max_vertices > scene::kMaxVertices)
     return fail(LRN_ERR_BAD_SHAPE, "L=%d, longest polyline %d vertices (limit %d)", L, max_vertices, scene::kMaxVertices);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  scene::resample_kernel<<<L, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(vertices, reinterpret_cast<const long long*>(offsets), L,
-                                                                                line32, dense200, centers, noisy_centered);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  LRN_DEVICE(dev);
+  return launch(scene::resample_kernel, L, 256, 0, stream, vertices, reinterpret_cast<const long long*>(offsets), L, line32,
+                dense200, centers, noisy_centered);
 }
 
 size_t lrn_scene_workspace_bytes(int L, int64_t capacity) {
@@ -816,15 +781,11 @@ int lrn_scene_segments(const float* scene_pts, int64_t S, const float* scene_sor
   if (!(crop_radius > 0) || !(decay_scale > 0) || !(coord_extent >= 0) || (crop_radius + 2.0) / decay_scale > 25.0)
     return fail(LRN_ERR_BAD_ARG, "crop_radius=%g decay_scale=%g: (radius + 2) / decay must stay <= 25 (weights must not underflow)",
                 crop_radius, decay_scale);
-  if ((reinterpret_cast<uintptr_t>(scene_pts) & 15) || (reinterpret_cast<uintptr_t>(context) & 15) ||
-      (reinterpret_cast<uintptr_t>(workspace) & 255))
+  if (misaligned(16, scene_pts, context) || misaligned(256, workspace))
     return fail(LRN_ERR_MISALIGNED, "scene / context need 16-byte, workspace 256-byte alignment");
   const SceneLayout w = scene_layout(L, capacity);
   if (workspace_bytes < w.total) return fail(LRN_ERR_WORKSPACE, "workspace %zu < %zu bytes", workspace_bytes, w.total);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  LRN_DEVICE(dev);
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   float* aabb = reinterpret_cast<float*>(ws + w.aabb);
   float* dense_f = reinterpret_cast<float*>(ws + w.dense_f);
@@ -842,29 +803,24 @@ int lrn_scene_segments(const float* scene_pts, int64_t S, const float* scene_sor
   const float r2_lo = float(rlo * rlo * (1.0 - 1e-6)), r2_hi = float(rhi * rhi * (1.0 + 1e-6));
   const float4* pts = reinterpret_cast<const float4*>(scene_pts);
   if ((scene_sorted != nullptr) != (perm != nullptr)) return fail(LRN_ERR_BAD_ARG, "scene_sorted and perm come together");
-  if (reinterpret_cast<uintptr_t>(scene_sorted) & 15) return fail(LRN_ERR_MISALIGNED, "scene_sorted needs 16-byte alignment");
+  if (misaligned(16, scene_sorted)) return fail(LRN_ERR_MISALIGNED, "scene_sorted needs 16-byte alignment");
   const float4* crop_pts = scene_sorted ? reinterpret_cast<const float4*>(scene_sorted) : pts;
-  scene::prep_kernel<<<L, 128, 0, s>>>(dense200, L, float(rhi * (1.0 + 1e-6)), aabb, dense_f, count, fill, imin, imax);
-  LRN_CUDA(cudaGetLastError());
+  LRN_TRY(launch(scene::prep_kernel, L, 128, 0, stream, dense200, L, float(rhi * (1.0 + 1e-6)), aabb, dense_f, count, fill, imin,
+                 imax));
   const int grid = int((S + 255) / 256);
-  scene::tube_crop_kernel<false><<<grid, 256, 0, s>>>(crop_pts, S, L, aabb, dense_f, dense200, crop_radius, r2_lo, r2_hi, count, imin,
-                                                      imax, fill, offset, capacity, perm, cand);
-  LRN_CUDA(cudaGetLastError());
-  scene::scan_kernel<<<1, 1024, 0, s>>>(count, L, capacity, offset, stat);
-  LRN_CUDA(cudaGetLastError());
-  scene::tube_crop_kernel<true><<<grid, 256, 0, s>>>(crop_pts, S, L, aabb, dense_f, dense200, crop_radius, r2_lo, r2_hi, count, imin,
-                                                     imax, fill, offset, capacity, perm, cand);
-  LRN_CUDA(cudaGetLastError());
-  scene::sample_keys_kernel<<<dim3(32, L), 256, 0, s>>>(pts, line32, count, offset, imin, imax, N, decay_scale, seed, stat, cand, keys);
-  LRN_CUDA(cudaGetLastError());
+  LRN_TRY(launch(scene::tube_crop_kernel<false>, grid, 256, 0, stream, crop_pts, S, L, aabb, dense_f, dense200, crop_radius, r2_lo,
+                 r2_hi, count, imin, imax, fill, offset, capacity, perm, cand));
+  LRN_TRY(launch(scene::scan_kernel, 1, 1024, 0, stream, count, L, capacity, offset, stat));
+  LRN_TRY(launch(scene::tube_crop_kernel<true>, grid, 256, 0, stream, crop_pts, S, L, aabb, dense_f, dense200, crop_radius, r2_lo,
+                 r2_hi, count, imin, imax, fill, offset, capacity, perm, cand));
+  LRN_TRY(launch(scene::sample_keys_kernel, dim3(32, L), 256, 0, stream, pts, line32, count, offset, imin, imax, N, decay_scale,
+                 seed, stat, cand, keys));
   const int cap = scene_cap(N);
   const size_t smem = size_t(cap) * 12;
   // the opt-in above 48 KB is per device and the size depends on N: set it on every call (a host-side attribute write)
   LRN_CUDA(cudaFuncSetAttribute(scene::select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  scene::select_kernel<<<L, 256, smem, s>>>(pts, centers, count, offset, N, cap, seed, stat, cand, keys, context,
-                                            reinterpret_cast<long long*>(indices), counts);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(scene::select_kernel, L, 256, smem, stream, pts, centers, count, offset, N, cap, seed, stat, cand, keys, context,
+                reinterpret_cast<long long*>(indices), counts);
 }
 
 int lrn_debug_timeline(long long* device_buffer) {
@@ -905,37 +861,27 @@ int lrn_point_embed(const void* packed, int precision, const float* context, int
   if ((precision != LRN_PREC_BF16 && precision != LRN_PREC_TF32) || !packed || !context || !operand_rows || rows <= 0)
     return fail(LRN_ERR_BAD_ARG, "bad argument");
   if (tiled && precision != LRN_PREC_BF16) return fail(LRN_ERR_BAD_ARG, "the tiled operand layout is the bf16 tier's");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const PackedLayout L = packed_layout(precision);
   const uint8_t* pk = static_cast<const uint8_t*>(packed);
   EmbedWeights ew{reinterpret_cast<const float*>(pk + L.w1), reinterpret_cast<const float*>(pk + L.b1),
                   reinterpret_cast<const float*>(pk + L.wg1), reinterpret_cast<const float*>(pk + L.bg1)};
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const int grid = int(std::min<int64_t>((rows + 15) / 16, int64_t(dev.sms) * 16));
   if (precision == LRN_PREC_TF32)
-    point_embed_kernel<true><<<grid, 256, 0, s>>>(reinterpret_cast<const float4*>(context), rows, ew, operand_rows, kCat);
-  else
-    point_embed_kernel<false><<<grid, 256, 0, s>>>(reinterpret_cast<const float4*>(context), rows, ew, operand_rows, tiled ? 0 : kCat);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+    return launch(point_embed_kernel<true>, grid, 256, 0, stream, reinterpret_cast<const float4*>(context), rows, ew, operand_rows,
+                  kCat, 0);
+  return launch(point_embed_kernel<false>, grid, 256, 0, stream, reinterpret_cast<const float4*>(context), rows, ew, operand_rows,
+                tiled ? 0 : kCat, 0);
 }
 
 int lrn_head_forward(const float* w1, const float* b1, const float* w2, const float* b2, const float* tgt,
                      int64_t rows, float* current, const float* noisy, float* cum_out, lrn_stream_t stream) {
   if (!w1 || !b1 || !w2 || !b2 || !tgt || !current || !noisy || !cum_out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (rows <= 0 || rows > (int64_t(1) << 31)) return fail(LRN_ERR_BAD_SHAPE, "rows=%lld", (long long)rows);
-  if ((reinterpret_cast<uintptr_t>(tgt) & 15) || (reinterpret_cast<uintptr_t>(w1) & 15))
-    return fail(LRN_ERR_MISALIGNED, "tgt/w1 need 16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, tgt, w1)) return fail(LRN_ERR_MISALIGNED, "tgt/w1 need 16-byte alignment");
+  LRN_DEVICE(dev);
   const int grid = int((rows + kHeadRows - 1) / kHeadRows);
-  head_kernel<<<grid, 128, 0, reinterpret_cast<cudaStream_t>(stream)>>>(w1, b1, w2, b2, tgt, rows, current, noisy,
-                                                                         cum_out);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(head_kernel, grid, 128, 0, stream, w1, b1, w2, b2, tgt, rows, current, noisy, cum_out);
 }
 
 int lrn_gemm_bias_act(int precision, const void* A, int64_t lda, const void* Wt, int64_t ldw, const float* bias,
@@ -946,19 +892,15 @@ int lrn_gemm_bias_act(int precision, const void* A, int64_t lda, const void* Wt,
   const int bk = int(128 / es);
   if (M <= 0 || N <= 0 || K <= 0 || K % bk || N % 128 || M >= (int64_t(1) << 31))
     return fail(LRN_ERR_BAD_SHAPE, "M=%lld N=%lld K=%lld", (long long)M, (long long)N, (long long)K);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   GemmPlan g = plan_gemm(N, EPI_ACT);
   if (g.bn == 256 && ((M + g.m_rows - 1) / g.m_rows) * (N / 256) < dev.sms / 2) {
     g.bn = 128;  // few tiles (the decoder's query side: a few thousand rows): 128-column tiles give the idle CTA pairs work
     g.b_box_rows = 64;
   }
   CUtensorMap ta, tb;
-  st = make_tmap(&ta, precision, A, M, K, lda, BM);
-  if (st) return st;
-  st = make_tmap(&tb, precision, Wt, N, K, ldw, g.b_box_rows);
-  if (st) return st;
+  LRN_TRY(make_tmap(&ta, precision, A, M, K, lda, BM));
+  LRN_TRY(make_tmap(&tb, precision, Wt, N, K, ldw, g.b_box_rows));
   GemmParams p{};
   p.M = int(M);
   p.m_tiles = int((M + g.m_rows - 1) / g.m_rows);
@@ -977,18 +919,13 @@ int lrn_gemm_bias_act(int precision, const void* A, int64_t lda, const void* Wt,
     if (want > 1) {
       p.kb_per_split = (p.kb_main + want - 1) / want;
       p.k_splits = (p.kb_main + p.kb_per_split - 1) / p.kb_per_split;
-      LRN_CUDA(cudaMemset2DAsync(out, size_t(ldo) * 4, 0, size_t(N) * 4, size_t(M), reinterpret_cast<cudaStream_t>(stream)));
+      LRN_CUDA(cudaMemset2DAsync(out, size_t(ldo) * 4, 0, size_t(N) * 4, size_t(M), stream));
     }
   }
   CUtensorMap tout;
-  const bool staged_ok = precision == LRN_PREC_BF16 && !out_f32 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
-                         (ldo * 2) % 16 == 0;
-  if (staged_ok) {
-    st = make_tmap(&tout, precision, out, M, N, ldo, BM);
-    if (st) return st;
-  }
-  return launch_gemm(precision, g, EPI_ACT, ta, tb, p, dev.sms, reinterpret_cast<cudaStream_t>(stream),
-                     staged_ok ? &tout : nullptr);
+  const bool staged_ok = precision == LRN_PREC_BF16 && !out_f32 && !misaligned(16, out) && (ldo * 2) % 16 == 0;
+  if (staged_ok) LRN_TRY(make_tmap(&tout, precision, out, M, N, ldo, BM));
+  return launch_gemm(precision, g, EPI_ACT, ta, tb, p, dev.sms, stream, staged_ok ? &tout : nullptr);
 }
 
 }  // extern "C"
@@ -1060,10 +997,8 @@ int run_gemm_bf16(const void* A, int64_t lda, int64_t M, int64_t K, const void* 
 
 int pack_w(const float* src, int rows, int cols, void* dst, int64_t ld, bool transpose, cudaStream_t s) {
   const long long total = static_cast<long long>(rows) * cols;
-  pack_bf16_kernel<<<int(std::min<long long>((total + 255) / 256, 2048)), 256, 0, s>>>(
-      src, rows, cols, static_cast<__nv_bfloat16*>(dst), ld, transpose ? 1 : 0);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(pack_bf16_kernel, int(std::min<long long>((total + 255) / 256, 2048)), 256, 0, s, src, rows, cols,
+                static_cast<__nv_bfloat16*>(dst), ld, transpose ? 1 : 0);
 }
 
 // Streaming kernels over a (rows x C) bf16 matrix: grid = (column blocks of 64 channels, row slabs), blocks loop over the rows.
@@ -1096,13 +1031,10 @@ int lrn_encoder_train_forward(const lrn_encoder_params* pr, const lrn_bn_running
   if ((global_feat != nullptr) != (argmax != nullptr) || (global_feat && fused_point_major))
     return fail(LRN_ERR_BAD_ARG, "global_feat and argmax come together and need the (B,1024,N) fused layout");
   if (B <= 0 || N <= 0 || B * N >= (int64_t(1) << 31) - 256) return fail(LRN_ERR_BAD_SHAPE, "B=%lld N=%lld", (long long)B, (long long)N);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const TrainWs W = train_layout(B, N);
   if (workspace_bytes < W.total) return fail(LRN_ERR_WORKSPACE, "workspace %zu < %zu", workspace_bytes, W.total);
-  if (reinterpret_cast<uintptr_t>(workspace) & 1023) return fail(LRN_ERR_MISALIGNED, "workspace must be 1024-byte aligned");
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  if (misaligned(1024, workspace)) return fail(LRN_ERR_MISALIGNED, "workspace must be 1024-byte aligned");
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   auto* X = reinterpret_cast<__nv_bfloat16*>(ws + W.X);
   auto* U = reinterpret_cast<__nv_bfloat16*>(ws + W.U);
@@ -1112,61 +1044,50 @@ int lrn_encoder_train_forward(const lrn_encoder_params* pr, const lrn_bn_running
         *scale = stats + 4 * kStatLd, *shift = stats + 5 * kStatLd;
   const int64_t P = W.P;
 
-  LRN_CUDA(cudaMemsetAsync(stats, 0, size_t(2 * kStatLd) * 4, s));
-  LRN_CUDA(cudaMemsetAsync(ws + W.w[2], 0, W.wpack_end - W.w[2], s));
+  LRN_CUDA(cudaMemsetAsync(stats, 0, size_t(2 * kStatLd) * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(ws + W.w[2], 0, W.wpack_end - W.w[2], stream));
   for (int k = 2; k <= 5; ++k) {  // bf16 copies of the (unfolded) weights, and transposed for the dgrads
-    if ((st = pack_w(pr->conv_w[k - 1], kChan[k], kChan[k - 1], ws + W.w[k], kChan[k - 1], false, s))) return st;
-    if ((st = pack_w(pr->conv_w[k - 1], kChan[k], kChan[k - 1], ws + W.wt[k], kChan[k], true, s))) return st;
+    LRN_TRY(pack_w(pr->conv_w[k - 1], kChan[k], kChan[k - 1], ws + W.w[k], kChan[k - 1], false, stream));
+    LRN_TRY(pack_w(pr->conv_w[k - 1], kChan[k], kChan[k - 1], ws + W.wt[k], kChan[k], true, stream));
   }
-  if ((st = pack_w(pr->fusion_w, 1024, kFusionK, ws + W.wf, kCat, false, s))) return st;
-  if ((st = pack_w(pr->fusion_w, 1024, kFusionK, ws + W.wft, 1024, true, s))) return st;
-  if ((st = pack_w(pr->gate2_w, 1024, 64, ws + W.wg2, 64, false, s))) return st;
-  if ((st = pack_w(pr->gate2_w, 1024, 64, ws + W.wg2t, 1024, true, s))) return st;
+  LRN_TRY(pack_w(pr->fusion_w, 1024, kFusionK, ws + W.wf, kCat, false, stream));
+  LRN_TRY(pack_w(pr->fusion_w, 1024, kFusionK, ws + W.wft, 1024, true, stream));
+  LRN_TRY(pack_w(pr->gate2_w, 1024, 64, ws + W.wg2, 64, false, stream));
+  LRN_TRY(pack_w(pr->gate2_w, 1024, 64, ws + W.wg2t, 1024, true, stream));
 
-  train_embed_kernel<<<int(std::min<int64_t>((P + 15) / 16, int64_t(dev.sms) * 16)), 256, 0, s>>>(
-      reinterpret_cast<const float4*>(context), P, pr->conv_w[0], pr->conv_b[0], pr->gate0_w, pr->gate0_b, U, kULd, X, kCat);
-  LRN_CUDA(cudaGetLastError());
+  LRN_TRY(launch(train_embed_kernel, int(std::min<int64_t>((P + 15) / 16, int64_t(dev.sms) * 16)), 256, 0, stream,
+                 reinterpret_cast<const float4*>(context), P, pr->conv_w[0], pr->conv_b[0], pr->gate0_w, pr->gate0_b, U, kULd, X,
+                 kCat));
 
   for (int i = 0; i < 6; ++i) {  // i = 0..4: conv1..conv5, i = 5: fusion
     const int C = kUW[i], uo = kUOff[i];
     const float* gamma = i < 5 ? pr->bn_w[i] : pr->fusion_bn_w;
     const float* beta = i < 5 ? pr->bn_b[i] : pr->fusion_bn_b;
-    col_stats_kernel<<<stream_grid(col_stats_kernel, C, P, dev.sms), 256, 0, s>>>(U + uo, kULd, P, sum + uo, sumsq + uo, 1);
-    LRN_CUDA(cudaGetLastError());
-    bn_finalize_kernel<<<(C + 127) / 128, 128, 0, s>>>(sum + uo, sumsq + uo, U + uo, P, C, gamma, beta, pr->bn_eps, momentum,
-                                                       running ? running->mean[i] : nullptr,
-                                                       running ? running->var[i] : nullptr, mean + uo, rstd + uo,
-                                                       scale + uo, shift + uo);
-    LRN_CUDA(cudaGetLastError());
+    LRN_TRY(launch(col_stats_kernel, stream_grid(col_stats_kernel, C, P, dev.sms), 256, 0, stream, U + uo, kULd, P, sum + uo,
+                   sumsq + uo, 1));
+    LRN_TRY(launch(bn_finalize_kernel, (C + 127) / 128, 128, 0, stream, sum + uo, sumsq + uo, U + uo, P, C, gamma, beta, pr->bn_eps,
+                   momentum, running ? running->mean[i] : nullptr, running ? running->var[i] : nullptr, mean + uo, rstd + uo,
+                   scale + uo, shift + uo));
     if (i == 5) break;
-    bn_relu_apply_kernel<<<stream_grid(bn_relu_apply_kernel, C, P, dev.sms), 256, 0, s>>>(U + uo, kULd, P, C, scale + uo, shift + uo, X + kCatOff[i + 1], kCat);
-    LRN_CUDA(cudaGetLastError());
+    LRN_TRY(launch(bn_relu_apply_kernel, stream_grid(bn_relu_apply_kernel, C, P, dev.sms), 256, 0, stream, U + uo, kULd, P, C,
+                   scale + uo, shift + uo, X + kCatOff[i + 1], kCat));
     if (i < 4) {  // next layer's pre-activation: U_{k+1} = X_k W_{k+1}^T + b_{k+1}
       const int k = i + 2;
-      st = run_gemm_bf16(X + kCatOff[i + 1], kCat, P, kChan[k - 1], ws + W.w[k], kChan[k - 1], kChan[k], pr->conv_b[k - 1],
-                         U + kUOff[i + 1], kULd, 0, 0, s);
-      if (st) return st;
+      LRN_TRY(run_gemm_bf16(X + kCatOff[i + 1], kCat, P, kChan[k - 1], ws + W.w[k], kChan[k - 1], kChan[k], pr->conv_b[k - 1],
+                            U + kUOff[i + 1], kULd, 0, 0, stream));
     } else {  // fusion conv over the whole operand row, and gate layer 2 over the gate hidden block
-      st = run_gemm_bf16(X, kCat, P, kFusionK, ws + W.wf, kCat, 1024, pr->fusion_b, U + kUOff[5], kULd, 0, 0, s);
-      if (st) return st;
-      st = run_gemm_bf16(X + kFusionK, kCat, P, kGateK, ws + W.wg2, kGateK, 1024, pr->gate2_b, Z, 1024, 0, 0, s);
-      if (st) return st;
+      LRN_TRY(run_gemm_bf16(X, kCat, P, kFusionK, ws + W.wf, kCat, 1024, pr->fusion_b, U + kUOff[5], kULd, 0, 0, stream));
+      LRN_TRY(run_gemm_bf16(X + kFusionK, kCat, P, kGateK, ws + W.wg2, kGateK, 1024, pr->gate2_b, Z, 1024, 0, 0, stream));
     }
   }
-  if (fused_point_major) {
-    fusion_gate_fwd_pm_kernel<<<stream_grid(fusion_gate_fwd_pm_kernel, 1024, P, dev.sms), 256, 0, s>>>(U + kUOff[5], kULd, Z, 1024, P, scale + kUOff[5],
-                                                                   shift + kUOff[5], static_cast<__nv_bfloat16*>(fused));
-  } else {
-    dim3 grid(unsigned((P + 31) / 32), 32);
-    fusion_gate_fwd_kernel<<<grid, 256, 0, s>>>(U + kUOff[5], kULd, Z, 1024, P, int(N), scale + kUOff[5], shift + kUOff[5],
-                                                static_cast<float*>(fused));
-    if (global_feat) {
-      LRN_CUDA(cudaGetLastError());
-      pool_rows_kernel<<<int(std::min<int64_t>((B * 1024 + 7) / 8, int64_t(dev.sms) * 16)), 256, 0, s>>>(
-          static_cast<const float*>(fused), B * 1024, int(N), global_feat, reinterpret_cast<long long*>(argmax));
-    }
-  }
-  LRN_CUDA(cudaGetLastError());
+  if (fused_point_major)
+    return launch(fusion_gate_fwd_pm_kernel, stream_grid(fusion_gate_fwd_pm_kernel, 1024, P, dev.sms), 256, 0, stream, U + kUOff[5],
+                  kULd, Z, 1024, P, scale + kUOff[5], shift + kUOff[5], static_cast<__nv_bfloat16*>(fused));
+  LRN_TRY(launch(fusion_gate_fwd_kernel, dim3(unsigned((P + 31) / 32), 32), 256, 0, stream, U + kUOff[5], kULd, Z, 1024, P, int(N),
+                 scale + kUOff[5], shift + kUOff[5], static_cast<float*>(fused)));
+  if (global_feat)
+    LRN_TRY(launch(pool_rows_kernel, int(std::min<int64_t>((B * 1024 + 7) / 8, int64_t(dev.sms) * 16)), 256, 0, stream,
+                   static_cast<const float*>(fused), B * 1024, int(N), global_feat, reinterpret_cast<long long*>(argmax)));
   return LRN_OK;
 }
 
@@ -1178,12 +1099,9 @@ int lrn_encoder_train_backward(const lrn_encoder_params* pr, const float* contex
   if (!d_fused && !d_global_feat) return fail(LRN_ERR_BAD_ARG, "no output gradient (d_fused and d_global_feat are null)");
   if (d_global_feat && (!argmax || fused_point_major))
     return fail(LRN_ERR_BAD_ARG, "d_global_feat needs the forward's argmax and the (B,1024,N) fused layout");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const TrainWs W = train_layout(B, N);
   if (workspace_bytes < W.total) return fail(LRN_ERR_WORKSPACE, "workspace %zu < %zu", workspace_bytes, W.total);
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   auto* X = reinterpret_cast<__nv_bfloat16*>(ws + W.X);
   auto* U = reinterpret_cast<__nv_bfloat16*>(ws + W.U);
@@ -1198,85 +1116,76 @@ int lrn_encoder_train_backward(const lrn_encoder_params* pr, const float* contex
   float *mean = stats + 2 * kStatLd, *rstd = stats + 3 * kStatLd, *scale = stats + 4 * kStatLd, *shift = stats + 5 * kStatLd,
         *S1 = stats + 6 * kStatLd, *S2 = stats + 7 * kStatLd, *Sz = stats + 8 * kStatLd;
   const int64_t P = W.P;
-  auto d2d = [&](float* dst, const float* src, int n) { return cudaMemcpyAsync(dst, src, size_t(n) * 4, cudaMemcpyDeviceToDevice, s); };
+  auto d2d = [&](float* dst, const float* src, int n) { return cudaMemcpyAsync(dst, src, size_t(n) * 4, cudaMemcpyDeviceToDevice, stream); };
   auto copy_sub = [&](const float* src, int64_t ld, int c0, int rows, int cols, float* dst) {
-    copy_submatrix_kernel<<<elem_grid(static_cast<long long>(rows) * cols), 256, 0, s>>>(src, ld, c0, rows, cols, dst);
-    return cudaGetLastError();
+    return launch(copy_submatrix_kernel, elem_grid(static_cast<long long>(rows) * cols), 256, 0, stream, src, ld, c0, rows, cols, dst);
   };
 
-  LRN_CUDA(cudaMemsetAsync(S1, 0, size_t(2 * kStatLd + 1024) * 4, s));
-  LRN_CUDA(cudaMemsetAsync(g->conv_w[0], 0, 64 * 4 * 4, s));
-  LRN_CUDA(cudaMemsetAsync(g->conv_b[0], 0, 64 * 4, s));
-  LRN_CUDA(cudaMemsetAsync(g->gate0_w, 0, 64 * 4, s));
-  LRN_CUDA(cudaMemsetAsync(g->gate0_b, 0, 64 * 4, s));
-  for (int k = 1; k < 5; ++k) LRN_CUDA(cudaMemsetAsync(g->conv_b[k], 0, size_t(kChan[k + 1]) * 4, s));
-  LRN_CUDA(cudaMemsetAsync(g->fusion_b, 0, 1024 * 4, s));
+  LRN_CUDA(cudaMemsetAsync(S1, 0, size_t(2 * kStatLd + 1024) * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(g->conv_w[0], 0, 64 * 4 * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(g->conv_b[0], 0, 64 * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(g->gate0_w, 0, 64 * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(g->gate0_b, 0, 64 * 4, stream));
+  for (int k = 1; k < 5; ++k) LRN_CUDA(cudaMemsetAsync(g->conv_b[k], 0, size_t(kChan[k + 1]) * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(g->fusion_b, 0, 1024 * 4, stream));
 
   // ---- fused output: gate, ReLU, fusion BatchNorm
   {
     const int uo = kUOff[5];
     if (fused_point_major) {   // dY, dZ and the column sums S1 / S2 (BatchNorm backward) and Sz (gate bias) in one pass
-      fusion_gate_bwd_pm_kernel<<<stream_grid(fusion_gate_bwd_pm_kernel, 1024, P, dev.sms), 256, 0, s>>>(static_cast<const __nv_bfloat16*>(d_fused), U + uo, kULd, Z,
-                                                                     1024, P, scale + uo, shift + uo, mean + uo, rstd + uo, dU, dZ,
-                                                                     1024, S1 + uo, S2 + uo, Sz);
-      LRN_CUDA(cudaGetLastError());
+      LRN_TRY(launch(fusion_gate_bwd_pm_kernel, stream_grid(fusion_gate_bwd_pm_kernel, 1024, P, dev.sms), 256, 0, stream,
+                     static_cast<const __nv_bfloat16*>(d_fused), U + uo, kULd, Z, 1024, P, scale + uo, shift + uo, mean + uo,
+                     rstd + uo, dU, dZ, 1024, S1 + uo, S2 + uo, Sz));
     } else {
-      dim3 grid(unsigned((P + 31) / 32), 32);
-      fusion_gate_bwd_kernel<<<grid, 256, 0, s>>>(static_cast<const float*>(d_fused), d_global_feat,
-                                                  reinterpret_cast<const long long*>(argmax), U + uo, kULd, Z, 1024, P, int(N),
-                                                  scale + uo, shift + uo, dU, dZ, 1024);
-      LRN_CUDA(cudaGetLastError());
-      col_stats_kernel<<<stream_grid(col_stats_kernel, 1024, P, dev.sms), 256, 0, s>>>(dZ, 1024, P, Sz, nullptr, 0);  // d(gate layer 2 bias)
-      LRN_CUDA(cudaGetLastError());
-      bn_bwd_reduce_kernel<<<stream_grid(bn_bwd_reduce_kernel, 1024, P, dev.sms), 256, 0, s>>>(dU, 1024, nullptr, 0, nullptr, nullptr, U + uo, kULd, P, mean + uo,
-                                                               rstd + uo, S1 + uo, S2 + uo);
-      LRN_CUDA(cudaGetLastError());
+      LRN_TRY(launch(fusion_gate_bwd_kernel, dim3(unsigned((P + 31) / 32), 32), 256, 0, stream, static_cast<const float*>(d_fused),
+                     d_global_feat, reinterpret_cast<const long long*>(argmax), U + uo, kULd, Z, 1024, P, int(N), scale + uo,
+                     shift + uo, dU, dZ, 1024));
+      LRN_TRY(launch(col_stats_kernel, stream_grid(col_stats_kernel, 1024, P, dev.sms), 256, 0, stream, dZ, 1024, P, Sz, nullptr,
+                     0));  // d(gate layer 2 bias)
+      LRN_TRY(launch(bn_bwd_reduce_kernel, stream_grid(bn_bwd_reduce_kernel, 1024, P, dev.sms), 256, 0, stream, dU, 1024, nullptr, 0,
+                     nullptr, nullptr, U + uo, kULd, P, mean + uo, rstd + uo, S1 + uo, S2 + uo));
     }
     LRN_CUDA(d2d(g->gate2_b, Sz, 1024));
     LRN_CUDA(d2d(g->fusion_bn_b, S1 + uo, 1024));
     LRN_CUDA(d2d(g->fusion_bn_w, S2 + uo, 1024));
-    bn_bwd_apply_kernel<<<stream_grid(bn_bwd_apply_kernel, 1024, P, dev.sms), 256, 0, s>>>(dU, 1024, nullptr, 0, nullptr, nullptr, U + uo, kULd, P, 1024, mean + uo,
-                                                            rstd + uo, pr->fusion_bn_w, S1 + uo, S2 + uo, dU, 1024);
-    LRN_CUDA(cudaGetLastError());
+    LRN_TRY(launch(bn_bwd_apply_kernel, stream_grid(bn_bwd_apply_kernel, 1024, P, dev.sms), 256, 0, stream, dU, 1024, nullptr, 0,
+                   nullptr, nullptr, U + uo, kULd, P, 1024, mean + uo, rstd + uo, pr->fusion_bn_w, S1 + uo, S2 + uo, dU, 1024));
     // d(fusion conv bias) = sum_p dU is exactly zero: dU is the output of a batch-statistic BatchNorm backward, whose
     // columns sum to zero over the batch (the bias only shifts the batch mean).  It stays at the memset above instead of
     // the bf16 rounding noise a column sum of dU would give; same for conv2..conv5 below.
     // d(operand row) = dUf Wf  (columns >= 1984 of the padded transposed weight are zero)
-    if ((st = run_gemm_bf16(dU, 1024, P, 1024, ws + W.wft, 1024, kCat, nullptr, dA, kCat, 0, 0, s))) return st;
+    LRN_TRY(run_gemm_bf16(dU, 1024, P, 1024, ws + W.wft, 1024, kCat, nullptr, dA, kCat, 0, 0, stream));
     // dWf = dUf^T X   (K = points; MN-major operands straight from the point-major buffers)
-    if ((st = lrn_gemm_tn(dU, 1024, X, kCat, gW, kCat, 1024, kCat, P, stream))) return st;
-    LRN_CUDA(copy_sub(gW, kCat, 0, 1024, kFusionK, g->fusion_w));
+    LRN_TRY(lrn_gemm_tn(dU, 1024, X, kCat, gW, kCat, 1024, kCat, P, stream));
+    LRN_TRY(copy_sub(gW, kCat, 0, 1024, kFusionK, g->fusion_w));
     // gate layer 2: dH = dZ Wg2, dWg2 = dZ^T H
-    if ((st = run_gemm_bf16(dZ, 1024, P, 1024, ws + W.wg2t, 1024, 128, nullptr, dHp, 128, 0, 0, s))) return st;
-    if ((st = lrn_gemm_tn(dZ, 1024, X + 1920, kCat, gW, 128, 1024, 128, P, stream))) return st;
-    LRN_CUDA(copy_sub(gW, 128, 64, 1024, 64, g->gate2_w));
+    LRN_TRY(run_gemm_bf16(dZ, 1024, P, 1024, ws + W.wg2t, 1024, 128, nullptr, dHp, 128, 0, 0, stream));
+    LRN_TRY(lrn_gemm_tn(dZ, 1024, X + 1920, kCat, gW, 128, 1024, 128, P, stream));
+    LRN_TRY(copy_sub(gW, 128, 64, 1024, 64, g->gate2_w));
   }
   // ---- chain, back to front: layer k consumes d(feat_k) = fusion dgrad slice (+ dgrad of layer k + 1)
   for (int k = 5; k >= 1; --k) {
     const int i = k - 1, C = kChan[k], uo = kUOff[i], xo = kCatOff[k];
     const __nv_bfloat16* d2 = k < 5 ? dB : nullptr;
-    bn_bwd_reduce_kernel<<<stream_grid(bn_bwd_reduce_kernel, C, P, dev.sms), 256, 0, s>>>(dA + xo, kCat, d2, 512, scale + uo, shift + uo, U + uo, kULd, P, mean + uo,
-                                                          rstd + uo, S1 + uo, S2 + uo);
-    LRN_CUDA(cudaGetLastError());
+    LRN_TRY(launch(bn_bwd_reduce_kernel, stream_grid(bn_bwd_reduce_kernel, C, P, dev.sms), 256, 0, stream, dA + xo, kCat, d2, 512,
+                   scale + uo, shift + uo, U + uo, kULd, P, mean + uo, rstd + uo, S1 + uo, S2 + uo));
     LRN_CUDA(d2d(g->bn_b[i], S1 + uo, C));
     LRN_CUDA(d2d(g->bn_w[i], S2 + uo, C));
-    bn_bwd_apply_kernel<<<stream_grid(bn_bwd_apply_kernel, C, P, dev.sms), 256, 0, s>>>(dA + xo, kCat, d2, 512, scale + uo, shift + uo, U + uo, kULd, P, C, mean + uo,
-                                                         rstd + uo, pr->bn_w[i], S1 + uo, S2 + uo, dU, 1024);
-    LRN_CUDA(cudaGetLastError());
+    LRN_TRY(launch(bn_bwd_apply_kernel, stream_grid(bn_bwd_apply_kernel, C, P, dev.sms), 256, 0, stream, dA + xo, kCat, d2, 512,
+                   scale + uo, shift + uo, U + uo, kULd, P, C, mean + uo, rstd + uo, pr->bn_w[i], S1 + uo, S2 + uo, dU, 1024));
     if (k == 1) break;
     const int cin = kChan[k - 1], cin_p = std::max(cin, 128);
     // dW_k = dU_k^T X_{k-1}
-    if ((st = lrn_gemm_tn(dU, 1024, X + kCatOff[k - 1], kCat, gW, cin_p, C, cin_p, P, stream))) return st;
-    LRN_CUDA(copy_sub(gW, cin_p, 0, C, cin, g->conv_w[i]));
+    LRN_TRY(lrn_gemm_tn(dU, 1024, X + kCatOff[k - 1], kCat, gW, cin_p, C, cin_p, P, stream));
+    LRN_TRY(copy_sub(gW, cin_p, 0, C, cin, g->conv_w[i]));
     // d(feat_{k-1}) += dU_k W_k
-    if ((st = run_gemm_bf16(dU, 1024, P, C, ws + W.wt[k], C, cin_p, nullptr, dB, 512, 0, 0, s))) return st;
+    LRN_TRY(run_gemm_bf16(dU, 1024, P, C, ws + W.wt[k], C, cin_p, nullptr, dB, 512, 0, 0, stream));
   }
   // ---- conv1 and gate layer 1 (fp32 reductions over the points)
-  conv1_gate1_bwd_kernel<<<int(std::min<int64_t>((P + 2047) / 2048, 1024)), 256, 0, s>>>(
-      reinterpret_cast<const float4*>(context), P, dU, 1024, dHp, 128, X + kFusionK, kCat, g->conv_w[0], g->conv_b[0],
-      g->gate0_w, g->gate0_b);
-  LRN_CUDA(cudaGetLastError());
-  LRN_CUDA(cudaMemsetAsync(g->conv_b[0], 0, 64 * 4, s));  // in front of bn1: exactly zero as well (see fusion_b above)
+  LRN_TRY(launch(conv1_gate1_bwd_kernel, int(std::min<int64_t>((P + 2047) / 2048, 1024)), 256, 0, stream,
+                 reinterpret_cast<const float4*>(context), P, dU, 1024, dHp, 128, X + kFusionK, kCat, g->conv_w[0], g->conv_b[0],
+                 g->gate0_w, g->gate0_b));
+  LRN_CUDA(cudaMemsetAsync(g->conv_b[0], 0, 64 * 4, stream));  // in front of bn1: exactly zero as well (see fusion_b above)
   return LRN_OK;
 }
 
@@ -1284,108 +1193,73 @@ int lrn_adam_step(float* params, const float* grads, float* exp_avg, float* exp_
                   float beta2, float eps, float weight_decay, int64_t step, lrn_stream_t stream) {
   if (!params || !grads || !exp_avg || !exp_avg_sq) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (n <= 0 || step < 1) return fail(LRN_ERR_BAD_SHAPE, "n=%lld step=%lld", (long long)n, (long long)step);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   const double bc1 = 1.0 - pow(double(beta1), double(step)), bc2 = 1.0 - pow(double(beta2), double(step));
   const int grid = int(std::min<int64_t>((n + 255) / 256, int64_t(dev.sms) * 16));
-  adam_step_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(params, grads, exp_avg, exp_avg_sq, n, float(double(lr) / bc1),
-                                                                              beta1, beta2, eps, weight_decay, float(1.0 / sqrt(bc2)));
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(adam_step_kernel, grid, 256, 0, stream, params, grads, exp_avg, exp_avg_sq, n, float(double(lr) / bc1), beta1,
+                beta2, eps, weight_decay, float(1.0 / sqrt(bc2)));
 }
 
 int lrn_adam_step_capturable(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
                              float beta2, float eps, float weight_decay, int64_t* step_state, lrn_stream_t stream) {
   if (!params || !grads || !exp_avg || !exp_avg_sq || !step_state) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (n <= 0) return fail(LRN_ERR_BAD_SHAPE, "n=%lld", (long long)n);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  LRN_DEVICE(dev);
   const int grid = int(std::min<int64_t>((n + 255) / 256, int64_t(dev.sms) * 16));
-  adam_bump_step_kernel<<<1, 1, 0, s>>>(reinterpret_cast<long long*>(step_state));
-  adam_step_dev_kernel<<<grid, 256, 0, s>>>(params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay,
-                                            reinterpret_cast<const long long*>(step_state));
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  LRN_TRY(launch(adam_bump_step_kernel, 1, 1, 0, stream, reinterpret_cast<long long*>(step_state)));
+  return launch(adam_step_dev_kernel, grid, 256, 0, stream, params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps,
+                weight_decay, reinterpret_cast<const long long*>(step_state));
 }
 
 int lrn_l1_deep_supervision(const float* pred, const float* target, int L, int64_t n, float* loss, float* dpred,
                             lrn_stream_t stream) {
   if (!pred || !target || !loss) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (L <= 0 || n <= 0) return fail(LRN_ERR_BAD_SHAPE, "L=%d n=%lld", L, (long long)n);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  LRN_CUDA(cudaMemsetAsync(loss, 0, 4, s));
+  LRN_DEVICE(dev);
+  LRN_CUDA(cudaMemsetAsync(loss, 0, 4, stream));
   const int grid = int(std::min<int64_t>((int64_t(L) * n + 255) / 256, int64_t(dev.sms) * 4));
-  l1_deep_supervision_kernel<<<grid, 256, 0, s>>>(pred, target, L, n, loss, dpred);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(l1_deep_supervision_kernel, grid, 256, 0, stream, pred, target, L, n, loss, dpred);
 }
 
 int lrn_add_layernorm(const float* x, const float* y, const float* gamma, const float* beta, float eps, float* out,
                       float* stats, int64_t rows, int64_t cols, lrn_stream_t stream) {
   if (!x || !gamma || !beta || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (rows <= 0 || cols != 256) return fail(LRN_ERR_BAD_SHAPE, "rows=%lld cols=%lld (d_model = 256)", (long long)rows, (long long)cols);
-  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(out) |
-       reinterpret_cast<uintptr_t>(gamma) | reinterpret_cast<uintptr_t>(beta)) & 15)
-    return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, x, y, out, gamma, beta)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
+  LRN_DEVICE(dev);
   const int grid = int(std::min<int64_t>((rows + 7) / 8, int64_t(dev.sms) * 8));
-  add_layernorm256_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(x, y, gamma, beta, eps, out, stats, rows);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(add_layernorm256_kernel, grid, 256, 0, stream, x, y, gamma, beta, eps, out, stats, rows);
 }
 
 int lrn_add_layernorm_backward(const float* dy, const float* x, const float* y, const float* stats, const float* gamma, float* dz,
                                float* dgamma, float* dbeta, int64_t rows, int64_t cols, lrn_stream_t stream) {
   if (!dy || !x || !stats || !gamma || !dz || !dgamma || !dbeta) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (rows <= 0 || cols != 256) return fail(LRN_ERR_BAD_SHAPE, "rows=%lld cols=%lld (d_model = 256)", (long long)rows, (long long)cols);
-  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dz) |
-       reinterpret_cast<uintptr_t>(gamma)) & 15)
-    return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  LRN_CUDA(cudaMemsetAsync(dgamma, 0, 256 * 4, s));
-  LRN_CUDA(cudaMemsetAsync(dbeta, 0, 256 * 4, s));
+  if (misaligned(16, x, y, dy, dz, gamma)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
+  LRN_DEVICE(dev);
+  LRN_CUDA(cudaMemsetAsync(dgamma, 0, 256 * 4, stream));
+  LRN_CUDA(cudaMemsetAsync(dbeta, 0, 256 * 4, stream));
   const int grid = int(std::min<int64_t>((rows + 7) / 8, int64_t(dev.sms) * 4));
-  add_layernorm256_bwd_kernel<<<grid, 256, 0, s>>>(dy, x, y, stats, gamma, dz, dgamma, dbeta, rows);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(add_layernorm256_bwd_kernel, grid, 256, 0, stream, dy, x, y, stats, gamma, dz, dgamma, dbeta, rows);
 }
 
 int lrn_self_attention32(const float* qk, const float* v, float* out, int B, lrn_stream_t stream) {
   if (!qk || !v || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (B <= 0) return fail(LRN_ERR_BAD_SHAPE, "B=%d", B);
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  LRN_DEVICE(dev);
   static std::atomic<uint64_t> configured{0};
-  if ((st = configure_smem(self_attn32_kernel, int(kSelfAttnSmem), configured))) return st;
-  self_attn32_kernel<<<std::min(B, dev.sms * 2), 256, kSelfAttnSmem, reinterpret_cast<cudaStream_t>(stream)>>>(qk, v, out, B);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  LRN_TRY(configure_smem(self_attn32_kernel, int(kSelfAttnSmem), configured));
+  return launch(self_attn32_kernel, std::min(B, dev.sms * 2), 256, kSelfAttnSmem, stream, qk, v, out, B);
 }
 
 int lrn_head_update(const float* hidden, const float* w2, const float* b2, int64_t rows, float* current, const float* noisy,
                     float* cum, lrn_stream_t stream) {
   if (!hidden || !w2 || !b2 || !current || !noisy || !cum) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (rows <= 0) return fail(LRN_ERR_BAD_SHAPE, "rows=%lld", (long long)rows);
-  if ((reinterpret_cast<uintptr_t>(hidden) | reinterpret_cast<uintptr_t>(w2)) & 15) return fail(LRN_ERR_MISALIGNED, "hidden / w2 need 16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, hidden, w2)) return fail(LRN_ERR_MISALIGNED, "hidden / w2 need 16-byte alignment");
+  LRN_DEVICE(dev);
   const int grid = int(std::min<int64_t>((rows + 7) / 8, int64_t(dev.sms) * 8));
-  head_update_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(hidden, w2, b2, rows, current, noisy, cum);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(head_update_kernel, grid, 256, 0, stream, hidden, w2, b2, rows, current, noisy, cum);
 }
 
 int lrn_rows_linear(const float* x, int64_t ldx, const float* x2, int64_t ldx2, const float* mlp3_w1, const float* mlp3_b1,
@@ -1394,10 +1268,8 @@ int lrn_rows_linear(const float* x, int64_t ldx, const float* x2, int64_t ldx2, 
   if (!x || !w || !out || (mlp3_w1 && (!mlp3_b1 || x2))) return fail(LRN_ERR_BAD_ARG, "null pointer or both x2 and mlp3_w1 given");
   if (M <= 0 || M > (int64_t(1) << 24) || N <= 0 || N % 8 || K <= 0 || K % 32 || K > (1 << 20))
     return fail(LRN_ERR_BAD_SHAPE, "M=%lld N=%lld K=%lld (N %% 8 == 0, K %% 32 == 0)", (long long)M, (long long)N, (long long)K);
-  if ((reinterpret_cast<uintptr_t>(w) & 15)) return fail(LRN_ERR_MISALIGNED, "w needs 16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, w)) return fail(LRN_ERR_MISALIGNED, "w needs 16-byte alignment");
+  LRN_DEVICE(dev);
   RowsLinearArgs a{};
   a.x = x; a.x2 = x2; a.w1 = mlp3_w1; a.b1 = mlp3_b1; a.w = w; a.bias = bias; a.out = out;
   a.ldx = ldx; a.ldx2 = ldx2; a.ldo = ldo;
@@ -1408,76 +1280,55 @@ int lrn_rows_linear(const float* x, int64_t ldx, const float* x2, int64_t ldx2, 
   if (row_tiles > 65535) return fail(LRN_ERR_BAD_SHAPE, "M=%lld: more than 65535 row tiles", (long long)M);
   const bool nb4 = (N / 8) * row_tiles < unsigned(dev.sms);  // few blocks: halve the columns per block
   const dim3 grid(unsigned(N / (nb4 ? 4 : 8)), row_tiles);
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   if (nb4) {
-    if (mlp3_w1) rows_linear_kernel<ROWS_IN_MLP3, 4><<<grid, 256, 0, s>>>(a);
-    else if (x2) rows_linear_kernel<ROWS_IN_SUM, 4><<<grid, 256, 0, s>>>(a);
-    else rows_linear_kernel<ROWS_IN_PLAIN, 4><<<grid, 256, 0, s>>>(a);
-  } else {
-    if (mlp3_w1) rows_linear_kernel<ROWS_IN_MLP3, 8><<<grid, 256, 0, s>>>(a);
-    else if (x2) rows_linear_kernel<ROWS_IN_SUM, 8><<<grid, 256, 0, s>>>(a);
-    else rows_linear_kernel<ROWS_IN_PLAIN, 8><<<grid, 256, 0, s>>>(a);
+    if (mlp3_w1) return launch(rows_linear_kernel<ROWS_IN_MLP3, 4>, grid, 256, 0, stream, a);
+    if (x2) return launch(rows_linear_kernel<ROWS_IN_SUM, 4>, grid, 256, 0, stream, a);
+    return launch(rows_linear_kernel<ROWS_IN_PLAIN, 4>, grid, 256, 0, stream, a);
   }
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  if (mlp3_w1) return launch(rows_linear_kernel<ROWS_IN_MLP3, 8>, grid, 256, 0, stream, a);
+  if (x2) return launch(rows_linear_kernel<ROWS_IN_SUM, 8>, grid, 256, 0, stream, a);
+  return launch(rows_linear_kernel<ROWS_IN_PLAIN, 8>, grid, 256, 0, stream, a);
 }
 
 int lrn_query_pos_hidden(const float* w1, const float* b1, const float* coords, int64_t ld, int64_t rows, float* out,
                          int round_tf32, lrn_stream_t stream) {
   if (!w1 || !b1 || !coords || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (rows <= 0 || ld < 3) return fail(LRN_ERR_BAD_SHAPE, "rows=%lld ld=%lld", (long long)rows, (long long)ld);
-  if (reinterpret_cast<uintptr_t>(out) & 15) return fail(LRN_ERR_MISALIGNED, "out needs 16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, out)) return fail(LRN_ERR_MISALIGNED, "out needs 16-byte alignment");
+  LRN_DEVICE(dev);
   const int grid = int(std::min<int64_t>((rows + 7) / 8, int64_t(dev.sms) * 8));
-  query_pos_hidden_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(coords, ld, rows, w1, b1, out, round_tf32 ? 1 : 0);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(query_pos_hidden_kernel, grid, 256, 0, stream, coords, ld, rows, w1, b1, out, round_tf32 ? 1 : 0);
 }
 
 int lrn_add(const float* a, const float* b, float* out, int64_t n, int round_tf32, lrn_stream_t stream) {
   if (!a || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (n <= 0 || n % 4) return fail(LRN_ERR_BAD_SHAPE, "n=%lld (a positive multiple of 4)", (long long)n);
-  if ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(out)) & 15)
-    return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, a, b, out)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
+  LRN_DEVICE(dev);
   const int grid = int(std::min<int64_t>((n / 4 + 255) / 256, int64_t(dev.sms) * 8));
-  add_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float4*>(a), reinterpret_cast<const float4*>(b),
-                                                                       reinterpret_cast<float4*>(out), n / 4, round_tf32 ? 1 : 0);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(add_kernel, grid, 256, 0, stream, reinterpret_cast<const float4*>(a), reinterpret_cast<const float4*>(b),
+                reinterpret_cast<float4*>(out), n / 4, round_tf32 ? 1 : 0);
 }
 
 int lrn_cross_attention32(const float* q, const float* k, const float* v, int64_t ld_kv, int B, int N, float* out,
                           lrn_stream_t stream) {
   if (!q || !k || !v || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (B <= 0 || N <= 0 || ld_kv < 256 || int64_t(B) * 8 >= (int64_t(1) << 31)) return fail(LRN_ERR_BAD_SHAPE, "B=%d N=%d ld=%lld", B, N, (long long)ld_kv);
-  if (reinterpret_cast<uintptr_t>(q) & 15) return fail(LRN_ERR_MISALIGNED, "q needs 16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, q)) return fail(LRN_ERR_MISALIGNED, "q needs 16-byte alignment");
+  LRN_DEVICE(dev);
   static std::atomic<uint64_t> configured{0};
-  if ((st = configure_smem(cross_attn32_kernel, int(kCrossAttnSmem), configured))) return st;
-  cross_attn32_kernel<<<B * 8, 256, kCrossAttnSmem, reinterpret_cast<cudaStream_t>(stream)>>>(q, k, v, ld_kv, N, out);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  LRN_TRY(configure_smem(cross_attn32_kernel, int(kCrossAttnSmem), configured));
+  return launch(cross_attn32_kernel, B * 8, 256, kCrossAttnSmem, stream, q, k, v, ld_kv, N, out);
 }
 
 int lrn_ctx_attention_merge(const float* part, const float* lse, int B, int splits, void* out, int out_bf16, lrn_stream_t stream) {
   if (!part || !lse || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (B <= 0 || splits <= 0 || int64_t(B) * 256 >= (int64_t(1) << 31)) return fail(LRN_ERR_BAD_SHAPE, "B=%d splits=%d", B, splits);
-  if ((reinterpret_cast<uintptr_t>(part) | reinterpret_cast<uintptr_t>(out)) & 15) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, part, out)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
+  LRN_DEVICE(dev);
   const int rows = B * 256;
   const int grid = std::min((rows + 7) / 8, dev.sms * 8);
-  ctx_merge_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(part, lse, rows, splits, out, out_bf16 ? 1 : 0);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(ctx_merge_kernel, grid, 256, 0, stream, part, lse, rows, splits, out, out_bf16 ? 1 : 0);
 }
 
 static int train_attn_args(TrainAttnParams* p, const float* q, const void* k, int64_t ld_k, const void* v, int64_t ld_v, int B, int N,
@@ -1486,8 +1337,7 @@ static int train_attn_args(TrainAttnParams* p, const float* q, const void* k, in
   if (B <= 0 || N <= 0 || ld_k < 32 || ld_k % 8 || ld_v < 32 || ld_v % 8 || int64_t(B) * 8 >= (int64_t(1) << 31))
     return fail(LRN_ERR_BAD_SHAPE, "B=%d N=%d ld_k=%lld ld_v=%lld", B, N, (long long)ld_k, (long long)ld_v);
   if (!(p_drop >= 0.f && p_drop < 1.f)) return fail(LRN_ERR_BAD_ARG, "dropout probability %f", p_drop);
-  if ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(out)) & 15)
-    return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
+  if (misaligned(16, q, k, v, out)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
   p->q = q;
   p->k = static_cast<const __nv_bfloat16*>(k);
   p->v = static_cast<const __nv_bfloat16*>(v);
@@ -1506,24 +1356,18 @@ static int train_attn_args(TrainAttnParams* p, const float* q, const void* k, in
 int lrn_train_attention_forward(const float* q, const void* k, int64_t ld_k, const void* v, int64_t ld_v, int B, int N, float* out,
                                 float* lse, float p_drop, uint64_t seed, const uint64_t* seed_state, lrn_stream_t stream) {
   TrainAttnParams p{};
-  int st = train_attn_args(&p, q, k, ld_k, v, ld_v, B, N, out, lse, p_drop, seed, seed_state);
-  if (st) return st;
-  DeviceInfo dev;
-  if ((st = device_info(&dev))) return st;
-  train_attn_fwd_kernel<<<B * 8, 128, kTaFwdSmem, reinterpret_cast<cudaStream_t>(stream)>>>(p);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  LRN_TRY(train_attn_args(&p, q, k, ld_k, v, ld_v, B, N, out, lse, p_drop, seed, seed_state));
+  LRN_DEVICE(dev);
+  return launch(train_attn_fwd_kernel, B * 8, 128, kTaFwdSmem, stream, p);
 }
 
 int lrn_train_attention_backward(const float* q, const void* k, int64_t ld_k, const void* v, int64_t ld_v, int B, int N,
                                  const float* out, const float* lse, const float* dout, float* dq, void* dk, int64_t ld_dk, void* dv,
                                  int64_t ld_dv, float p_drop, uint64_t seed, const uint64_t* seed_state, lrn_stream_t stream) {
   TrainAttnParams p{};
-  int st = train_attn_args(&p, q, k, ld_k, v, ld_v, B, N, const_cast<float*>(out), const_cast<float*>(lse), p_drop, seed, seed_state);
-  if (st) return st;
+  LRN_TRY(train_attn_args(&p, q, k, ld_k, v, ld_v, B, N, const_cast<float*>(out), const_cast<float*>(lse), p_drop, seed, seed_state));
   if (!dout || !dq || !dk || !dv) return fail(LRN_ERR_BAD_ARG, "null pointer");
-  if (ld_dk < 32 || ld_dk % 2 || ld_dv < 32 || ld_dv % 2 || (reinterpret_cast<uintptr_t>(dout) | reinterpret_cast<uintptr_t>(dq)) & 15 ||
-      (reinterpret_cast<uintptr_t>(dk) | reinterpret_cast<uintptr_t>(dv)) & 3)
+  if (ld_dk < 32 || ld_dk % 2 || ld_dv < 32 || ld_dv % 2 || misaligned(16, dout, dq) || misaligned(4, dk, dv))
     return fail(LRN_ERR_MISALIGNED, "dout / dq need 16-byte, dk / dv 4-byte alignment; gradient row pitches even and >= 32");
   p.dout = dout;
   p.dq = dq;
@@ -1531,40 +1375,29 @@ int lrn_train_attention_backward(const float* q, const void* k, int64_t ld_k, co
   p.dv = static_cast<__nv_bfloat16*>(dv);
   p.ldg = ld_dk;
   p.ldgv = ld_dv;
-  DeviceInfo dev;
-  if ((st = device_info(&dev))) return st;
-  train_attn_bwd_kernel<<<B * 8, 128, kTaBwdSmem, reinterpret_cast<cudaStream_t>(stream)>>>(p);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  LRN_DEVICE(dev);
+  return launch(train_attn_bwd_kernel, B * 8, 128, kTaBwdSmem, stream, p);
 }
 
 int lrn_col_sum_bf16(const void* A, int64_t ld, int64_t rows, int64_t cols, float* out, lrn_stream_t stream) {
   if (!A || !out) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (rows <= 0 || cols <= 0 || cols % 64 || ld < cols || ld % 8) return fail(LRN_ERR_BAD_SHAPE, "rows=%lld cols=%lld ld=%lld (cols %% 64 == 0, ld %% 8 == 0)", (long long)rows, (long long)cols, (long long)ld);
-  if (reinterpret_cast<uintptr_t>(A) & 15) return fail(LRN_ERR_MISALIGNED, "A needs 16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  LRN_CUDA(cudaMemsetAsync(out, 0, size_t(cols) * 4, s));
-  col_stats_kernel<<<stream_grid(col_stats_kernel, int(cols), rows, dev.sms), 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(A), ld, rows, out, nullptr, 0);
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  if (misaligned(16, A)) return fail(LRN_ERR_MISALIGNED, "A needs 16-byte alignment");
+  LRN_DEVICE(dev);
+  LRN_CUDA(cudaMemsetAsync(out, 0, size_t(cols) * 4, stream));
+  return launch(col_stats_kernel, stream_grid(col_stats_kernel, int(cols), rows, dev.sms), 256, 0, stream,
+                reinterpret_cast<const __nv_bfloat16*>(A), ld, rows, out, nullptr, 0);
 }
 
 int lrn_gather_heads(const void* src, int B, int H, int N, int layer, int L, void* dst, lrn_stream_t stream) {
   if (!src || !dst) return fail(LRN_ERR_BAD_ARG, "null pointer");
   if (B <= 0 || H <= 0 || N <= 0 || L <= 0 || layer < 0 || layer >= L) return fail(LRN_ERR_BAD_SHAPE, "B=%d H=%d N=%d layer=%d L=%d", B, H, N, layer, L);
-  if ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
-  DeviceInfo dev;
-  int st = device_info(&dev);
-  if (st) return st;
+  if (misaligned(16, src, dst)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
+  LRN_DEVICE(dev);
   const long long groups = static_cast<long long>(B) * H * ((N + 7) / 8);
   const int grid = int(std::min<long long>((groups + 7) / 8, static_cast<long long>(dev.sms) * 16));
-  gather_heads_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const uint4*>(src), B, H, N, layer, L,
-                                                                                reinterpret_cast<uint4*>(dst));
-  LRN_CUDA(cudaGetLastError());
-  return LRN_OK;
+  return launch(gather_heads_kernel, grid, 256, 0, stream, reinterpret_cast<const uint4*>(src), B, H, N, layer, L,
+                reinterpret_cast<uint4*>(dst));
 }
 
 }  // extern "C"

@@ -12,8 +12,12 @@ from ._lib import OUT_ARGMAX, OUT_FUSED, OUT_MEMORY, OUT_MEMORY_BF16, OUT_POOL, 
 DEFAULT_CHUNK_ROWS = 148 * 128 * 16   # keep in sync with kDefaultChunkRows (csrc/lrn_abi.cu)
 
 
-def _stream_ptr(device) -> int:
-    return torch.cuda.current_stream(device).cuda_stream
+def _call(fn: str, device, *args) -> None:
+    """lib.<fn>(*args, stream) on `device` and its current stream: a tensor is passed as its data pointer, None as NULL;
+    a non-zero status raises RuntimeError."""
+    with torch.cuda.device(device):
+        args = [a.data_ptr() if isinstance(a, torch.Tensor) else a for a in args]
+        _lib.check(getattr(lib, fn)(*args, torch.cuda.current_stream(device).cuda_stream), fn)
 
 
 def _aligned_bytes(nbytes: int, device, align: int = 1024):
@@ -66,10 +70,7 @@ class FoldedEncoder:
         p.bn_eps = bn_eps
         nbytes = lib.lrn_encoder_packed_bytes(self.prec_id)
         self.blob = _aligned_bytes(nbytes, dev)
-        with torch.cuda.device(dev):
-            _lib.check(lib.lrn_encoder_fold(C.byref(p), self.prec_id, self.blob.data_ptr(), nbytes, _stream_ptr(dev)),
-                       "lrn_encoder_fold")
-        _lib.launch_counter += 7 if self.has_proj else 6
+        _call("lrn_encoder_fold", dev, C.byref(p), self.prec_id, self.blob, nbytes)
         del keep
 
 
@@ -121,23 +122,9 @@ def encoder_forward(folded: FoldedEncoder, context: torch.Tensor, *, pool=True, 
                                torch.empty(B, N, 256, dtype=torch.float32, device=dev))
     nbytes = lib.lrn_encoder_workspace_bytes(B, N, folded.prec_id, flags, chunk_rows)
     ws = _workspace(nbytes, dev)
-    dp = lambda t: t.data_ptr() if t is not None else None
-    with torch.cuda.device(dev):
-        _lib.check(lib.lrn_encoder_forward(folded.blob.data_ptr(), folded.prec_id, context.data_ptr(), B, N, flags,
-                                           dp(gf), dp(fz), dp(am), dp(mem), chunk_rows, ws.data_ptr(), ws.numel(),
-                                           _stream_ptr(dev)), "lrn_encoder_forward")
-    _lib.launch_counter += encoder_launches(B * N, flags, chunk_rows, folded.precision)
+    _call("lrn_encoder_forward", dev, folded.blob, folded.prec_id, context, B, N, flags, gf, fz, am, mem, chunk_rows, ws,
+          ws.numel())
     return out
-
-
-def encoder_launches(P: int, flags: int, chunk_rows: int = 0, precision: str = "bf16") -> int:
-    """Kernels lrn_encoder_forward enqueues for P points (mirrors the chunk loop in csrc/lrn_abi.cu):
-    bf16 tier = fused conv1..conv5 kernel + fusion kernel; tf32 tier = one kernel per layer."""
-    al = lambda v: (v + 127) // 128 * 128
-    chunk = min(al(max(chunk_rows or DEFAULT_CHUNK_ROWS, 128)), al(P))
-    chunks = (P + chunk - 1) // chunk
-    per_chunk = (2 if precision == "bf16" else 6) + (1 if flags & OUT_MEMORY else 0)
-    return chunks * per_chunk + (1 if flags & OUT_ARGMAX else 0)
 
 
 def _cum_out(out, current):
@@ -154,13 +141,7 @@ def head_forward(w1, b1, w2, b2, tgt, current, noisy, out=None):
     tgt = _f32c(tgt)
     rows = tgt.numel() // 256
     cum = _cum_out(out, current)
-    dev = tgt.device
-    with torch.cuda.device(dev):
-        _lib.check(lib.lrn_head_forward(_f32c(w1).data_ptr(), _f32c(b1).data_ptr(), _f32c(w2).data_ptr(),
-                                        _f32c(b2).data_ptr(), tgt.data_ptr(), rows, current.data_ptr(),
-                                        _f32c(noisy).data_ptr(), cum.data_ptr(), _stream_ptr(dev)),
-                   "lrn_head_forward")
-    _lib.launch_counter += 1
+    _call("lrn_head_forward", tgt.device, _f32c(w1), _f32c(b1), _f32c(w2), _f32c(b2), tgt, rows, current, _f32c(noisy), cum)
     return cum
 
 
@@ -176,11 +157,7 @@ def gemm_bias_act(a: torch.Tensor, w: torch.Tensor, bias, *, relu=False, out_dty
     out_dtype = out_dtype or (torch.float32 if prec == _lib.PREC_TF32 else torch.bfloat16)
     out = torch.empty(M, N, dtype=out_dtype, device=a.device)
     b = bias.contiguous().float() if bias is not None else None
-    with torch.cuda.device(a.device):
-        _lib.check(lib.lrn_gemm_bias_act(prec, a.data_ptr(), K, w.data_ptr(), K, b.data_ptr() if b is not None else None,
-                                         out.data_ptr(), N, int(out_dtype == torch.float32), int(relu), M, N, K,
-                                         _stream_ptr(a.device)), "lrn_gemm_bias_act")
-    _lib.launch_counter += 1
+    _call("lrn_gemm_bias_act", a.device, prec, a, K, w, K, b, out, N, int(out_dtype == torch.float32), int(relu), M, N, K)
     return out
 
 
@@ -203,10 +180,7 @@ def gemm_tn(at: torch.Tensor, bt: torch.Tensor) -> torch.Tensor:
     K, M = at.shape
     N = bt.shape[1]
     out = torch.empty(M, N, dtype=torch.float32, device=at.device)
-    with torch.cuda.device(at.device):
-        _lib.check(lib.lrn_gemm_tn(at.data_ptr(), at.stride(0), bt.data_ptr(), bt.stride(0), out.data_ptr(), N, M, N, K,
-                                   _stream_ptr(at.device)), "lrn_gemm_tn")
-    _lib.launch_counter += 1
+    _call("lrn_gemm_tn", at.device, at, at.stride(0), bt, bt.stride(0), out, N, M, N, K)
     return out
 
 
@@ -234,18 +208,11 @@ def ctx_attention(qfold: torch.Tensor, kp: torch.Tensor, mem: torch.Tensor, spli
     direct_bf16 = out_dtype == torch.bfloat16 and splits == 1
     out = torch.empty(B, splits, 256, 256, dtype=torch.bfloat16 if direct_bf16 else torch.float32, device=kp.device)
     lse = torch.empty(B, splits, 256, dtype=torch.float32, device=kp.device)
-    with torch.cuda.device(kp.device):
-        _lib.check(lib.lrn_ctx_attention(qfold.data_ptr(), kp.data_ptr(), ld_kp, mem.data_ptr(), ld_mem, B, N, splits,
-                                         out.data_ptr(), int(direct_bf16), lse.data_ptr(), _stream_ptr(kp.device)),
-                   "lrn_ctx_attention")
-    _lib.launch_counter += 1
+    _call("lrn_ctx_attention", kp.device, qfold, kp, ld_kp, mem, ld_mem, B, N, splits, out, int(direct_bf16), lse)
     if splits == 1 and (direct_bf16 or out_dtype == torch.float32):
         return out[:, 0]
     merged = torch.empty(B, 256, 256, dtype=out_dtype, device=kp.device)     # merge the splits by their log-sum-exp
-    with torch.cuda.device(kp.device):
-        _lib.check(lib.lrn_ctx_attention_merge(out.data_ptr(), lse.data_ptr(), B, splits, merged.data_ptr(),
-                                               int(out_dtype == torch.bfloat16), _stream_ptr(kp.device)), "lrn_ctx_attention_merge")
-    _lib.launch_counter += 1
+    _call("lrn_ctx_attention_merge", kp.device, out, lse, B, splits, merged, int(out_dtype == torch.bfloat16))
     return merged
 
 
@@ -259,10 +226,7 @@ def pos_hidden(w1: torch.Tensor, b1: torch.Tensor, context: torch.Tensor, out: t
     ld = out.stride(-2)
     if out.dim() == 3 and out.shape[0] > 1 and out.stride(0) != out.shape[1] * ld:
         raise ValueError("pos_hidden: segments of `out` must be back to back")
-    with torch.cuda.device(context.device):
-        _lib.check(lib.lrn_pos_hidden(_f32c(w1).data_ptr(), _f32c(b1).data_ptr(), context.data_ptr(), P, out.data_ptr(), ld,
-                                      _stream_ptr(context.device)), "lrn_pos_hidden")
-    _lib.launch_counter += 1
+    _call("lrn_pos_hidden", context.device, _f32c(w1), _f32c(b1), context, P, out, ld)
     return out
 
 
@@ -271,11 +235,8 @@ def add_layernorm(x: torch.Tensor, y, norm: torch.nn.LayerNorm) -> torch.Tensor:
     x = _f32c(x)
     y = _f32c(y) if y is not None else None
     out = torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        _lib.check(lib.lrn_add_layernorm(x.data_ptr(), y.data_ptr() if y is not None else None, _f32c(norm.weight.detach()).data_ptr(),
-                                         _f32c(norm.bias.detach()).data_ptr(), float(norm.eps), out.data_ptr(), None,
-                                         x.numel() // x.shape[-1], x.shape[-1], _stream_ptr(x.device)), "lrn_add_layernorm")
-    _lib.launch_counter += 1
+    _call("lrn_add_layernorm", x.device, x, y, _f32c(norm.weight.detach()), _f32c(norm.bias.detach()), float(norm.eps), out, None,
+          x.numel() // x.shape[-1], x.shape[-1])
     return out
 
 
@@ -287,10 +248,7 @@ def self_attention32(qk: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
     if tuple(qk.shape) != (B, 32, 512) or tuple(v.shape) != (B, 32, 256):
         raise ValueError(f"self_attention32 shapes {tuple(qk.shape)}, {tuple(v.shape)}")
     out = torch.empty_like(v)
-    with torch.cuda.device(v.device):
-        _lib.check(lib.lrn_self_attention32(qk.data_ptr(), v.data_ptr(), out.data_ptr(), B, _stream_ptr(v.device)),
-                   "lrn_self_attention32")
-    _lib.launch_counter += 1
+    _call("lrn_self_attention32", v.device, qk, v, out, B)
     return out
 
 
@@ -300,11 +258,7 @@ def head_update(hidden: torch.Tensor, w2, b2, current: torch.Tensor, noisy: torc
     hidden = _f32c(hidden)
     rows = hidden.numel() // 128
     cum = _cum_out(out, current)
-    with torch.cuda.device(hidden.device):
-        _lib.check(lib.lrn_head_update(hidden.data_ptr(), _f32c(w2.detach()).data_ptr(), _f32c(b2.detach()).data_ptr(), rows,
-                                       current.data_ptr(), _f32c(noisy).data_ptr(), cum.data_ptr(), _stream_ptr(hidden.device)),
-                   "lrn_head_update")
-    _lib.launch_counter += 1
+    _call("lrn_head_update", hidden.device, hidden, _f32c(w2.detach()), _f32c(b2.detach()), rows, current, _f32c(noisy), cum)
     return cum
 
 
@@ -315,6 +269,7 @@ def rows_linear(x: torch.Tensor, w: torch.Tensor, bias, *, add: torch.Tensor | N
     layer of pos_emb / point_mlp fused into the operand load.  Leading dimensions of x are flattened."""
     w = _f32c(w.detach())
     N, K = w.shape
+    w1 = b1 = None
     lead = x.shape[:-1]
     x = _f32c(x).reshape(-1, x.shape[-1])
     M = x.shape[0]
@@ -333,12 +288,8 @@ def rows_linear(x: torch.Tensor, w: torch.Tensor, bias, *, add: torch.Tensor | N
             raise ValueError("rows_linear: addend shape")
     b = _f32c(bias.detach()) if bias is not None else None
     out = torch.empty(M, N, dtype=out_dtype, device=x.device)
-    with torch.cuda.device(x.device):
-        _lib.check(lib.lrn_rows_linear(x.data_ptr(), x.stride(0), x2.data_ptr() if x2 is not None else None, K,
-                                       w1.data_ptr() if mlp3 is not None else None, b1.data_ptr() if mlp3 is not None else None,
-                                       w.data_ptr(), b.data_ptr() if b is not None else None, out.data_ptr(), N,
-                                       int(out_dtype == torch.bfloat16), int(relu), M, N, K, _stream_ptr(x.device)), "lrn_rows_linear")
-    _lib.launch_counter += 1
+    _call("lrn_rows_linear", x.device, x, x.stride(0), x2, K, w1, b1, w, b, out, N, int(out_dtype == torch.bfloat16), int(relu),
+          M, N, K)
     return out.view(*lead, N)
 
 
@@ -349,10 +300,7 @@ def query_pos_hidden(w1: torch.Tensor, b1: torch.Tensor, coords: torch.Tensor, r
     ld = coords.shape[-1]
     rows = coords.numel() // ld
     out = torch.empty(*coords.shape[:-1], 256, dtype=torch.float32, device=coords.device)
-    with torch.cuda.device(coords.device):
-        _lib.check(lib.lrn_query_pos_hidden(_f32c(w1.detach()).data_ptr(), _f32c(b1.detach()).data_ptr(), coords.data_ptr(), ld, rows,
-                                            out.data_ptr(), int(round_tf32), _stream_ptr(coords.device)), "lrn_query_pos_hidden")
-    _lib.launch_counter += 1
+    _call("lrn_query_pos_hidden", coords.device, _f32c(w1.detach()), _f32c(b1.detach()), coords, ld, rows, out, int(round_tf32))
     return out
 
 
@@ -363,10 +311,7 @@ def add(a: torch.Tensor, b: torch.Tensor | None, round_tf32: bool = False) -> to
     if (b is not None and a.shape != b.shape) or a.numel() % 4:
         raise ValueError("add: equal shapes with a multiple of 4 elements expected")
     out = torch.empty_like(a)
-    with torch.cuda.device(a.device):
-        _lib.check(lib.lrn_add(a.data_ptr(), b.data_ptr() if b is not None else None, out.data_ptr(), a.numel(), int(round_tf32),
-                               _stream_ptr(a.device)), "lrn_add")
-    _lib.launch_counter += 1
+    _call("lrn_add", a.device, a, b, out, a.numel(), int(round_tf32))
     return out
 
 
@@ -384,10 +329,7 @@ def cross_attention32(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor) -> torc
     if k.stride(1) != v.stride(1):
         raise ValueError("cross_attention32: k and v must share their row pitch")
     out = torch.empty(B, 32, 256, dtype=torch.float32, device=q.device)
-    with torch.cuda.device(q.device):
-        _lib.check(lib.lrn_cross_attention32(q.data_ptr(), k.data_ptr(), v.data_ptr(), k.stride(1), B, N, out.data_ptr(),
-                                             _stream_ptr(q.device)), "lrn_cross_attention32")
-    _lib.launch_counter += 1
+    _call("lrn_cross_attention32", q.device, q, k, v, k.stride(1), B, N, out)
     return out
 
 
@@ -405,8 +347,5 @@ def point_embed(folded: FoldedEncoder, context: torch.Tensor, tiled: bool = Fals
         out = torch.empty(shape, dtype=dt, device=context.device)
     elif tuple(out.shape) != shape or out.dtype != dt or not out.is_contiguous():
         raise ValueError("point_embed: `out` does not match the requested layout")
-    with torch.cuda.device(context.device):
-        _lib.check(lib.lrn_point_embed(folded.blob.data_ptr(), folded.prec_id, context.data_ptr(), P, out.data_ptr(), int(tiled),
-                                       _stream_ptr(context.device)), "lrn_point_embed")
-    _lib.launch_counter += 1
+    _call("lrn_point_embed", context.device, folded.blob, folded.prec_id, context, P, out, int(tiled))
     return out

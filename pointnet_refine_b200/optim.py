@@ -9,10 +9,8 @@ from __future__ import annotations
 
 import torch
 
-from . import _lib
-from ._lib import lib
 from .flat import FlatParams
-from .ops import _stream_ptr
+from .ops import _call
 
 
 class FlatAdam(torch.optim.Optimizer):
@@ -83,21 +81,14 @@ class FlatAdam(torch.optim.Optimizer):
         self._attach()
         g = self.param_groups[0]
         self._step += 1
-        dev = self._flat.device
+        hyper = (float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]))
         if self.capturable:
-            with torch.cuda.device(dev):
-                _lib.check(lib.lrn_adam_step_capturable(self._flat.data_ptr(), self._grad.data_ptr(), self._m.data_ptr(),
-                                                        self._v.data_ptr(), self._flat.numel(), float(g["lr"]), float(g["betas"][0]),
-                                                        float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]),
-                                                        self._step_dev.data_ptr(), _stream_ptr(dev)), "lrn_adam_step_capturable")
-            _lib.launch_counter += 2
+            _call("lrn_adam_step_capturable", self._flat.device, self._flat, self._grad, self._m, self._v, self._flat.numel(),
+                  *hyper, self._step_dev)
             torch.autograd.graph.increment_version([p for p, _ in self._views])
             return loss
-        with torch.cuda.device(dev):
-            _lib.check(lib.lrn_adam_step(self._flat.data_ptr(), self._grad.data_ptr(), self._m.data_ptr(), self._v.data_ptr(),
-                                         self._flat.numel(), float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]),
-                                         float(g["eps"]), float(g["weight_decay"]), self._step, _stream_ptr(dev)), "lrn_adam_step")
-        _lib.launch_counter += 1
+        _call("lrn_adam_step", self._flat.device, self._flat, self._grad, self._m, self._v, self._flat.numel(), *hyper,
+              self._step)
         # the kernel wrote through raw pointers: tell autograd / the weight-folding caches (data_ptr + _version
         # fingerprints in model.py) that every parameter changed
         torch.autograd.graph.increment_version([p for p, _ in self._views])
@@ -114,10 +105,7 @@ class _DeepSupervisionL1(torch.autograd.Function):
             raise ValueError(f"pred {tuple(pred.shape)} is not (L, *target.shape) for target {tuple(target.shape)}")
         loss = torch.empty((), dtype=torch.float32, device=pred.device)
         dpred = torch.empty_like(pred_c)
-        with torch.cuda.device(pred.device):
-            _lib.check(lib.lrn_l1_deep_supervision(pred_c.data_ptr(), tgt_c.data_ptr(), L, n, loss.data_ptr(), dpred.data_ptr(),
-                                                   _stream_ptr(pred.device)), "lrn_l1_deep_supervision")
-        _lib.launch_counter += 1
+        _call("lrn_l1_deep_supervision", pred.device, pred_c, tgt_c, L, n, loss, dpred)
         ctx.save_for_backward(dpred)
         ctx.pred_dtype = pred.dtype
         return loss

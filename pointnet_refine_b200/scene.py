@@ -17,9 +17,8 @@ from typing import NamedTuple, Sequence
 import numpy as np
 import torch
 
-from . import _lib
 from ._lib import lib
-from .ops import _aligned_bytes, _stream_ptr
+from .ops import _aligned_bytes, _call
 
 
 def resample_polyline(points, num_points: int = 32) -> np.ndarray:
@@ -77,11 +76,7 @@ def _resample_on_device(raw_lines: Sequence, dev):
     d_dense = torch.empty(L, 200, 3, dtype=torch.float64, device=dev)
     d_cent = torch.empty(L, 3, dtype=torch.float64, device=dev)
     centred = torch.empty(L, 32, 3, dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(lib.lrn_scene_resample(d_verts.data_ptr(), d_off.data_ptr(), L, int(lens.max()), d_line.data_ptr(),
-                                          d_dense.data_ptr(), d_cent.data_ptr(), centred.data_ptr(), _stream_ptr(dev)),
-                   "lrn_scene_resample")
-    _lib.launch_counter += 1
+    _call("lrn_scene_resample", dev, d_verts, d_off, L, int(lens.max()), d_line, d_dense, d_cent, centred)
     return d_line, d_dense, d_cent, centred, float(np.abs(verts).max())
 
 
@@ -114,15 +109,9 @@ def build_segments(scene, raw_lines: Sequence, num_context_points: int = 1024, c
     cap = int(capacity) if capacity else max(1 << 20, min(S * L, 8 * L * N))
     for _ in range(2):
         ws = _aligned_bytes(lib.lrn_scene_workspace_bytes(L, cap), dev)
-        with torch.cuda.device(dev):
-            _lib.check(lib.lrn_scene_segments(scene.data_ptr(), S,
-                                              prepared.sorted_points.data_ptr() if prepared.perm is not None else None,
-                                              prepared.perm.data_ptr() if prepared.perm is not None else None,
-                                              d_dense.data_ptr(), d_line.data_ptr(), d_cent.data_ptr(), L, N,
-                                              float(crop_radius), float(decay_scale), extent, int(seed) & (2 ** 64 - 1), cap,
-                                              context.data_ptr(), indices.data_ptr(), counts.data_ptr(), status.data_ptr(),
-                                              ws.data_ptr(), ws.numel(), _stream_ptr(dev)), "lrn_scene_segments")
-        _lib.launch_counter += 6
+        _call("lrn_scene_segments", dev, scene, S, prepared.sorted_points, prepared.perm,
+              d_dense, d_line, d_cent, L, N, float(crop_radius), float(decay_scale), extent, int(seed) & (2 ** 64 - 1), cap,
+              context, indices, counts, status, ws, ws.numel())
         total, flags = (int(v) for v in status.tolist())        # synchronises
         if flags & 2:
             raise RuntimeError("lrn_scene_segments: too many candidates tie exactly at a threshold key")

@@ -12,29 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import lib
-from .ops import _aligned_bytes, _f32c, _stream_ptr
-
-
-class BnRunning(C.Structure):
-    _fields_ = [("mean", C.c_void_p * 6), ("var", C.c_void_p * 6)]
-
-
-class EncoderGrads(C.Structure):
-    _fields_ = ([(n, C.c_void_p * 5) for n in ("conv_w", "conv_b", "bn_w", "bn_b")]
-                + [(n, C.c_void_p) for n in ("fusion_w", "fusion_b", "fusion_bn_w", "fusion_bn_b",
-                                             "gate0_w", "gate0_b", "gate2_w", "gate2_b")])
-
-
-lib.lrn_train_workspace_bytes.restype = C.c_size_t
-lib.lrn_train_workspace_bytes.argtypes = [C.c_int64, C.c_int64]
-lib.lrn_encoder_train_forward.restype = C.c_int
-lib.lrn_encoder_train_forward.argtypes = [C.POINTER(_lib.EncoderParams), C.POINTER(BnRunning), C.c_float, C.c_void_p,
-                                          C.c_int64, C.c_int64, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
-                                          C.c_size_t, C.c_void_p]
-lib.lrn_encoder_train_backward.restype = C.c_int
-lib.lrn_encoder_train_backward.argtypes = [C.POINTER(_lib.EncoderParams), C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
-                                           C.c_int, C.c_void_p, C.c_void_p, C.POINTER(EncoderGrads), C.c_void_p, C.c_size_t,
-                                           C.c_void_p]
+from .ops import _aligned_bytes, _call, _f32c
 
 # parameter order of the autograd node (names relative to MultiScalePointNetEncoder)
 PARAM_NAMES = ([f"conv{k}.weight" for k in range(1, 6)] + [f"conv{k}.bias" for k in range(1, 6)]
@@ -76,17 +54,11 @@ class EncoderTrainFn(torch.autograd.Function):
             am = torch.empty(B, 1024, dtype=torch.int64, device=dev)
         rs = None
         if running is not None:
-            rs = BnRunning()
+            rs = _lib.BnRunning()
             for i in range(6):
                 rs.mean[i], rs.var[i] = running[i].data_ptr(), running[6 + i].data_ptr()
-        with torch.cuda.device(dev):
-            _lib.check(lib.lrn_encoder_train_forward(C.byref(ps), C.byref(rs) if rs is not None else None, momentum,
-                                                     context.data_ptr(), B, N, fused.data_ptr(), int(point_major),
-                                                     gf.data_ptr() if gf is not None else None,
-                                                     am.data_ptr() if am is not None else None,
-                                                     ws.data_ptr(), ws.numel(), _stream_ptr(dev)),
-                       "lrn_encoder_train_forward")
-        _lib.launch_counter += 12 + 1 + 6 * 2 + 5 + 6 + 1 + (0 if point_major else 1)
+        _call("lrn_encoder_train_forward", dev, C.byref(ps), C.byref(rs) if rs is not None else None, momentum, context, B, N,
+              fused, int(point_major), gf, am, ws, ws.numel())
         ctx.save_for_backward(context, *t)
         ctx.ws, ctx.shape, ctx.point_major, ctx.argmax, ctx.eps = ws, (B, N), bool(point_major), am, float(eps)
         if point_major:
@@ -109,21 +81,15 @@ class EncoderTrainFn(torch.autograd.Function):
             d_gf = _f32c(douts[0]) if douts[0] is not None else None
             d_fused = _f32c(douts[1]) if douts[1] is not None else None
         grads = [torch.empty_like(x) for x in t]
-        g = EncoderGrads()
+        g = _lib.EncoderGrads()
         for k in range(5):
             g.conv_w[k], g.conv_b[k] = grads[k].data_ptr(), grads[5 + k].data_ptr()
             g.bn_w[k], g.bn_b[k] = grads[10 + k].data_ptr(), grads[15 + k].data_ptr()
         g.fusion_w, g.fusion_b, g.fusion_bn_w, g.fusion_bn_b = (x.data_ptr() for x in grads[20:24])
         g.gate0_w, g.gate0_b, g.gate2_w, g.gate2_b = (x.data_ptr() for x in grads[24:28])
         ps = _params_struct(t, ctx.eps)
-        with torch.cuda.device(dev):
-            _lib.check(lib.lrn_encoder_train_backward(C.byref(ps), context.data_ptr(), B, N,
-                                                      d_fused.data_ptr() if d_fused is not None else None, int(ctx.point_major),
-                                                      d_gf.data_ptr() if d_gf is not None else None,
-                                                      ctx.argmax.data_ptr() if d_gf is not None else None,
-                                                      C.byref(g), ctx.ws.data_ptr(), ctx.ws.numel(),
-                                                      _stream_ptr(dev)), "lrn_encoder_train_backward")
-        _lib.launch_counter += 60
+        _call("lrn_encoder_train_backward", dev, C.byref(ps), context, B, N, d_fused, int(ctx.point_major), d_gf,
+              ctx.argmax if d_gf is not None else None, C.byref(g), ctx.ws, ctx.ws.numel())
         ctx.ws = None
         return (None, None, None, None, None, *grads)
 
@@ -165,10 +131,7 @@ def _col_sum(dyb):
     if cols % 64:
         return dyb.sum(dim=0, dtype=torch.float32)
     out = torch.empty(cols, dtype=torch.float32, device=dyb.device)
-    with torch.cuda.device(dyb.device):
-        _lib.check(lib.lrn_col_sum_bf16(dyb.data_ptr(), dyb.stride(0), rows, cols, out.data_ptr(), _stream_ptr(dyb.device)),
-                   "lrn_col_sum_bf16")
-    _lib.launch_counter += 1
+    _call("lrn_col_sum_bf16", dyb.device, dyb, dyb.stride(0), rows, cols, out)
     return out
 
 
@@ -259,10 +222,8 @@ class KVProjFn(torch.autograd.Function):
                 if g is None:
                     dy[:, :, i].zero_()
                 elif hd == 32 and g.dtype == torch.bfloat16 and g.is_contiguous():
-                    with torch.cuda.device(g.device):      # (B,H,N,32) as SDPA returns it -> its column block, one pass
-                        _lib.check(lib.lrn_gather_heads(g.data_ptr(), B, H, N, i, L, dy.data_ptr(), _stream_ptr(g.device)),
-                                   "lrn_gather_heads")
-                    _lib.launch_counter += 1
+                    # (B,H,N,32) as SDPA returns it -> its column block, one pass
+                    _call("lrn_gather_heads", g.device, g, B, H, N, i, L, dy)
                 else:
                     dy[:, :, i].copy_(g.transpose(1, 2))
         dyb = dy.view(B * N, -1)
@@ -322,11 +283,7 @@ class CrossAttnTrainFn(torch.autograd.Function):
         out = torch.empty_like(q)
         lse = torch.empty(B, 8, 32, dtype=torch.float32, device=q.device)
         seed, seed_state = DropoutSeedState.next(p_drop)
-        with torch.cuda.device(q.device):
-            _lib.check(lib.lrn_train_attention_forward(q.data_ptr(), k.data_ptr(), ldk, v.data_ptr(), ldv, B, N, out.data_ptr(),
-                                                       lse.data_ptr(), float(p_drop), seed, seed_state, _stream_ptr(q.device)),
-                       "lrn_train_attention_forward")
-        _lib.launch_counter += 1
+        _call("lrn_train_attention_forward", q.device, q, k, ldk, v, ldv, B, N, out, lse, float(p_drop), seed, seed_state)
         ctx.save_for_backward(q, k, v, out, lse)
         ctx.cfg = (float(p_drop), seed, seed_state, share, int(layer))
         return out
@@ -345,12 +302,8 @@ class CrossAttnTrainFn(torch.autograd.Function):
         else:
             gk = torch.empty(B, N, H, hd, dtype=torch.bfloat16, device=q.device).transpose(1, 2)
             gv = torch.empty(B, N, H, hd, dtype=torch.bfloat16, device=q.device).transpose(1, 2)
-        with torch.cuda.device(q.device):
-            _lib.check(lib.lrn_train_attention_backward(q.data_ptr(), k.data_ptr(), k.stride(2), v.data_ptr(), v.stride(2), B, N,
-                                                        out.data_ptr(), lse.data_ptr(), dout.data_ptr(), dq.data_ptr(),
-                                                        gk.data_ptr(), gk.stride(2), gv.data_ptr(), gv.stride(2), p_drop, seed,
-                                                        seed_state, _stream_ptr(q.device)), "lrn_train_attention_backward")
-        _lib.launch_counter += 1
+        _call("lrn_train_attention_backward", q.device, q, k, k.stride(2), v, v.stride(2), B, N, out, lse, dout, dq, gk,
+              gk.stride(2), gv, gv.stride(2), p_drop, seed, seed_state)
         return dq, gk, gv, None, None, None
 
 
@@ -378,10 +331,7 @@ class PosHiddenFn(torch.autograd.Function):
         context = _f32c(context)
         B, N, _ = context.shape
         h = torch.empty(B, N, 256, dtype=torch.bfloat16, device=context.device)
-        with torch.cuda.device(context.device):
-            _lib.check(lib.lrn_pos_hidden(_f32c(w1.detach()).data_ptr(), _f32c(b1.detach()).data_ptr(), context.data_ptr(), B * N,
-                                          h.data_ptr(), 256, _stream_ptr(context.device)), "lrn_pos_hidden")
-        _lib.launch_counter += 1
+        _call("lrn_pos_hidden", context.device, _f32c(w1.detach()), _f32c(b1.detach()), context, B * N, h, 256)
         ctx.save_for_backward(context, h)
         return h
 
@@ -391,10 +341,7 @@ class PosHiddenFn(torch.autograd.Function):
         dh = dh.to(torch.bfloat16).contiguous()
         dw = torch.empty(256, 3, dtype=torch.float32, device=h.device)
         db = torch.empty(256, dtype=torch.float32, device=h.device)
-        with torch.cuda.device(h.device):
-            _lib.check(lib.lrn_pos_hidden_backward(context.data_ptr(), h.numel() // 256, h.data_ptr(), 256, dh.data_ptr(), 256,
-                                                   dw.data_ptr(), db.data_ptr(), _stream_ptr(h.device)), "lrn_pos_hidden_backward")
-        _lib.launch_counter += 1
+        _call("lrn_pos_hidden_backward", h.device, context, h.numel() // 256, h, 256, dh, 256, dw, db)
         return None, dw, db
 
 
@@ -413,10 +360,7 @@ class AddLayerNormFn(torch.autograd.Function):
         rows = x.numel() // 256
         out = torch.empty_like(x)
         stats = torch.empty(rows, 2, dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(lib.lrn_add_layernorm(x.data_ptr(), y.data_ptr(), g.data_ptr(), b.data_ptr(), float(eps), out.data_ptr(),
-                                             stats.data_ptr(), rows, 256, _stream_ptr(x.device)), "lrn_add_layernorm")
-        _lib.launch_counter += 1
+        _call("lrn_add_layernorm", x.device, x, y, g, b, float(eps), out, stats, rows, 256)
         ctx.save_for_backward(x, y, stats, g)
         return out
 
@@ -427,11 +371,7 @@ class AddLayerNormFn(torch.autograd.Function):
         dz = torch.empty_like(x)
         dgamma = torch.empty(256, dtype=torch.float32, device=x.device)
         dbeta = torch.empty(256, dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(lib.lrn_add_layernorm_backward(dout.data_ptr(), x.data_ptr(), y.data_ptr(), stats.data_ptr(), g.data_ptr(),
-                                                      dz.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), x.numel() // 256, 256,
-                                                      _stream_ptr(x.device)), "lrn_add_layernorm_backward")
-        _lib.launch_counter += 1
+        _call("lrn_add_layernorm_backward", x.device, dout, x, y, stats, g, dz, dgamma, dbeta, x.numel() // 256, 256)
         return dz, dz, dgamma, dbeta, None
 
 

@@ -11,24 +11,31 @@ import torch
 
 import pointnet_refine_b200 as prb
 from oracle import synth
-from pointnet_refine_b200 import _lib, ops, shard
+from pointnet_refine_b200 import _lib, shard
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_abi_v3():
     header = open(os.path.join(ROOT, "include", "lrn_b200.h")).read()
     declared = set(re.findall(r"^(?:int|size_t|const char\*) (lrn_[a-z0-9_]+)\(", header, re.M))
     assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 2
+    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 3
     assert _lib.lib.lrn_status_string(3).decode().startswith("unsupported")
     assert _lib.lib.lrn_encoder_packed_bytes(0) > 2 * 2_803_000 - 700      # bf16 blob holds all matrices
     assert _lib.lib.lrn_encoder_packed_bytes(1) > _lib.lib.lrn_encoder_packed_bytes(0)
     assert _lib.lib.lrn_encoder_packed_bytes(7) == 0
     assert _lib.lib.lrn_encoder_workspace_bytes(0, 10, 0, 1, 0) == 0        # empty input has no workspace
+
+
+def test_refused_call_enqueues_no_kernel():
+    """_lib.launch_counter is the library's own count (lrn_launch_count): a call that validation refuses adds nothing."""
+    launches = _lib.launch_counter
+    assert _lib.lib.lrn_encoder_forward(None, 0, None, 1, 16, 1, None, None, None, None, 0, None, 0, None) == 6
+    assert _lib.launch_counter == launches                                  # a call refused by validation enqueues nothing
 
 
 def test_state_dict_is_the_reference_tree():
@@ -51,14 +58,6 @@ def test_cpu_tensors_fail_loudly():
         m(torch.zeros(1, 8, 4), torch.zeros(1, 32, 3))
     with torch.no_grad(), pytest.raises(RuntimeError, match="no CPU implementation"):
         m.context_encoder(torch.zeros(1, 4, 8))
-
-
-def test_launch_accounting_matches_chunk_loop():
-    P = 4096 * 4096
-    assert ops.encoder_launches(P, _lib.OUT_POOL, precision="tf32") == -(-P // ops.DEFAULT_CHUNK_ROWS) * 6
-    assert ops.encoder_launches(P, _lib.OUT_POOL, precision="bf16") == -(-P // ops.DEFAULT_CHUNK_ROWS) * 2
-    assert ops.encoder_launches(1000, _lib.OUT_POOL | _lib.OUT_ARGMAX | _lib.OUT_MEMORY, precision="tf32") == 7 + 1
-    assert ops.encoder_launches(300, _lib.OUT_POOL, chunk_rows=128, precision="tf32") == 3 * 6
 
 
 def test_segment_shard_partitions_exactly():
