@@ -38,6 +38,27 @@ def test_refused_call_enqueues_no_kernel():
     assert _lib.launch_counter == launches                                  # a call refused by validation enqueues nothing
 
 
+def test_packed_layout_mirror_matches_library():
+    """The Python copy of the folded blob's layout, which the stage tests read the blob through, totals what the library
+    allocates for every tier: a drift of the C++ layout fails here, without a GPU."""
+    from tests.test_gpu_encoder_stages import PackedLayout
+    for prec, pid in _lib.PRECISIONS.items():
+        assert PackedLayout(prec).total == _lib.lib.lrn_encoder_packed_bytes(pid), prec
+
+
+def test_workspace_layout_mirror_matches_library():
+    from tests.test_gpu_encoder_stages import WorkspaceLayout
+    flag_sets = (_lib.OUT_POOL, _lib.OUT_ARGMAX, _lib.OUT_FUSED, _lib.OUT_MEMORY, _lib.OUT_POOL | _lib.OUT_ARGMAX,
+                 _lib.OUT_FUSED | _lib.OUT_MEMORY, _lib.OUT_POOL | _lib.OUT_ARGMAX | _lib.OUT_FUSED | _lib.OUT_MEMORY,
+                 _lib.OUT_MEMORY | _lib.OUT_MEMORY_BF16)
+    for B, N in ((1, 1), (1, 127), (3, 1000), (7, 31), (74, 4096), (4096, 4096), (4, 65536)):
+        for prec, pid in _lib.PRECISIONS.items():
+            for flags in flag_sets:
+                for chunk_rows in (0, -1, 1, 127, 128, 129, 128 * 37 * 5, 148 * 128 * 16, 10 ** 8):
+                    want = _lib.lib.lrn_encoder_workspace_bytes(B, N, pid, flags, chunk_rows)
+                    assert WorkspaceLayout(B, N, prec, flags, chunk_rows).total == want, (B, N, prec, flags, chunk_rows)
+
+
 def test_state_dict_is_the_reference_tree():
     m = prb.LineRefineNet()
     sd = synth.make_state_dict(0)
