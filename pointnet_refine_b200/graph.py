@@ -2,10 +2,10 @@
 model once per lane line with B = 1 (inference_whole_scene.py:130-139), where ~100 small launches, not the GPU,
 set the latency.  Capture happens once; every call copies the inputs into static buffers and replays.
 
-The captured launches hold raw pointers: the encoder's scratch buffer, the BN-folded operand blob and the folded decoder
-weights.  The wrapper keeps all of them alive (warm-up and capture run on the same side stream, so the scratch buffer the
-warm-up sized is the one the graph uses), and a replay after a parameter change would silently use the old weights: call
-`recapture()` after load_state_dict / an optimizer step."""
+The captured launches hold raw pointers: the encoder's scratch buffer and every prepared weight (the BN-folded operand
+blob, the folded decoder weights, the TF32-rounded copies).  The wrapper keeps all of them alive (warm-up and capture run
+on the same side stream, so the scratch buffer the warm-up sized is the one the graph uses), and a replay after a
+parameter change would silently use the old weights: call `recapture()` after load_state_dict / an optimizer step."""
 from __future__ import annotations
 
 import torch
@@ -34,9 +34,9 @@ class GraphedLineRefineNet:
         self.graph = torch.cuda.CUDAGraph()
         with torch.no_grad(), torch.cuda.graph(self.graph, stream=side):
             self.out = model(self.ctx, self.line)
-        # everything the captured kernels point at that the graph's own memory pool does not own
-        self._keep = (ops.workspaces_of(dev), model.context_encoder._folded, getattr(model, "_attn_cache", None),
-                      getattr(model, "_pm_cache", None), getattr(model, "_kv_cache", None))
+        # everything the captured kernels point at that the graph's own memory pool does not own; a copy of the prepared
+        # weights, so that invalidate() or a rebuild by a later eager call cannot free what the graph reads
+        self._keep = (ops.workspaces_of(dev), dict(model._prepared))
 
     @torch.no_grad()
     def __call__(self, context: torch.Tensor, noisy_line: torch.Tensor) -> torch.Tensor:

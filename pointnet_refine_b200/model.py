@@ -7,8 +7,9 @@ reference checkpoint works and ``train.py`` / ``inference*.py`` run unchanged wi
 
 What runs where
   * eval mode, CUDA tensors: the context encoder (+ pooling, + context_proj) and the regression
-    heads run in the hand-written sm_100a library through the C ABI (ops.py).  The DETR decoder,
-    point_mlp and pos_emb (SURVEY.md section 8f "next" rows) use stock PyTorch CUDA ops.
+    heads run in the hand-written sm_100a library through the C ABI (ops.py).  In the bf16 and tf32 tiers
+    with M = 32 polyline points the whole decoder does too (LineRefineNet._refine_native); the fp32x3 tier
+    and M != 32 run the DETR decoder and pos_emb in stock fp32 PyTorch ops (LineRefineNet._refine).
   * train mode (batch-statistic BatchNorm, autograd): by default the stock PyTorch fp32 formulation, i.e. exactly
     the reference's numerics (a bf16 forward flips the ReLU mask of a few per mille of the activations, which is
     within tolerance for inference but changes gradients -- the caller decides).  `native_training = True` /
@@ -58,6 +59,17 @@ def _require_cuda(t: torch.Tensor, who: str):
                            f"its inputs to a CUDA device (sm_100a).")
 
 
+def _prepared(cache: dict, name, sources, build, key=()):
+    """cache[name], a weight prepared from parameters (BN fold, re-packed or rounded copy): build() is called again when
+    the (data_ptr, _version) fingerprint of `sources` or the extra `key` changes.  That catches optimizer steps,
+    load_state_dict and .to(); an in-place edit through `.data` bumps no version, hence the modules' invalidate()."""
+    fp = key + tuple((t.data_ptr(), t._version) for t in sources)
+    hit = cache.get(name)
+    if hit is None or hit[0] != fp:
+        cache[name] = hit = (fp, build())
+    return hit[1]
+
+
 class MultiScalePointNetEncoder(nn.Module):
     """Per-point shared MLP 4->64->128->256->512->1024, multi-scale fusion 1984->1024, intensity
     gate, max+avg pooling.  Interface of reference src/model.py:5-62:
@@ -78,33 +90,29 @@ class MultiScalePointNetEncoder(nn.Module):
         self.precision = _DEFAULT_PRECISION     # "bf16" | "tf32" | "fp32x3" (tensor-core operand tier; fp32x3 = 3 x TF32 split, fp32-class)
         self.chunk_rows = 0                     # 0 = library default
         self.native_training = os.environ.get("LRN_NATIVE_TRAIN", "0") == "1"   # opt-in: train mode on the sm_100a kernels (bf16)
-        self._folded = None                     # (fingerprint, FoldedEncoder); never in the state_dict
+        self._prepared = {}                     # prepared weights (_prepared); never in the state_dict
         self._proj = None                       # optional nn.Linear(1024,256) folded alongside (set by LineRefineNet)
-
-    # -- folded-weight cache -------------------------------------------------------------------
-    def _fingerprint(self):
-        ts = list(self.parameters()) + list(self.buffers())
-        if self._proj is not None:
-            ts += list(self._proj[0].parameters())
-        return (self.precision,) + tuple((t.data_ptr(), t._version) for t in ts)
 
     def folded(self) -> ops.FoldedEncoder:
         """BN-folded operand blob for the current parameters; re-folded whenever a parameter or
         running statistic changes (optimizer step, load_state_dict, .to())."""
-        fp = self._fingerprint()
-        if self._folded is None or self._folded[0] != fp:
+        ts = list(self.parameters()) + list(self.buffers())
+        if self._proj is not None:
+            ts += list(self._proj[0].parameters())
+
+        def fold():
             tensors = {k: v for k, v in self.state_dict().items() if v.is_floating_point()}
             if self._proj is not None:
                 tensors["context_proj.weight"] = self._proj[0].weight
                 tensors["context_proj.bias"] = self._proj[0].bias
-            self._folded = (fp, ops.FoldedEncoder(tensors, self.precision, bn_eps=self.bn1.eps))
-        return self._folded[1]
+            return ops.FoldedEncoder(tensors, self.precision, bn_eps=self.bn1.eps)
+        return _prepared(self._prepared, "fold", ts, fold, key=(self.precision,))
 
     def invalidate(self):
-        """Drop the folded-weight cache.  The cache is keyed on (data_ptr, _version) of every parameter and buffer, which
+        """Drop the prepared weights.  They are keyed on (data_ptr, _version) of every parameter and buffer, which
         catches optimizer steps, load_state_dict and .to(); an in-place edit THROUGH `.data` (p.data.copy_(ema),
         p.data.mul_(...)) does not bump `_version` - call this (or LineRefineNet.invalidate()) after such an edit."""
-        self._folded = None
+        self._prepared.clear()
 
     # -- forward ---------------------------------------------------------------------------------
     def run_native(self, context, **outputs):
@@ -195,18 +203,14 @@ class LineRefineNet(nn.Module):
              for _ in range(self.num_decoder_layers)])
         # context_proj is folded into the encoder's operand blob (tuple hides it from the module tree)
         self.context_encoder._proj = (self.context_proj,)
+        self._prepared = self.context_encoder._prepared   # one cache for the encoder fold and the decoder's prepared weights
         self.segment_chunk = 256   # segments per decoder pass in eval mode (bounds the (B,N,256) temporaries)
-        self.fast_decoder = os.environ.get("LRN_FAST_DECODER", "1") != "0"   # bf16 tier: context side on the tensor cores
-        self.ctx_attention = os.environ.get("LRN_CTX_ATTN", "1") != "0"      # ... folded-query attention kernel (else K/V GEMMs + SDPA)
-        self._kv_cache = None
 
     def invalidate(self):
-        """Drop every prepared-weight cache (encoder fold, folded attention weights, point_mlp fold, K / V copies, TF32
+        """Drop every prepared weight (encoder fold, folded attention weights, point_mlp fold, K / V copies, TF32
         copies): needed only after in-place parameter edits through `.data`, which the (data_ptr, _version) fingerprints
         cannot see; optimizer steps, load_state_dict and .to() are detected automatically."""
-        self.context_encoder.invalidate()
-        self._kv_cache = self._attn_cache = self._pm_cache = None
-        self.__dict__.pop("_w32_cache", None)
+        self._prepared.clear()
 
     @property
     def precision(self):
@@ -242,15 +246,15 @@ class LineRefineNet(nn.Module):
         otherwise truncate the low 13 mantissa bits of every operand, a bias that adds up over K."""
         return ((t.contiguous().view(torch.int32) + 0x1000) & ~0x1FFF).view(torch.float32)
 
-    def _kv_weights(self, op):
-        """Copies in the operand type `op` (bf16, or fp32 rounded to the nearest TF32 value for the tf32 tier) of
-        pos_emb.mlp.2 and of the K / V rows of all six cross-attention in_proj matrices ([Wq; Wk; Wv] packing of
-        nn.MultiheadAttention), re-made when a parameter changes.  Host-side weight preparation (like _attn_weights)."""
+    def _kv_weights(self):
+        """Copies, rounded to the nearest TF32 value, of pos_emb.mlp.2 and of the K / V rows of all six cross-attention
+        in_proj matrices ([Wq; Wk; Wv] packing of nn.MultiheadAttention), re-made when a parameter changes: the operands
+        of the tf32 tier's context-side GEMMs.  Host-side weight preparation (like _attn_weights)."""
         ps = [self.pos_emb.mlp[2].weight, self.pos_emb.mlp[2].bias]
         for l in self.decoder_layers:
             ps += [l.cross_attn.in_proj_weight, l.cross_attn.in_proj_bias]
-        fp = (op,) + tuple((t.data_ptr(), t._version) for t in ps)
-        if getattr(self, "_kv_cache", None) is None or self._kv_cache[0] != fp:
+
+        def build():
             d = self.d_model
             dev = ps[0].device
             host = lambda t: t.detach().cpu().float()
@@ -258,110 +262,15 @@ class LineRefineNet(nn.Module):
             wv = torch.cat([host(l.cross_attn.in_proj_weight)[2 * d:] for l in self.decoder_layers])
             bk = torch.cat([host(l.cross_attn.in_proj_bias)[d:2 * d] for l in self.decoder_layers])
             bv = torch.cat([host(l.cross_attn.in_proj_bias)[2 * d:] for l in self.decoder_layers])
-            cast = (lambda t: t.bfloat16().contiguous().to(dev)) if op == torch.bfloat16 else (lambda t: self._rna_tf32(t).to(dev))
-            self._kv_cache = (fp, cast(wk), bk.contiguous().to(dev), cast(wv), bv.contiguous().to(dev),
-                              cast(host(self.pos_emb.mlp[2].weight)))
-        return self._kv_cache[1:]
+            cast = lambda t: self._rna_tf32(t).to(dev)
+            return (cast(wk), bk.contiguous().to(dev), cast(wv), bv.contiguous().to(dev), cast(host(self.pos_emb.mlp[2].weight)))
+        return _prepared(self._prepared, "kv", ps, build)
 
     def _tf32_weight(self, w):
         """fp32 weight (or a row slice of one) rounded to the nearest TF32 value, cached until the parameter changes:
         the operand form of the tf32 tier's tensor-core linears (native rounding kernel, once per parameter update)."""
-        cache = self.__dict__.setdefault("_w32_cache", {})
-        key = (w.data_ptr(), tuple(w.shape))
-        hit = cache.get(key)
-        if hit is None or hit[0] != w._version:
-            cache[key] = hit = (w._version, ops.add(w.detach(), None, round_tf32=True))
-        return hit[1]
-
-    def _refine_tf32(self, context, noisy_line, memory, out):
-        """Eval-mode decoder of the tf32 tier, every step on this library's kernels.  The context-side work is hoisted out
-        of the layer loop: the memory positional embedding and the K / V projections of ALL six cross-attention layers
-        are three TF32 tensor-core GEMMs over the points (they do not depend on the decoder state, src/model.py:123-126;
-        operands rounded to the nearest TF32 value where they are produced - the tensor core would truncate, a bias that
-        adds up over K), and every layer's cross attention is one fp32 lrn_cross_attention32 launch on its column block
-        of those K / V.  Query side as in _refine_attn: tensor-core linears from 256 polyline rows on, fp32 rows_linear
-        below.  Same parameters and math as DetrTransformerDecoderLayer.forward (src/model.py:104-135) in eval mode."""
-        B, N, _ = context.shape
-        d = self.d_model
-        wk, bk, wv, bv, w2 = self._kv_weights(torch.float32)
-        (pw1, pb1), (pw2, pb2), (pw3, pb3) = self._point_mlp_weights()
-        pe0, pe2 = self.pos_emb.mlp[0], self.pos_emb.mlp[2]
-        mem = memory.reshape(B * N, d)
-        h = ops.query_pos_hidden(pe0.weight, pe0.bias, context, round_tf32=True).view(B * N, d)
-        posm = ops.gemm_bias_act(h, w2, pe2.bias.detach())
-        k_all = ops.gemm_bias_act(ops.add(mem, posm, round_tf32=True), wk, bk).view(B, N, 6 * d)
-        v_all = ops.gemm_bias_act(ops.add(mem, None, round_tf32=True), wv, bv).view(B, N, 6 * d)
-        del h, posm
-        rows = B * noisy_line.shape[1]
-        big = rows >= 256
-
-        def lin(x, w, b, relu=False, add=None):
-            if not big:
-                return ops.rows_linear(x, w, b, add=add, relu=relu)
-            x = ops.add(x, add, round_tf32=True)
-            return ops.gemm_bias_act(x.reshape(rows, -1), self._tf32_weight(w), b.detach(), relu=relu).view(B, -1, w.shape[0])
-
-        tgt = ops.rows_linear(ops.rows_linear(noisy_line, pw2, pb2, mlp3=(pw1, pb1), relu=True), pw3, pb3)   # point_mlp
-        current = noisy_line.clone()
-        for i, (layer, head) in enumerate(zip(self.decoder_layers, self.reg_branches)):
-            if big:
-                qpos = lin(ops.query_pos_hidden(pe0.weight, pe0.bias, current), pe2.weight, pe2.bias)
-            else:
-                qpos = ops.rows_linear(current, pe2.weight, pe2.bias, mlp3=(pe0.weight, pe0.bias))
-            sa, ca = layer.self_attn, layer.cross_attn
-            qk = lin(tgt, sa.in_proj_weight[:2 * d], sa.in_proj_bias[:2 * d], add=qpos)
-            v = lin(tgt, sa.in_proj_weight[2 * d:], sa.in_proj_bias[2 * d:])
-            tgt = ops.add_layernorm(tgt, lin(ops.self_attention32(qk, v), sa.out_proj.weight, sa.out_proj.bias), layer.norm1)
-            qh = lin(tgt, ca.in_proj_weight[:d], ca.in_proj_bias[:d], add=qpos)
-            att = ops.cross_attention32(qh, k_all[:, :, i * d:(i + 1) * d], v_all[:, :, i * d:(i + 1) * d])
-            tgt = ops.add_layernorm(tgt, lin(att, ca.out_proj.weight, ca.out_proj.bias), layer.norm2)
-            ffn = lin(lin(tgt, layer.linear1.weight, layer.linear1.bias, relu=True), layer.linear2.weight, layer.linear2.bias)
-            tgt = ops.add_layernorm(tgt, ffn, layer.norm3)
-            hid = lin(tgt, head[0].weight, head[0].bias, relu=True)
-            ops.head_update(hid, head[2].weight, head[2].bias, current, noisy_line, out=out[i])
-
-    def _refine_fast(self, context, noisy_line, memory):
-        """Eval-mode decoder with the context-side work hoisted out of the layer loop: the memory positional
-        embedding and the K / V projections of ALL six cross-attention layers are three tcgen05 GEMMs over the
-        points (they do not depend on the decoder state, src/model.py:123-126), and every layer's cross
-        attention is one scaled_dot_product_attention call on those K / V.  Operands are bf16 in the bf16 tier
-        (when the folded-query kernel is switched off) and fp32 / TF32 tensor cores in the tf32 tier; the larger
-        query-side linears take the tf32 GEMM too.  Same parameters and math as DetrTransformerDecoderLayer.forward
-        (src/model.py:104-135) in eval mode."""
-        B, N, _ = context.shape
-        d, H = self.d_model, 8
-        op = torch.bfloat16 if self.precision == "bf16" else torch.float32
-        wk, bk, wv, bv, w2 = self._kv_weights(op)
-        cast = (lambda t: t.bfloat16()) if op == torch.bfloat16 else self._rna_tf32
-        mem = memory.reshape(B * N, d)
-        h = cast(F.relu(self.pos_emb.mlp[0](context[:, :, :3])).reshape(B * N, d))
-        posm = ops.gemm_bias_act(h, w2, self.pos_emb.mlp[2].bias.detach(), out_dtype=op)
-        k_all = ops.gemm_bias_act(cast(mem + posm), wk, bk, out_dtype=op).view(B, N, 6, H, d // H)
-        v_all = ops.gemm_bias_act(cast(mem), wv, bv, out_dtype=op).view(B, N, 6, H, d // H)
-        rows = B * noisy_line.shape[1]
-
-        def lin(mod, x, relu=False):   # nn.Linear on the tf32 tensor-core GEMM once there are enough rows
-            if rows < 256:
-                y = mod(x)
-                return F.relu(y) if relu else y
-            return ops.gemm_bias_act(self._rna_tf32(x.reshape(rows, -1)), self._rna_tf32(mod.weight.detach()), mod.bias.detach(),
-                                     relu=relu).view(B, -1, mod.out_features)
-
-        tgt = self.point_mlp(noisy_line.transpose(2, 1)).transpose(2, 1)
-        current = noisy_line.clone()
-        outs = []
-        for i, (layer, head) in enumerate(zip(self.decoder_layers, self.reg_branches)):
-            qpos = lin(self.pos_emb.mlp[2], F.relu(self.pos_emb.mlp[0](current)))
-            q = tgt + qpos
-            tgt = layer.norm1(tgt + layer.self_attn(q, q, value=tgt, need_weights=False)[0])
-            ca = layer.cross_attn
-            qh = F.linear(tgt + qpos, ca.in_proj_weight[:d], ca.in_proj_bias[:d]).view(B, -1, H, d // H).transpose(1, 2)
-            att = F.scaled_dot_product_attention(qh.to(op), k_all[:, :, i].transpose(1, 2), v_all[:, :, i].transpose(1, 2))
-            att = att.transpose(1, 2).reshape(B, -1, d).float()
-            tgt = layer.norm2(tgt + lin(ca.out_proj, att))
-            tgt = layer.norm3(tgt + lin(layer.linear2, lin(layer.linear1, tgt, relu=True)))
-            outs.append(ops.head_forward(head[0].weight, head[0].bias, head[2].weight, head[2].bias, tgt, current, noisy_line))
-        return torch.stack(outs)
+        return _prepared(self._prepared, ("tf32", w.data_ptr()), [w], lambda: ops.add(w.detach(), None, round_tf32=True),
+                         key=tuple(w.shape))
 
     # -- cross attention without K / V: folded queries + lrn_ctx_attention ------------------------------------
     def _attn_weights(self):
@@ -374,8 +283,8 @@ class LineRefineNet(nn.Module):
         ps = [self.pos_emb.mlp[2].weight, self.pos_emb.mlp[2].bias]
         for l in self.decoder_layers:
             ps += [l.cross_attn.in_proj_weight, l.cross_attn.in_proj_bias, l.cross_attn.out_proj.weight, l.cross_attn.out_proj.bias]
-        fp = tuple((t.data_ptr(), t._version) for t in ps)
-        if getattr(self, "_attn_cache", None) is None or self._attn_cache[0] != fp:
+
+        def build():
             d, H = self.d_model, 8
             hd = d // H
             dev = ps[0].device
@@ -396,15 +305,15 @@ class LineRefineNet(nn.Module):
                 layers.append((up(wqk), up(bqk), up(wvo), up(bvo), up(wvo.float(), torch.bfloat16)))
             w2 = host(self.pos_emb.mlp[2].weight)
             wx = up(torch.cat([torch.eye(d, dtype=w2.dtype), w2], dim=1).float(), torch.bfloat16)
-            self._attn_cache = (fp, layers, wx, up(host(self.pos_emb.mlp[2].bias)))
-        return self._attn_cache[1:]
+            return layers, wx, up(host(self.pos_emb.mlp[2].bias))
+        return _prepared(self._prepared, "attn", ps, build)
 
     def _point_mlp_weights(self):
         """point_mlp (src/model.py:150-159) with its three eval-mode BatchNorms folded into the 1x1 convs:
         [(W1 (64,3), b1), (W2 (128,64), b2), (W3 (256,128), b3)] fp32.  Host-side weight preparation, cached like _attn_weights."""
         ts = list(self.point_mlp.parameters()) + list(self.point_mlp.buffers())
-        fp = tuple((t.data_ptr(), t._version) for t in ts)
-        if getattr(self, "_pm_cache", None) is None or self._pm_cache[0] != fp:
+
+        def build():
             dev = ts[0].device
             out = []
             for ci, bi in ((0, 1), (3, 4), (6, 7)):
@@ -413,40 +322,42 @@ class LineRefineNet(nn.Module):
                 w = conv.weight.detach().cpu().double().squeeze(-1) * s[:, None]
                 b = (conv.bias.detach().cpu().double() - bn.running_mean.detach().cpu().double()) * s + bn.bias.detach().cpu().double()
                 out.append((w.float().contiguous().to(dev), b.float().contiguous().to(dev)))
-            self._pm_cache = (fp, out)
-        return self._pm_cache[1]
+            return out
+        return _prepared(self._prepared, "point_mlp", ts, build)
 
-    def _refine_attn(self, context, noisy_line, memx, out):
-        """Eval-mode decoder, bf16 tier, M = 32, every step on this library's kernels: per layer the cross attention is ONE
-        lrn_ctx_attention launch over kp = memory + pos and memory (bf16), with Wk / Wv folded into the 32 x 8 queries and
-        into out_proj - K and V of nn.MultiheadAttention (src/model.py:123-128) are never formed.  `memx` (B,N,512) bf16 is
-        the encoder's LRN_OUT_MEMORY_BF16 buffer: [memory | room for the positional hidden layer].  The linears of the
-        query side (point_mlp, pos_emb, self-attention projections, FFN, the folded query / output maps) run on the tcgen05
-        GEMM in its tf32 tier when the batch has >= 256 polyline rows, and as fp32 rows_linear launches below that (B < 8:
-        the whole-scene loop's B = 1, inference_whole_scene.py:130-139); self attention, residual + LayerNorm, heads and
-        the cumulative offsets are the kernels of csrc/query_kernels.cuh.  The six cumulative offsets are written straight
-        into `out` (6,B,32,3).  Same parameters and math as DetrTransformerDecoderLayer.forward (src/model.py:104-135)."""
-        B, N, _ = context.shape
-        d, H = self.d_model, 8
-        layers_w, wx, b2 = self._attn_weights()
-        (pw1, pb1), (pw2, pb2), (pw3, pb3) = self._point_mlp_weights()
-        ops.pos_hidden(self.pos_emb.mlp[0].weight.detach(), self.pos_emb.mlp[0].bias.detach(), context, memx[:, :, d:])
-        kp = ops.gemm_bias_act(memx.view(B * N, 2 * d), wx, b2, out_dtype=torch.bfloat16).view(B, N, d)
-        mem = memx[:, :, :d]
+    def _refine_native(self, context, noisy_line, memory, out):
+        """Eval-mode decoder of the bf16 and tf32 tiers at M = 32, every step on this library's kernels.  The tier supplies
+        the context side and each layer's cross attention (_bf16_cross_attention over the encoder's (B,N,512) bf16
+        LRN_OUT_MEMORY_BF16 buffer, _tf32_cross_attention over the (B,N,256) fp32 memory) and the operand form of the
+        tensor-core linears.  The query side is shared: its linears run on the tcgen05 GEMM in its tf32 mode from 256
+        polyline rows on, and as fp32 rows_linear launches below that (B < 8: the whole-scene loop's B = 1,
+        inference_whole_scene.py:130-139); self attention, residual + LayerNorm, heads and the cumulative offsets are the
+        kernels of csrc/query_kernels.cuh.  The six cumulative offsets go straight into `out` (6,B,32,3).  Same parameters
+        and math as DetrTransformerDecoderLayer.forward (src/model.py:104-135)."""
+        B = context.shape[0]
+        d = self.d_model
+        bf16 = self.precision == "bf16"
         rows = B * noisy_line.shape[1]
         big = rows >= 256     # thousands of rows: tensor-core linears; else one fp32 rows_linear launch per nn.Linear
 
         def lin(x, w, b, relu=False, out_dtype=None, add=None):   # (B,32,K) fp32 [+ add] -> (B,32,N) fp32 (or out_dtype)
             if not big:
                 return ops.rows_linear(x, w, b, add=add, relu=relu, out_dtype=out_dtype or torch.float32)
-            if add is not None:
+            if not bf16:   # tf32 tier: operands rounded to the nearest TF32 value (the bf16 tier lets the tensor core truncate)
+                x, w = ops.add(x, add, round_tf32=True), self._tf32_weight(w)
+            elif add is not None:
                 x = ops.add(x, add)
             return ops.gemm_bias_act(x.reshape(rows, -1), w.detach(), b.detach(), relu=relu, out_dtype=out_dtype).view(B, -1, w.shape[0])
 
+        if bf16:
+            cross_attention = self._bf16_cross_attention(context, memory, lin, big)
+        else:
+            cross_attention = self._tf32_cross_attention(context, memory, lin)
+        (pw1, pb1), (pw2, pb2), (pw3, pb3) = self._point_mlp_weights()
         pe0, pe2 = self.pos_emb.mlp[0], self.pos_emb.mlp[2]
         tgt = ops.rows_linear(ops.rows_linear(noisy_line, pw2, pb2, mlp3=(pw1, pb1), relu=True), pw3, pb3)   # point_mlp
         current = noisy_line.clone()
-        for i, (layer, head, (wqk, bqk, wvo, bvo, wvo16)) in enumerate(zip(self.decoder_layers, self.reg_branches, layers_w)):
+        for i, (layer, head) in enumerate(zip(self.decoder_layers, self.reg_branches)):
             if big:
                 qpos = lin(ops.query_pos_hidden(pe0.weight, pe0.bias, current), pe2.weight, pe2.bias)
             else:
@@ -454,23 +365,62 @@ class LineRefineNet(nn.Module):
             sa = layer.self_attn
             qk = lin(tgt, sa.in_proj_weight[:2 * d], sa.in_proj_bias[:2 * d], add=qpos)
             v = lin(tgt, sa.in_proj_weight[2 * d:], sa.in_proj_bias[2 * d:])
-            att = ops.self_attention32(qk, v)
-            tgt = ops.add_layernorm(tgt, lin(att, sa.out_proj.weight, sa.out_proj.bias), layer.norm1)
-            # folded queries: row q * 8 + h of the segment's 256 (any row order works, rows are independent)
-            qf = lin(tgt, wqk, bqk, out_dtype=torch.bfloat16, add=qpos).view(B, H * 32, d)   # fp32 / tf32 accumulate, rounded once
-            if big:   # attention output leaves the kernel as bf16, Wv / out_proj (folded) is a bf16 GEMM with fp32 output
-                o = ops.ctx_attention(qf, kp, mem, out_dtype=torch.bfloat16).view(rows, H * d)
-                cross = ops.gemm_bias_act(o, wvo16, bvo, out_dtype=torch.float32).view(B, 32, d)
-            else:
-                cross = ops.rows_linear(ops.ctx_attention(qf, kp, mem).view(B, 32, H * d), wvo, bvo)
-            ffn_in = ops.add_layernorm(tgt, cross, layer.norm2)
-            ffn = lin(lin(ffn_in, layer.linear1.weight, layer.linear1.bias, relu=True), layer.linear2.weight, layer.linear2.bias)
-            tgt = ops.add_layernorm(ffn_in, ffn, layer.norm3)
+            tgt = ops.add_layernorm(tgt, lin(ops.self_attention32(qk, v), sa.out_proj.weight, sa.out_proj.bias), layer.norm1)
+            tgt = ops.add_layernorm(tgt, cross_attention(i, tgt, qpos), layer.norm2)
+            ffn = lin(lin(tgt, layer.linear1.weight, layer.linear1.bias, relu=True), layer.linear2.weight, layer.linear2.bias)
+            tgt = ops.add_layernorm(tgt, ffn, layer.norm3)
             hid = lin(tgt, head[0].weight, head[0].bias, relu=True)
             ops.head_update(hid, head[2].weight, head[2].bias, current, noisy_line, out=out[i])
 
+    def _bf16_cross_attention(self, context, memx, lin, big):
+        """bf16 tier: per layer the cross attention is ONE lrn_ctx_attention launch over kp = memory + pos and memory (bf16),
+        with Wk / Wv folded into the 32 x 8 queries and into out_proj (_attn_weights) - K and V of nn.MultiheadAttention
+        (src/model.py:123-128) are never formed.  `memx` (B,N,512) bf16 is the encoder's LRN_OUT_MEMORY_BF16 buffer:
+        [memory | room for the positional hidden layer].  Returns layer i's step (tgt, qpos) -> out_proj output."""
+        B, N, _ = context.shape
+        d, H = self.d_model, 8
+        layers_w, wx, b2 = self._attn_weights()
+        ops.pos_hidden(self.pos_emb.mlp[0].weight.detach(), self.pos_emb.mlp[0].bias.detach(), context, memx[:, :, d:])
+        kp = ops.gemm_bias_act(memx.view(B * N, 2 * d), wx, b2, out_dtype=torch.bfloat16).view(B, N, d)
+        mem = memx[:, :, :d]
+
+        def cross_attention(i, tgt, qpos):
+            wqk, bqk, wvo, bvo, wvo16 = layers_w[i]
+            # folded queries: row q * 8 + h of the segment's 256 (any row order works, rows are independent)
+            qf = lin(tgt, wqk, bqk, out_dtype=torch.bfloat16, add=qpos).view(B, H * 32, d)   # fp32 / tf32 accumulate, rounded once
+            if big:   # attention output leaves the kernel as bf16, Wv / out_proj (folded) is a bf16 GEMM with fp32 output
+                o = ops.ctx_attention(qf, kp, mem, out_dtype=torch.bfloat16).view(B * 32, H * d)
+                return ops.gemm_bias_act(o, wvo16, bvo, out_dtype=torch.float32).view(B, 32, d)
+            return ops.rows_linear(ops.ctx_attention(qf, kp, mem).view(B, 32, H * d), wvo, bvo)
+        return cross_attention
+
+    def _tf32_cross_attention(self, context, memory, lin):
+        """tf32 tier: the context-side work is hoisted out of the layer loop.  The memory positional embedding and the K / V
+        projections of ALL six cross-attention layers are three TF32 tensor-core GEMMs over the points (they do not depend
+        on the decoder state, src/model.py:123-126; operands rounded to the nearest TF32 value where they are produced -
+        the tensor core would truncate, a bias that adds up over K), and every layer's cross attention is one fp32
+        lrn_cross_attention32 launch on its column block of those K / V.  Returns layer i's step (tgt, qpos) -> out_proj
+        output."""
+        B, N, _ = context.shape
+        d = self.d_model
+        wk, bk, wv, bv, w2 = self._kv_weights()
+        pe0, pe2 = self.pos_emb.mlp[0], self.pos_emb.mlp[2]
+        mem = memory.reshape(B * N, d)
+        h = ops.query_pos_hidden(pe0.weight, pe0.bias, context, round_tf32=True).view(B * N, d)
+        posm = ops.gemm_bias_act(h, w2, pe2.bias.detach())
+        k_all = ops.gemm_bias_act(ops.add(mem, posm, round_tf32=True), wk, bk).view(B, N, 6 * d)
+        v_all = ops.gemm_bias_act(ops.add(mem, None, round_tf32=True), wv, bv).view(B, N, 6 * d)
+        del h, posm
+
+        def cross_attention(i, tgt, qpos):
+            ca = self.decoder_layers[i].cross_attn
+            qh = lin(tgt, ca.in_proj_weight[:d], ca.in_proj_bias[:d], add=qpos)
+            att = ops.cross_attention32(qh, k_all[:, :, i * d:(i + 1) * d], v_all[:, :, i * d:(i + 1) * d])
+            return lin(att, ca.out_proj.weight, ca.out_proj.bias)
+        return cross_attention
+
     def _refine_fast_train(self, context, noisy_line, fused_pm):
-        """Autograd-capable twin of _refine_fast for model.train(): context_proj, the memory positional embedding
+        """Autograd-capable decoder of model.train() on the native encoder: context_proj, the memory positional embedding
         and the K / V projections of all six cross-attention layers run as differentiable bf16 tensor-core linears
         (train_ops.linear_bf16: tcgen05 forward, dgrad and wgrad), the cross attention through
         scaled_dot_product_attention with the reference's dropout rate on the attention weights
@@ -542,42 +492,34 @@ class LineRefineNet(nn.Module):
                 or noisy_line.shape[-1] != 3:
             raise ValueError(f"expected context (B,N,4) and noisy_line (B,M,3), got {tuple(context.shape)} and {tuple(noisy_line.shape)}")
         if not _use_native(self, context, noisy_line):
-            from .train_ops import native_train_supported
-            if (self.training and self.fast_decoder and self.precision == "bf16" and self.context_encoder.native_training
-                    and native_train_supported(self.context_encoder)):
-                from .train_ops import encoder_train_forward
-                _, fused_pm = encoder_train_forward(self.context_encoder, context, point_major=True)
+            from .train_ops import encoder_train_forward, native_train_supported
+            enc = self.context_encoder
+            if self.training and self.precision == "bf16" and enc.native_training and native_train_supported(enc):
+                _, fused_pm = encoder_train_forward(enc, context, point_major=True)
                 return self._refine_fast_train(context, noisy_line, fused_pm)
-            _, fused = self.context_encoder(context.transpose(2, 1))   # train mode: native fwd/bwd (bf16 tier)
+            _, fused = enc(context.transpose(2, 1))   # train mode: native fwd/bwd (bf16 tier)
             memory = self.context_proj(fused.transpose(2, 1))
             return self._refine(context, noisy_line, memory, native_heads=False)
-        fast = self.fast_decoder and self.precision != "fp32x3"   # bf16 / tf32 tiers; the folded-query attention kernel below is bf16 only;
-        # the fp32x3 tier keeps the whole decoder in fp32 (stock attention / linears, native point_mlp and heads)
-        attn = fast and self.precision == "bf16" and self.ctx_attention and noisy_line.shape[1] == 32
-        N = context.shape[1]
-        if attn:
+        B, N = context.shape[:2]
+        # bf16 / tf32 tiers with M = 32: the native decoder; the fp32x3 tier and M != 32 keep the whole decoder in fp32
+        # (stock attention / linears, native point_mlp and heads)
+        native = self.precision != "fp32x3" and noisy_line.shape[1] == 32
+        bf16 = native and self.precision == "bf16"
+        if bf16:
             # ~1.2M context points per pass, up to 2048 segments: the query-side GEMMs (32 rows per segment) need
             # thousands of rows to fill the 74 CTA pairs, and no (B,N,1536) K / V temporaries exist on this path
             chunk = max(1, min(8 * self.segment_chunk, (4 * ops.DEFAULT_CHUNK_ROWS) // max(N, 1)))   # four full encoder waves
+        elif native:
+            chunk = max(1, min(self.segment_chunk, (1 << 20) // max(N, 1)))
         else:
-            chunk = max(1, min(self.segment_chunk, (1 << 20) // max(N, 1))) if fast else self.segment_chunk
-        native_tf32 = fast and self.precision == "tf32" and noisy_line.shape[1] == 32
-        if attn or native_tf32:
-            result = torch.empty(self.num_decoder_layers, context.shape[0], 32, 3, dtype=torch.float32, device=context.device)
-            for s in range(0, context.shape[0], chunk):
-                ctx = context[s:s + chunk].contiguous()
-                line = noisy_line[s:s + chunk].contiguous()
-                if attn:
-                    memx = self.context_encoder.run_native(ctx, pool=False, memory=True, memory_bf16=True)["memory"]
-                    self._refine_attn(ctx, line, memx, result[:, s:s + chunk])
-                else:
-                    memory = self.context_encoder.run_native(ctx, pool=False, memory=True)["memory"]
-                    self._refine_tf32(ctx, line, memory, result[:, s:s + chunk])
-            return result
-        outs = []
-        for s in range(0, context.shape[0], chunk):
+            chunk = self.segment_chunk
+        result = torch.empty(self.num_decoder_layers, *noisy_line.shape, dtype=torch.float32, device=context.device)
+        for s in range(0, B, chunk):
             ctx = context[s:s + chunk].contiguous()
             line = noisy_line[s:s + chunk].contiguous()
-            memory = self.context_encoder.run_native(ctx, pool=False, memory=True)["memory"]
-            outs.append(self._refine_fast(ctx, line, memory) if fast else self._refine(ctx, line, memory, native_heads=True))
-        return torch.cat(outs, dim=1)
+            memory = self.context_encoder.run_native(ctx, pool=False, memory=True, memory_bf16=bf16)["memory"]
+            if native:
+                self._refine_native(ctx, line, memory, result[:, s:s + chunk])
+            else:
+                result[:, s:s + chunk] = self._refine(ctx, line, memory, native_heads=True)
+        return result

@@ -74,19 +74,24 @@ def test_eval_forward(dev, prec):
 
 @pytest.mark.parametrize("point_major", [True, False])
 def test_native_train_step(dev, point_major):
-    """forward, fused loss, backward and a capturable FlatAdam step; fast_decoder=False takes the encoder's
-    (B,1024,N) fused layout (point_major off)."""
+    """forward, loss, backward and a capturable FlatAdam step, of the whole model (fused loss; the encoder hands the
+    decoder its point-major (B,N,1024) layout) or of the context encoder alone (its channel-major (B,1024,N) layout)."""
     from pointnet_refine_b200.optim import FlatAdam, deep_supervision_l1
     m = _model(dev, 2).train()
     m.context_encoder.native_training = True
-    m.fast_decoder = point_major
-    opt = FlatAdam(m.parameters(), lr=1e-4, capturable=True)
+    opt = FlatAdam((m if point_major else m.context_encoder).parameters(), lr=1e-4, capturable=True)
     ctx, line = (torch.from_numpy(a).to(dev) for a in synth.make_inputs(8, 512, seed=5))
     tgt = 0.1 * torch.randn(8, 32, 3, device=dev, generator=torch.Generator(device=dev).manual_seed(1))
 
+    def loss():
+        if point_major:
+            return deep_supervision_l1(m(ctx, line), tgt)
+        global_feat, fused = m.context_encoder(ctx.transpose(2, 1))
+        return global_feat.mean() + fused.mean()
+
     def step():
         opt.zero_grad()
-        deep_supervision_l1(m(ctx, line), tgt).backward()
+        loss().backward()
         opt.step()
     step()
     _assert_counted(step)

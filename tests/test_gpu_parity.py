@@ -255,35 +255,23 @@ def test_query_side_kernels_match_torch(dev):
             assert float((cur - want).abs().max()) <= 1e-4 and float((cum - (want - noisy)).abs().max()) <= 1e-4
 
 
+@pytest.mark.parametrize("M", [16, 32, 48])
 @pytest.mark.parametrize("B,N", [(9, 300), (16, 1024)])
-def test_full_forward_batched_vs_live_oracle(dev, B, N):
-    """B * 32 >= 256 query rows: the query-side linears take the tcgen05 tf32 GEMM (smaller batches use F.linear)."""
+def test_full_forward_batched_vs_live_oracle(dev, B, N, M):
+    """Every tier against the live oracle.  M = 32: the native decoder of the bf16 / tf32 tiers, B * 32 >= 256 query rows
+    on the tcgen05 GEMMs (smaller batches use rows_linear); M = 16 / 48, and the fp32x3 tier: the stock fp32 decoder."""
     sd = synth.make_state_dict(21)
-    ctx, line = synth.make_inputs(B, N, seed=5)
+    ctx, line = synth.make_inputs(B, N, M=M, seed=5)
     ref = orc.line_refine_forward(sd, ctx, line)
     rng = max(1.0, float(np.abs(ref).max()))
-    m = _model(sd, dev, "bf16")
-    assert m.fast_decoder and m.ctx_attention
-    with torch.no_grad():
-        out = m(torch.from_numpy(ctx).to(dev), torch.from_numpy(line).to(dev))
-        m.ctx_attention = False
-        out_kv = m(torch.from_numpy(ctx).to(dev), torch.from_numpy(line).to(dev))
-        m.fast_decoder = False
-        out_stock = m(torch.from_numpy(ctx).to(dev), torch.from_numpy(line).to(dev))
-    for tag, o in (("attn", out), ("kv", out_kv), ("stock", out_stock)):
-        err = float(np.abs(o.cpu().numpy() - ref).max())
-        report(test="full_forward_live", B=B, N=N, tier="bf16", path=tag, offsets_err=err, range=rng)
-        assert err <= _offset_tol("bf16", ref), (tag, err)
-    # tf32 tier: K / V GEMMs + SDPA in fp32 with RNA-rounded TF32 operands (fast) vs the stock decoder
-    m32 = _model(sd, dev, "tf32")
-    with torch.no_grad():
-        fast32 = m32(torch.from_numpy(ctx).to(dev), torch.from_numpy(line).to(dev))
-        m32.fast_decoder = False
-        stock32 = m32(torch.from_numpy(ctx).to(dev), torch.from_numpy(line).to(dev))
-    for tag, o in (("fast", fast32), ("stock", stock32)):
-        err = float(np.abs(o.cpu().numpy() - ref).max())
-        report(test="full_forward_live", B=B, N=N, tier="tf32", path=tag, offsets_err=err, range=rng)
-        assert err <= _offset_tol("tf32", ref), (tag, err)
+    for prec in TIERS:
+        m = _model(sd, dev, prec)
+        with torch.no_grad():
+            out = m(torch.from_numpy(ctx).to(dev), torch.from_numpy(line).to(dev))
+        assert out.shape == (6, B, M, 3)
+        err = float(np.abs(out.cpu().numpy() - ref).max())
+        report(test="full_forward_live", B=B, N=N, M=M, tier=prec, offsets_err=err, range=rng)
+        assert err <= _offset_tol(prec, ref), (prec, err)
 
 
 def test_full_forward_chunking_and_segment_independence_at_scale(dev):
@@ -460,17 +448,21 @@ def test_host_pipeline_matches_direct_call(dev):
     assert (got[:, 1024:] - direct[:, 1024:]).abs().max() <= 1e-5
 
 
+@pytest.mark.parametrize("prec", ["bf16", "tf32"])
 @pytest.mark.parametrize("B,N", [(1, 1024), (24, 512)])
-def test_cuda_graph_replay_is_bit_identical(dev, B, N):
+def test_cuda_graph_replay_is_bit_identical(dev, B, N, prec):
     """B = 1 whole-scene style call (inference_whole_scene.py:130-139) and a batch large enough for the native query side:
-    one graph replay == the eager launches."""
+    one graph replay == the eager launches, also after invalidate() and an eager call have rebuilt every prepared weight
+    (the graph reads the ones it was captured with, which it keeps alive)."""
     import pointnet_refine_b200 as prb
     sd = synth.make_state_dict(0)
-    m = _model(sd, dev, "bf16")
+    m = _model(sd, dev, prec)
     ctx, line = (torch.from_numpy(a).to(dev) for a in synth.make_inputs(B, N, seed=21))
     with torch.no_grad():
         eager = m(ctx, line).clone()
         runner = prb.GraphedLineRefineNet(m, B, N)
+        m.invalidate()
+        m(ctx, line)
         for _ in range(3):
             out = runner(ctx, line)
         torch.cuda.synchronize()

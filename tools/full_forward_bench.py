@@ -1,4 +1,4 @@
-"""Full LineRefineNet eval forward (encoder native + decoder in stock PyTorch ops): where does the time go?"""
+"""Full LineRefineNet eval forward against the encoder alone: where does the time go?"""
 import sys, os, time, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -19,7 +19,3 @@ with torch.no_grad():
     t_pool = timeit(lambda: m.context_encoder.run_native(ctx, pool=True))
 print(json.dumps({"B": B, "N": N, "full_forward_ms": round(t_full, 2), "encoder+proj_ms": round(t_enc, 2), "encoder_pool_ms": round(t_pool, 2),
                   "full_segments_per_s": round(B / t_full * 1e3, 1)}))
-m.fast_decoder = False
-with torch.no_grad():
-    t_slow = timeit(lambda: m(ctx, line))
-print(json.dumps({"stock_decoder_full_forward_ms": round(t_slow, 2)}))

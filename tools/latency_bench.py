@@ -20,7 +20,5 @@ with torch.no_grad():
     runner = prb.GraphedLineRefineNet(m, B, N)
     graphed = timeit(lambda: runner(ctx, line))
     out = runner(ctx, line)
-    m.fast_decoder = False
-    stock = timeit(lambda: m(ctx, line))
-print(json.dumps({"B": B, "N": N, "eager_ms": round(eager, 3), "cuda_graph_ms": round(graphed, 3), "stock_decoder_eager_ms": round(stock, 3),
+print(json.dumps({"B": B, "N": N, "eager_ms": round(eager, 3), "cuda_graph_ms": round(graphed, 3),
                   "graph_vs_eager_max_abs": float((out - ref).abs().max())}))
