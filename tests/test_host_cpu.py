@@ -260,3 +260,53 @@ def test_thin_linear_split_k_weight_gradient():
         gr = torch.autograd.grad((ref * r).sum(), (x, w, b))
         for a, c in zip(g, gr):
             assert float((a - c).abs().max()) <= 1e-10 * max(1.0, float(c.abs().max()))
+
+
+def test_folded_cross_attention_equals_multihead_attention():
+    """The fold behind the bf16 tier's cross attention (LineRefineNet._attn_weights, csrc/ctx_attn_sm100.cuh), in fp64 on
+    the CPU: softmax_2((tgt + qpos) Wqk^T + bqk) memory Wvo^T + bvo with the prepared weights up-cast equals
+    nn.MultiheadAttention(q = tgt + qpos, k = memory + pos, v = memory).  The prepared weights are fp32, so the two agree
+    within their rounding: every score is off by at most 2^-24 sum |x wqk| |kp| (+ |bqk| |kp|), which moves a softmax
+    average by at most 2 ln2 max(dS) sum P |mem|, and Wvo / bvo add 2^-24 (|O| |Wvo| + |bvo|); asserted with a factor
+    2 for the second-order terms.  The K bias is the one term the fold may drop (softmax-invariant: equal to 1e-12
+    without the fp32 weights); bqk is not (the fold without it is far outside the bound)."""
+    import math
+    torch.manual_seed(0)
+    m = prb.LineRefineNet().eval()
+    m.load_state_dict(synth.to_torch(synth.make_state_dict(3)), strict=True)
+    with torch.no_grad():
+        for layer in m.decoder_layers:          # biases large enough that a dropped or misplaced term shows
+            layer.cross_attn.in_proj_bias.normal_(0.0, 0.5)
+            layer.cross_attn.out_proj.bias.normal_(0.0, 0.5)
+    m = m.double()
+    layers, _, _ = m._attn_weights()
+    B, M, N, d = 2, 32, 300, 256
+    x = torch.randn(B, M, d, dtype=torch.float64)        # tgt + qpos
+    memory = torch.randn(B, N, d, dtype=torch.float64)
+    kp = memory + torch.randn(B, N, d, dtype=torch.float64)
+    with torch.no_grad():
+        for i, (wqk, bqk, wvo, bvo, _) in enumerate(layers):
+            ca = m.decoder_layers[i].cross_attn
+            ref = ca(x, kp, memory, need_weights=False)[0]
+            wqk, bqk, wvo, bvo = (t.double() for t in (wqk, bqk, wvo, bvo))
+
+            def folded(bq):
+                qf = (x @ wqk.T + bq).view(B, M, 8, d)   # 8 heads x 256 folded dims, scores in log2 units
+                p = torch.softmax(torch.einsum("bmhd,bnd->bmhn", qf, kp) * math.log(2.0), -1)
+                return torch.einsum("bmhn,bnd->bmhd", p, memory).reshape(B, M, 8 * d) @ wvo.T + bvo, p
+
+            got, p = folded(bqk)
+            dS = 2.0 ** -24 * torch.einsum("bmhd,bnd->bmhn", (x.abs() @ wqk.abs().T + bqk.abs()).view(B, M, 8, d), kp.abs())
+            a0 = torch.einsum("bmhn,bnd->bmhd", p, memory.abs())
+            o = torch.einsum("bmhn,bnd->bmhd", p, memory).reshape(B, M, 8 * d)
+            bound = 2 * ((2 * math.log(2.0) * dS.amax(-1, keepdim=True) * a0).reshape(B, M, 8 * d) @ wvo.abs().T
+                         + 2.0 ** -24 * (o.abs() @ wvo.abs().T + bvo.abs()))
+            ratio = float(((got - ref).abs() / bound).max())
+            assert ratio <= 1.0, (i, ratio)
+            no_bqk = float(((folded(torch.zeros_like(bqk))[0] - ref).abs() / bound).max())
+            assert no_bqk > 100.0, (i, no_bqk)
+            bias = ca.in_proj_bias.clone()
+            ca.in_proj_bias[d:2 * d] = 0.0          # the K bias: a per-row constant of the scores
+            same = ca(x, kp, memory, need_weights=False)[0]
+            ca.in_proj_bias.copy_(bias)
+            assert float((same - ref).abs().max()) <= 1e-12 * float(ref.abs().max())
