@@ -182,6 +182,9 @@ chain_pair_kernel(const __grid_constant__ CUtensorMap tmW2, const __grid_constan
   const bool leader = rank == 0;
   const int cluster_id = blockIdx.x >> 1;
   const int num_clusters = gridDim.x >> 1;
+  // Once every CTA of this grid (at most one per SM) runs, the fusion kernel behind it may be launched: its CTAs
+  // take over the SMs one by one as this grid's CTAs exit and wait in griddepcontrol.wait before their first operand load.
+  ptx::launch_dependents();
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmW2);
@@ -499,6 +502,10 @@ chain_pair_kernel(const __grid_constant__ CUtensorMap tmW2, const __grid_constan
       if (lane == 0) ptx::mbar_arrive_cluster(ready_leader0);
       ptx::named_bar_sync(1, 32 * kPairEpiWarps);
       if (issuer) {
+        // The first store into the operand matrix waits for the kernel this one was launched behind (the previous
+        // wave's fusion kernel reads the same buffer); everything up to here - setup, weight loads, the first tile's
+        // points, conv1 / gate layer 1, and conv2 on the tensor pipe - overlaps that kernel's last tiles.
+        if (tile == cluster_id) ptx::grid_dependency_wait();
         store_blk(smem + L::kF1, 0, row0);
         store_blk(smem + L::kGH, 1984, row0);
         ptx::bulk_commit();

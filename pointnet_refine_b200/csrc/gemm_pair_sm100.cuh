@@ -106,6 +106,9 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   constexpr uint32_t kIdesc = ptx::make_idesc(TF32, 2 * BM, BN, MN);
   constexpr int kHalfCols = BN / 2;  // columns handled by one epilogue warp
   constexpr int kChunks = kHalfCols / 32;
+  // bf16 fusion + gate + pooling: launched with programmatic stream serialization behind the chain kernel that writes its
+  // operand rows (lrn_abi.cu), and followed by the next wave's chain kernel, which overwrites them
+  constexpr bool kPdl = EPI == EPI_FUSION && !TF32;
 
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment by pointer arithmetic on the __shared__ array (keeps the shared address space: LDS/STS)
@@ -132,6 +135,8 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   const int kb_all = p.kb_main + p.kb_gate;
   auto kb_begin = [&](int w) { return splits > 1 ? (w / out_tiles) * p.kb_per_split : 0; };
   auto kb_count = [&](int w) { return splits > 1 ? min(p.kb_per_split, kb_all - kb_begin(w)) : kb_all; };
+  // the next wave's chain kernel may start on the SMs this grid's CTAs leave (its stores wait for this grid)
+  if (kPdl) ptx::launch_dependents();
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tmap(&tmA);
@@ -163,6 +168,27 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     uint32_t phase = 0;
     int it = 0;
     const uint32_t full_leader0 = ptx::mapa(ptx::smem_u32(&bar_full[0]), 0);
+    // Behind the chain kernel (kPdl), the weight halves of the first tile's first STAGES k-blocks are loaded before
+    // griddepcontrol.wait, and their operand-row halves, which the chain kernel writes, after it.  Each stage's
+    // expect_tx still counts both halves.
+    int b_early = 0;
+    if (kPdl) {
+      if (cluster_id < num_tiles) {
+        const int n_blk = (cluster_id % out_tiles) % p.n_tiles;
+        b_early = min(STAGES, kb_count(cluster_id));
+        for (int s = 0; s < b_early; ++s) {
+          const KbSlot slot = fusion_slot(fusion_gate_pos(0, p.kb_main), s, p.kb_gate);
+          const int kcol = slot.gate ? p.kb_main + slot.kb : slot.kb;
+          if (ptx::elect_one()) {
+            if (leader) ptx::mbar_arrive_expect_tx(&bar_full[s], 2 * L::kStage);
+            ptx::tma_load_2d_pair(smem + s * L::kStage + L::kA, &tmB, full_leader0 + 8u * s, kcol * BK,
+                                  n_blk * BN + static_cast<int>(rank) * (BN / 2));
+          }
+          __syncwarp();
+        }
+      }
+      ptx::grid_dependency_wait();
+    }
     for (int work = cluster_id; work < num_tiles; work += num_clusters, ++it) {
       const int tile = work % out_tiles;
       const int m_blk = tile / p.n_tiles;
@@ -185,11 +211,12 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           a_extra = pass == 1 ? p.a_lo_off : 0;
           b_extra = pass == 2 ? p.b_lo_off : 0;
         }
+        const bool b_loaded = kPdl && it == 0 && s < b_early;
         ptx::mbar_wait(&bar_empty[stage], phase ^ 1);
         if (ptx::elect_one()) {
           uint8_t* sa = smem + stage * L::kStage;
           const uint32_t full_leader = full_leader0 + 8u * stage;
-          if (leader) ptx::mbar_arrive_expect_tx(&bar_full[stage], 2 * L::kStage);
+          if (leader && !b_loaded) ptx::mbar_arrive_expect_tx(&bar_full[stage], 2 * L::kStage);
           if (MN) {  // boxes of 64 k-rows x 64 m/n columns: this CTA's 128 m and BN/2 n
 #pragma unroll
             for (int b = 0; b < 2; ++b)
@@ -209,7 +236,8 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               ptx::tma_load_4d_pair(sa, &tmA, full_leader, 0, 0, (p.a_col0 + kcol * BK) / BK, a_blk * 2 + static_cast<int>(rank));
             else
               ptx::tma_load_2d_pair(sa, &tmA, full_leader, p.a_col0 + kcol * BK + a_extra, m_blk * 2 * BM + static_cast<int>(rank) * BM);
-            ptx::tma_load_2d_pair(sa + L::kA, &tmB, full_leader, kcol * BK + b_extra, n_blk * BN + static_cast<int>(rank) * (BN / 2));
+            if (!b_loaded)
+              ptx::tma_load_2d_pair(sa + L::kA, &tmB, full_leader, kcol * BK + b_extra, n_blk * BN + static_cast<int>(rank) * (BN / 2));
           }
         }
         __syncwarp();
@@ -376,6 +404,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           seg_hi = vm ? __shfl_sync(0xffffffffu, seg, 31 - __clz(vm)) : seg_lo - 1;
         }
         const bool stamp = p.dbg && cluster_id == 0 && leader && warp == 2 && lane == 0 && it < 16;
+        if (kPdl && it == 0) ptx::grid_dependency_wait();  // pooling atomics and output stores only after the chain kernel
 
         // ---- phase A: G_t -> gamma = 0.5 + 0.5 * sigmoid(G + bg), kept in registers (16-bit fixed point)
         uint32_t gq[kHalfCols / 2];

@@ -69,6 +69,28 @@ int launch(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_
   return LRN_OK;
 }
 
+// launch() with programmatic stream serialization: the kernel may start once the previous kernel of the stream has
+// executed griddepcontrol.launch_dependents in every CTA (or completed), and must itself call griddepcontrol.wait
+// before it touches memory the previous kernel reads or writes.  With programmatic=false: an ordinary launch.
+template <typename... P, typename... A>
+int launch_programmatic(bool programmatic, void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
+                        A&&... args) {
+  if (!programmatic) return launch(kernel, grid, block, smem, s, std::forward<A>(args)...);
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = s;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  LRN_CUDA(cudaLaunchKernelEx(&cfg, kernel, std::forward<A>(args)...));
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  return LRN_OK;
+}
+
 // True when any of the pointers is not `align`-byte aligned (align is a power of two; NULL is aligned).
 template <typename... T>
 bool misaligned(uintptr_t align, T*... p) {
@@ -238,7 +260,8 @@ int launch_pair_t(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMa
   const int tiles = p.m_tiles * p.n_tiles * std::max(p.k_splits, 1);
   if (tiles <= 0) return LRN_OK;
   const int grid = 2 * std::min(tiles, sms / 2);  // one CTA pair (cluster of 2) per work-item slot
-  return launch(kern, grid, kPairThreads, L::kDynamic, stream, ta, tb, tout, p);
+  // the bf16 fusion kernel always follows the chain kernel of its wave (see lrn_encoder_forward)
+  return launch_programmatic(EPI == EPI_FUSION && !TF32, kern, grid, kPairThreads, L::kDynamic, stream, ta, tb, tout, p);
 }
 
 // How one GEMM is tiled over CTA pairs (cta_group::2, 256-row tiles).
@@ -515,8 +538,17 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
       const char* skip_chain = getenv("LRN_DBG_SKIP_CHAIN");
       if (!(skip_chain && atoi(skip_chain)))
 #endif
-      LRN_TRY(launch(chain_pair_kernel, grid, kPairThreads, ChainSmem::kDynamic, stream, tw_chain[0], tw_chain[1], tw_chain[2],
-                     tw_chain[3], ta, cp));
+      // Waves run back to back with programmatic dependent launch: each chain and fusion kernel starts on the SMs the
+      // kernel before it leaves, and sets up, loads weights (chain: also the first tile's points, conv1 / gate layer 1
+      // and conv2) before griddepcontrol.wait.  The hazards that wait covers, all on the single operand buffer `cat`:
+      //   chain(w) stores into cat  after  fusion(w - 1) has read it        (write after read; the first store waits)
+      //   fusion(w) loads cat       after  chain(w) has written it          (read after write; every A load waits)
+      //   fusion(w) pooling atomics after  the global_feat memset above     (chain(w) waited, so fusion(w - 1) is done)
+      // A second operand buffer would not let chain(w) start sooner: its CTA needs the SM that fusion(w - 1)'s CTA holds.
+      // The first chain kernel of a call is an ordinary launch: it follows the memsets and whatever the caller enqueued.
+      // (With LRN_OUT_MEMORY the projection, an ordinary launch, sits between fusion(w - 1) and chain(w).)
+      LRN_TRY(launch_programmatic(r0 > 0, chain_pair_kernel, grid, kPairThreads, ChainSmem::kDynamic, stream, tw_chain[0],
+                                  tw_chain[1], tw_chain[2], tw_chain[3], ta, cp));
     } else {  // layer 1 (+ gate layer 1): raw points -> operand columns
       StageTimer timer(LRN_STAGE_EMBED, stream);
       const int grid = int(std::min<int64_t>((rows + 15) / 16, int64_t(dev.sms) * 16));

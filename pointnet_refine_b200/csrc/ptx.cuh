@@ -172,6 +172,12 @@ __device__ __forceinline__ void cluster_sync() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
+// Programmatic dependent launch.  launch_dependents lets the next kernel of the stream (launched with programmatic
+// stream serialization) start once every CTA of this grid has executed it or exited; grid_dependency_wait blocks until
+// the grid this one depends on has completed and its memory operations are visible.  Both are no-ops in a kernel
+// launched without the attribute / without a programmatic dependent.
+__device__ __forceinline__ void launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void grid_dependency_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 // shared::cta address of a variable -> shared::cluster address of the same variable in CTA `rank`
 __device__ __forceinline__ uint32_t mapa(uint32_t smem_addr, uint32_t rank) {
   uint32_t r;
