@@ -31,7 +31,10 @@ extern "C" {
 #endif
 
 /* 2: lrn_train_attention_forward / _backward take `seed_state`; lrn_adam_step_capturable added
- * 3: lrn_launch_count added */
+ * 3: lrn_launch_count added; later, without a version change, lrn_scenes_segments / lrn_scenes_workspace_bytes (lines of
+ *    many scenes in one call).  Those are additions only: every entry point above keeps its signature and its results,
+ *    so a caller built against an earlier version-3 library runs unchanged, and a caller that needs the additions finds
+ *    them missing by name when it loads an older library (pointnet_refine_b200/_lib.py reports which). */
 #define LRN_ABI_VERSION 3
 
 typedef struct CUstream_st* lrn_stream_t; /* == cudaStream_t */
@@ -281,6 +284,34 @@ int lrn_scene_segments(const float* scene, int64_t S, const float* scene_sorted,
                        int L, int N, double crop_radius, double decay_scale, double coord_extent, uint64_t seed, int64_t capacity,
                        float* context, int64_t* indices, int32_t* counts, int64_t* status, void* workspace, size_t workspace_bytes,
                        lrn_stream_t stream);
+
+/* lrn_scene_segments for lines of MANY scenes in one call (training batches that mix scenes, a whole drive at inference).
+ *   points    (S_total, 4) fp32: K scenes back to back; scene_offsets (K+1) int64 device: scene k is
+ *             points[scene_offsets[k] .. scene_offsets[k+1])
+ *   sorted_points / perm: optional (both or neither): every scene's spatially sorted copy, concatenated the same way, with
+ *             perm[scene_offsets[k] + i] = index WITHIN scene k of sorted_points[scene_offsets[k] + i]
+ *   line_scene (L) int32: scene of every line, in the caller's order (lines of different scenes may be interleaved)
+ *   dense200, line32, centers: per line as for lrn_scene_segments (lrn_scene_resample)
+ *   seeds (L) uint64, line_ids (L) uint32: the RNG identity of every line
+ *   context (L, N, 4), indices (L, N), counts (L): in the caller's line order; indices are WITHIN the line's scene (-1: the
+ *             zero points of an empty crop), exactly what lrn_scene_segments returns for that scene
+ *   status    (2) int64 out: as for lrn_scene_segments (one status for the whole call), plus [1] bit 2: some line_scene[l] is
+ *             not in [0, K) (that line's outputs are not written)
+ *   coord_extent: largest |coordinate| over the scenes and lines of the call.  It only sizes the band in which the fp32
+ *             pre-filter defers to float64; the crop decision itself is exact for any extent at least that large (inside
+ *             the band the distance is evaluated in double), so one extent per call gives the per-scene results.
+ * RNG identity: the draw of line l is the RNG contract of oracle/scene_oracle.py with (seed, line, scene index) =
+ * (seeds[l], line_ids[l], index within scene line_scene[l]), i.e. scene_oracle.build_segment(scene_k, raw, N, r, decay,
+ * seeds[l], line_ids[l]).  lrn_scene_segments over the lines of one scene is the case seeds[l] = seed, line_ids[l] = position
+ * of l among that scene's lines, and gives the same bits.
+ * One pass: each point is tested only against the lines of its own scene; blocks of scenes without a line exit at once.
+ * Launches per call are independent of K.  S_total < 2^31, K <= 65535, L <= 65535, N <= 4096 (else LRN_ERR_BAD_SHAPE). */
+size_t lrn_scenes_workspace_bytes(int L, int K, int64_t capacity);
+int lrn_scenes_segments(const float* points, const int64_t* scene_offsets, int K, int64_t S_total, const float* sorted_points,
+                        const int32_t* perm, const int32_t* line_scene, const double* dense200, const double* line32,
+                        const double* centers, const uint64_t* seeds, const uint32_t* line_ids, int L, int N, double crop_radius,
+                        double decay_scale, double coord_extent, int64_t capacity, float* context, int64_t* indices, int32_t* counts,
+                        int64_t* status, void* workspace, size_t workspace_bytes, lrn_stream_t stream);
 
 /* ---- query side of the decoder (SURVEY.md 8f row 2; DetrTransformerDecoderLayer.forward, src/model.py:104-135) ----
  * out = LayerNorm(x + y) * gamma + beta over rows of 256 (norm1 / norm2 / norm3 with their residual adds, :117,:129,:134);

@@ -11,5 +11,6 @@ from .model import (DetrTransformerDecoderLayer, LineRefineNet, MultiScalePointN
 from .graph import GraphedLineRefineNet, GraphedTrainStep  # noqa: F401,E402
 from .ddp import FlatDataParallel  # noqa: F401,E402  (flat-gradient data parallelism for train_dist.py-style loops)
 from . import scene  # noqa: F401,E402  (whole-scene front end: build_segments, refine_scene)
+from . import data  # noqa: F401,E402  (SceneTrainingSet: shuffled training batches from device-resident scenes)
 
-__all__ = ["FlatDataParallel", "GraphedLineRefineNet", "GraphedTrainStep", "LineRefineNet", "MultiScalePointNetEncoder", "PositionalEncoding", "DetrTransformerDecoderLayer", "ops", "scene"]
+__all__ = ["FlatDataParallel", "GraphedLineRefineNet", "GraphedTrainStep", "LineRefineNet", "MultiScalePointNetEncoder", "PositionalEncoding", "DetrTransformerDecoderLayer", "ops", "scene", "data"]

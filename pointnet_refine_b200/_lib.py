@@ -77,6 +77,9 @@ SIGNATURES = {
     "lrn_scene_workspace_bytes": (sz, [ci, i64]),
     "lrn_scene_segments": (ci, [vp, i64, vp, vp, vp, vp, vp, ci, ci, f64, f64, f64, u64, i64, vp, vp, vp, vp, vp, sz, vp]),
     "lrn_scene_resample": (ci, [vp, vp, ci, ci, vp, vp, vp, vp, vp]),
+    "lrn_scenes_workspace_bytes": (sz, [ci, ci, i64]),
+    "lrn_scenes_segments": (ci, [vp, vp, ci, i64, vp, vp, vp, vp, vp, vp, vp, vp, ci, ci, f64, f64, f64, i64, vp, vp, vp, vp, vp, sz,
+                                 vp]),
     "lrn_adam_step": (ci, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, i64, vp]),
     "lrn_adam_step_capturable": (ci, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, vp, vp]),
     "lrn_l1_deep_supervision": (ci, [vp, vp, ci, i64, vp, vp, vp]),
@@ -106,6 +109,9 @@ def _load():
     if lib.lrn_abi_version() != ABI_VERSION:
         raise RuntimeError(f"liblrn_b200.so has ABI version {lib.lrn_abi_version()}, this package binds version {ABI_VERSION}; rebuild it "
                            "(python pointnet_refine_b200/build.py --force)")
+    missing = [name for name in SIGNATURES if not hasattr(lib, name)]
+    if missing:   # an older build of the same version (entry points added without a version change, see the header)
+        raise RuntimeError(f"liblrn_b200.so lacks {', '.join(missing)}; rebuild it (python pointnet_refine_b200/build.py --force)")
     for name, (restype, argtypes) in SIGNATURES.items():
         fn = getattr(lib, name)
         fn.restype, fn.argtypes = restype, argtypes

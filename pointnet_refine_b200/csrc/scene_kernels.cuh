@@ -70,6 +70,83 @@ __device__ __forceinline__ uint64_t double_to_sortable(double d) {
   return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
 
+// ------------------------------------------------------------------------------------------------ one scene or many
+// Where line l's points and RNG identity come from.  lrn_scene_segments: one scene, (seed, l).  lrn_scenes_segments
+// (scene_off != null): the points of scene line_scene[l], starting at scene_off[line_scene[l]], and (seeds[l],
+// line_ids[l]).  Scene indices (candidates, `indices`, the RNG counter) are always within the line's own scene.
+struct Lines {
+  const long long* scene_off;  // (K+1) first point of every scene, or null
+  const int* line_scene;       // (L)
+  const uint64_t* seeds;       // (L)
+  const uint32_t* line_ids;    // (L)
+  uint64_t seed;
+  int K;
+  __device__ __forceinline__ bool bad(int l) const {
+    return scene_off && static_cast<unsigned>(line_scene[l]) >= static_cast<unsigned>(K);
+  }
+  __device__ __forceinline__ long long base(int l) const { return scene_off ? scene_off[line_scene[l]] : 0; }
+  __device__ __forceinline__ uint64_t seed_of(int l) const { return scene_off ? seeds[l] : seed; }
+  __device__ __forceinline__ uint64_t id_of(int l) const { return scene_off ? static_cast<uint64_t>(line_ids[l]) : static_cast<uint64_t>(l); }
+};
+
+// Lines of a many-scene call grouped by scene (group_kernel): order[first[k] .. first[k+1]) are the lines of scene k, in
+// no particular order (nothing downstream depends on it: per-line counters, candidates sorted before use).
+struct Groups {
+  const long long* scene_off;  // (K+1)
+  const int* first;            // (K+1)
+  const int* order;            // (L)
+  int K;
+};
+
+// largest k in [lo, hi] with off[k] <= i (the scene of point i; an empty scene k has off[k] == off[k+1] and is skipped)
+__device__ __forceinline__ int scene_of(const long long* __restrict__ off, int lo, int hi, long long i) {
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (off[mid] <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// One block: counting sort of the lines by scene.  Lines whose scene is out of range join no group (select_kernel flags
+// them).  Global counters are read back through L2 (__ldcg) after the block's atomics.
+__global__ void __launch_bounds__(1024) group_kernel(const int* __restrict__ line_scene, int L, int K, int* __restrict__ first,
+                                                     int* __restrict__ cursor, int* __restrict__ order) {
+  __shared__ int part[1024];
+  __shared__ int carry;
+  for (int k = threadIdx.x; k < K; k += blockDim.x) cursor[k] = 0;
+  if (threadIdx.x == 0) carry = 0;
+  __syncthreads();
+  for (int l = threadIdx.x; l < L; l += blockDim.x) {
+    const int k = line_scene[l];
+    if (static_cast<unsigned>(k) < static_cast<unsigned>(K)) atomicAdd(&cursor[k], 1);
+  }
+  __syncthreads();
+  for (int b = 0; b < K; b += blockDim.x) {
+    const int k = b + threadIdx.x;
+    const int v = k < K ? __ldcg(cursor + k) : 0;
+    part[threadIdx.x] = v;
+    __syncthreads();
+    for (int o = 1; o < blockDim.x; o <<= 1) {
+      const int t = threadIdx.x >= o ? part[threadIdx.x - o] : 0;
+      __syncthreads();
+      part[threadIdx.x] += t;
+      __syncthreads();
+    }
+    if (k < K) first[k] = carry + part[threadIdx.x] - v;
+    __syncthreads();
+    if (threadIdx.x == blockDim.x - 1) carry += part[threadIdx.x];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) first[K] = carry;
+  __syncthreads();
+  for (int k = threadIdx.x; k < K; k += blockDim.x) cursor[k] = __ldcg(first + k);
+  __syncthreads();
+  for (int l = threadIdx.x; l < L; l += blockDim.x) {
+    const int k = line_scene[l];
+    if (static_cast<unsigned>(k) < static_cast<unsigned>(K)) order[atomicAdd(&cursor[k], 1)] = l;
+  }
+}
+
 // squared distance exactly as the oracle: (dx*dx + dy*dy) + dz*dz in double, no contraction
 __device__ __forceinline__ double dist2_exact(double px, double py, double pz, const double* q) {
   const double dx = __dsub_rn(px, q[0]), dy = __dsub_rn(py, q[1]), dz = __dsub_rn(pz, q[2]);
@@ -204,28 +281,62 @@ __global__ void prep_kernel(const double* __restrict__ dense, int L, float grow,
 // pieces whose box contains it, and the exact double evaluation only inside the band where fp32 cannot decide
 // `distance < radius`.
 // FILL = false: count the candidates of every line (+ intensity range).  FILL = true: write their scene indices.
-template <bool FILL>
+// MANY = true (lrn_scenes_segments): `pts` holds K scenes back to back (grp.scene_off) and a point is tested only against
+// the lines of its own scene (grp.order[grp.first[k] .. grp.first[k+1])); a block whose scenes have no line in the call
+// exits at once.  The candidate written is the point's index within its scene.
+template <bool FILL, bool MANY>
 __global__ void __launch_bounds__(256) tube_crop_kernel(const float4* __restrict__ pts, long long S, int L,
                                                         const float* __restrict__ aabb, const float* __restrict__ dense_f,
                                                         const double* __restrict__ dense, double radius, float r2_lo, float r2_hi,
                                                         int* __restrict__ count, int* __restrict__ imin, int* __restrict__ imax,
                                                         int* __restrict__ fill, const long long* __restrict__ offset,
                                                         long long capacity, const int* __restrict__ perm,
-                                                        uint32_t* __restrict__ cand) {
+                                                        uint32_t* __restrict__ cand, Groups grp) {
   __shared__ float box[kLineTile * 6];
+  __shared__ int line_s[MANY ? kLineTile : 1];
+  __shared__ int s_k0, s_k1;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
   if (i < S) p = pts[i];
   auto inside = [&](const float* b) { return !(p.x < b[0] || p.y < b[1] || p.z < b[2] || p.x > b[3] || p.y > b[4] || p.z > b[5]); };
-  for (int l0 = 0; l0 < L; l0 += kLineTile) {
-    const int nl = min(kLineTile, L - l0);
+  // grouped line positions [g_lo, g_hi) of this block's scenes, [my_lo, my_hi) of this thread's scene
+  int g_lo = 0, g_hi = L, my_lo = 0, my_hi = L;
+  long long base = 0;
+  if constexpr (MANY) {
+    if (threadIdx.x == 0) {
+      const long long b0 = static_cast<long long>(blockIdx.x) * blockDim.x;
+      const long long b1 = min(b0 + static_cast<long long>(blockDim.x), S) - 1;
+      s_k0 = scene_of(grp.scene_off, 0, grp.K - 1, b0);
+      s_k1 = scene_of(grp.scene_off, s_k0, grp.K - 1, b1);
+    }
     __syncthreads();
-    for (int t = threadIdx.x; t < nl * 6; t += blockDim.x) box[t] = aabb[(l0 + t / 6) * kBoxFloats + t % 6];
+    const int k0 = s_k0, k1 = s_k1;
+    g_lo = grp.first[k0];
+    g_hi = grp.first[k1 + 1];
+    if (g_lo >= g_hi) return;  // no line of the call in this block's scenes (uniform over the block)
+    const int k = (k0 == k1 || i >= S) ? k0 : scene_of(grp.scene_off, k0, k1, i);
+    my_lo = grp.first[k];
+    my_hi = grp.first[k + 1];
+    base = grp.scene_off[k];
+  }
+  for (int l0 = g_lo; l0 < g_hi; l0 += kLineTile) {
+    const int nl = min(kLineTile, g_hi - l0);
+    __syncthreads();
+    if constexpr (MANY) {
+      for (int t = threadIdx.x; t < nl; t += blockDim.x) line_s[t] = grp.order[l0 + t];
+      __syncthreads();
+      for (int t = threadIdx.x; t < nl * 6; t += blockDim.x) box[t] = aabb[line_s[t / 6] * kBoxFloats + t % 6];
+    } else {
+      for (int t = threadIdx.x; t < nl * 6; t += blockDim.x) box[t] = aabb[(l0 + t / 6) * kBoxFloats + t % 6];
+    }
     __syncthreads();
     if (i >= S) continue;
     for (int j = 0; j < nl; ++j) {
+      if constexpr (MANY) {
+        if (l0 + j < my_lo || l0 + j >= my_hi) continue;
+      }
       if (!inside(box + j * 6)) continue;
-      const int l = l0 + j;
+      const int l = MANY ? line_s[j] : l0 + j;
       const float* sb = aabb + l * kBoxFloats + 6;
       const float* q = dense_f + static_cast<size_t>(l) * kDense * 3;
       float best = 3.4e38f;
@@ -257,7 +368,7 @@ __global__ void __launch_bounds__(256) tube_crop_kernel(const float4* __restrict
         atomicMax(&imax[l], o);
       } else {
         const long long pos = offset[l] + atomicAdd(&fill[l], 1);
-        if (pos < capacity) cand[pos] = perm ? static_cast<uint32_t>(perm[i]) : static_cast<uint32_t>(i);
+        if (pos < capacity) cand[pos] = perm ? static_cast<uint32_t>(perm[i]) : static_cast<uint32_t>(i - base);
       }
     }
   }
@@ -299,11 +410,13 @@ __global__ void scan_kernel(const int* __restrict__ count, int L, long long capa
 __global__ void __launch_bounds__(256) sample_keys_kernel(const float4* __restrict__ pts, const double* __restrict__ line32,
                                                           const int* __restrict__ count, const long long* __restrict__ offset,
                                                           const int* __restrict__ imin, const int* __restrict__ imax, int N,
-                                                          double decay, uint64_t seed, const long long* __restrict__ status,
+                                                          double decay, Lines src, const long long* __restrict__ status,
                                                           const uint32_t* __restrict__ cand, uint64_t* __restrict__ keys) {
   const int l = blockIdx.y;
   const int n = count[l];
   if (n <= N || status[1]) return;
+  pts += src.base(l);
+  const uint64_t seed = src.seed_of(l), line = src.id_of(l);
   __shared__ double lp[kLine * 3];
   for (int t = threadIdx.x; t < kLine * 3; t += blockDim.x) lp[t] = line32[static_cast<size_t>(l) * kLine * 3 + t];
   __syncthreads();
@@ -320,7 +433,7 @@ __global__ void __launch_bounds__(256) sample_keys_kernel(const float4* __restri
     const float norm = hi > lo ? __fdiv_rn(__fsub_rn(p.w, lo), span) : 0.5f;
     const float iw = __fadd_rn(0.5f, norm);
     const double w = __dmul_rn(det_exp(__ddiv_rn(-d, decay)), static_cast<double>(iw));
-    const double key = __ddiv_rn(det_log(det_uniform(seed, l, idx)), w);
+    const double key = __ddiv_rn(det_log(det_uniform(seed, line, idx)), w);
     keys[off + c] = double_to_sortable(key);
   }
 }
@@ -358,7 +471,7 @@ __device__ void bitonic_sort(uint64_t* k, uint32_t* v, int n /* power of two */)
 //   count  > N      : the N largest keys (radix select + sort)         (src/dataset.py:128, RNG contract)
 __global__ void __launch_bounds__(256) select_kernel(const float4* __restrict__ pts, const double* __restrict__ centers,
                                                      const int* __restrict__ count, const long long* __restrict__ offset, int N,
-                                                     int cap /* power of two >= 2 N */, uint64_t seed,
+                                                     int cap /* power of two >= 2 N */, Lines src,
                                                      long long* __restrict__ status, const uint32_t* __restrict__ cand,
                                                      const uint64_t* __restrict__ keys, float* __restrict__ context,
                                                      long long* __restrict__ indices, int* __restrict__ counts_out) {
@@ -371,7 +484,13 @@ __global__ void __launch_bounds__(256) select_kernel(const float4* __restrict__ 
   const int l = blockIdx.x;
   const int n = count[l];
   if (threadIdx.x == 0) counts_out[l] = n;
+  if (src.bad(l)) {  // scene number out of range: the line joined no group; reported, nothing written
+    if (threadIdx.x == 0) atomicOr(reinterpret_cast<unsigned long long*>(&status[1]), 4ull);
+    return;
+  }
   if (status[1] & 1) return;  // candidate buffer too small: the host re-runs with status[0] entries
+  pts += src.base(l);
+  const uint64_t seed = src.seed_of(l), line = src.id_of(l);
   const long long off = offset[l];
   const double cx = centers[l * 3], cy = centers[l * 3 + 1], cz = centers[l * 3 + 2];
   float* ctx = context + static_cast<size_t>(l) * N * 4;
@@ -388,7 +507,7 @@ __global__ void __launch_bounds__(256) select_kernel(const float4* __restrict__ 
       long long idx = -1;
       float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
       if (n > 0) {
-        const double u = det_uniform(seed, l, (1ull << 40) + j);
+        const double u = det_uniform(seed, line, (1ull << 40) + j);
         long long pick = static_cast<long long>(__dmul_rn(u, static_cast<double>(n)));
         pick = pick < n - 1 ? pick : n - 1;
         idx = sv[pick];
