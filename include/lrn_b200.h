@@ -34,8 +34,10 @@ extern "C" {
  * 3: lrn_launch_count added; later, without a version change, lrn_scenes_segments / lrn_scenes_workspace_bytes (lines of
  *    many scenes in one call).  Those are additions only: every entry point above keeps its signature and its results,
  *    so a caller built against an earlier version-3 library runs unchanged, and a caller that needs the additions finds
- *    them missing by name when it loads an older library (pointnet_refine_b200/_lib.py reports which). */
-#define LRN_ABI_VERSION 3
+ *    them missing by name when it loads an older library (pointnet_refine_b200/_lib.py reports which).
+ * 4: the per-scene segment builder and its workspace-size function removed: the lines of one scene are the K = 1 case
+ *    of lrn_scenes_segments, which gives the same bits. */
+#define LRN_ABI_VERSION 4
 
 typedef struct CUstream_st* lrn_stream_t; /* == cudaStream_t */
 
@@ -251,23 +253,6 @@ int lrn_ctx_attention(const void* qfold, const void* kp, int64_t ld_kp, const vo
 int lrn_pos_hidden(const float* w1, const float* b1, const float* context, int64_t P, void* out, int64_t ld_out,
                    lrn_stream_t stream);
 
-/* Scene preprocessing for all L lines of one scene (SURVEY.md 8f row 3): the tube crop, weighted sampling and centroid
- * normalisation of LaneRefineDataset.__getitem__ steps 4-6 (src/dataset.py:214-237, weighted_sampling :78-130) and of
- * process_single_line (inference_whole_scene.py:95-121), which the reference runs on the host with one KD-tree per line.
- *   scene     (S, 4) fp32 [x, y, z, intensity] device        dense200 (L, 200, 3) f64: resample_polyline(raw, 200)
- *   line32    (L, 32, 3) f64: resample_polyline(raw, 32)      centers  (L, 3) f64: mean of the 32 points
- *   context   (L, N, 4) fp32 out: sampled points, xyz - center (float64 subtraction, rounded once), intensity
- *   indices   (L, N) int64 out: scene index of every sample (-1: the zero points of an empty crop)
- *   counts    (L) int32 out: points inside the tube (distance to the 200-point polyline < crop_radius, float64 compare)
- *   status    (2) int64 out: [0] total candidates, [1] bit 0: `capacity` < [0] -> nothing was sampled, call again with
- *             capacity >= status[0]; bit 1: more than 2^k - N candidates tie exactly at a line's threshold key
- *   scene_sorted / perm: optional (both or neither): the same points in a spatially coherent order (e.g. Morton order of
- *             x, y) with perm[i] = scene index of scene_sorted[i]; the crop then walks this copy, so that the 32 points of a
- *             warp are neighbours and only enter the tests of the lines that pass near them.  Results are identical.
- *   coord_extent: largest |coordinate| of the scene (sizes the band in which the fp32 pre-filter defers to float64)
- * The draw follows the RNG contract documented in oracle/scene_oracle.py (counter-based hash of seed, line, scene index;
- * Efraimidis-Spirakis keys; samples in descending key order): same distribution as the reference's
- * np.random.choice(replace=False, p), reproducible and independent of thread order.  N <= 4096, L <= 65535. */
 /* Parameter gradients of lrn_pos_hidden (train mode): d_w1 (256,3), d_b1 (256) fp32 (zeroed here) from the bf16 hidden
  * activations (ReLU mask) and their bf16 gradient, both (P, 256) with row pitches in elements. */
 int lrn_pos_hidden_backward(const float* context, int64_t P, const void* hidden, int64_t ld_hidden, const void* d_hidden,
@@ -279,31 +264,37 @@ int lrn_pos_hidden_backward(const float* context, int64_t P, const void* hidden,
  * (src/dataset.py:232-237).  A polyline with fewer than two vertices gives zeros; at most 2048 vertices per line. */
 int lrn_scene_resample(const double* vertices, const int64_t* offsets, int L, int max_vertices, double* line32, double* dense200,
                        double* centers, float* noisy_centered, lrn_stream_t stream);
-size_t lrn_scene_workspace_bytes(int L, int64_t capacity);
-int lrn_scene_segments(const float* scene, int64_t S, const float* scene_sorted, const int32_t* perm, const double* dense200, const double* line32, const double* centers,
-                       int L, int N, double crop_radius, double decay_scale, double coord_extent, uint64_t seed, int64_t capacity,
-                       float* context, int64_t* indices, int32_t* counts, int64_t* status, void* workspace, size_t workspace_bytes,
-                       lrn_stream_t stream);
-
-/* lrn_scene_segments for lines of MANY scenes in one call (training batches that mix scenes, a whole drive at inference).
- *   points    (S_total, 4) fp32: K scenes back to back; scene_offsets (K+1) int64 device: scene k is
- *             points[scene_offsets[k] .. scene_offsets[k+1])
- *   sorted_points / perm: optional (both or neither): every scene's spatially sorted copy, concatenated the same way, with
- *             perm[scene_offsets[k] + i] = index WITHIN scene k of sorted_points[scene_offsets[k] + i]
+/* Scene preprocessing for L lines of K scenes in one call (SURVEY.md 8f row 3): the tube crop, weighted sampling and
+ * centroid normalisation of LaneRefineDataset.__getitem__ steps 4-6 (src/dataset.py:214-237, weighted_sampling :78-130)
+ * and of process_single_line (inference_whole_scene.py:95-121), which the reference runs on the host with one KD-tree per
+ * line.  The lines of one scene are the case K = 1; lines of many scenes serve training batches that mix scenes and a
+ * whole drive at inference.
+ *   points    (S_total, 4) fp32 [x, y, z, intensity] device: K scenes back to back
+ *   scene_offsets (K+1) int64 device: scene k is points[scene_offsets[k] .. scene_offsets[k+1])
  *   line_scene (L) int32: scene of every line, in the caller's order (lines of different scenes may be interleaved)
- *   dense200, line32, centers: per line as for lrn_scene_segments (lrn_scene_resample)
+ *   dense200  (L, 200, 3) f64: resample_polyline(raw, 200)    line32  (L, 32, 3) f64: resample_polyline(raw, 32)
+ *   centers   (L, 3) f64: mean of the 32 points                (all three as lrn_scene_resample writes them)
  *   seeds (L) uint64, line_ids (L) uint32: the RNG identity of every line
- *   context (L, N, 4), indices (L, N), counts (L): in the caller's line order; indices are WITHIN the line's scene (-1: the
- *             zero points of an empty crop), exactly what lrn_scene_segments returns for that scene
- *   status    (2) int64 out: as for lrn_scene_segments (one status for the whole call), plus [1] bit 2: some line_scene[l] is
- *             not in [0, K) (that line's outputs are not written)
+ *   context   (L, N, 4) fp32 out: sampled points, xyz - center (float64 subtraction, rounded once), intensity
+ *   indices   (L, N) int64 out: index WITHIN the line's scene of every sample (-1: the zero points of an empty crop)
+ *   counts    (L) int32 out: points inside the tube (distance to the 200-point polyline < crop_radius, float64 compare)
+ *             (context, indices and counts in the caller's line order)
+ *   status    (2) int64 out, one for the whole call: [0] total candidates, [1] bit 0: `capacity` < [0] -> nothing was
+ *             sampled, call again with capacity >= status[0]; bit 1: more than 2^k - N candidates tie exactly at a line's
+ *             threshold key; bit 2: some line_scene[l] is not in [0, K) (that line's outputs are not written)
+ *   sorted_points / perm: optional (both or neither): every scene's points in a spatially coherent order (e.g. Morton order
+ *             of x, y), concatenated as `points`, with perm[scene_offsets[k] + i] = index WITHIN scene k of
+ *             sorted_points[scene_offsets[k] + i]; the crop then walks this copy, so that the 32 points of a warp are
+ *             neighbours and only enter the tests of the lines that pass near them.  Results are identical.
  *   coord_extent: largest |coordinate| over the scenes and lines of the call.  It only sizes the band in which the fp32
  *             pre-filter defers to float64; the crop decision itself is exact for any extent at least that large (inside
  *             the band the distance is evaluated in double), so one extent per call gives the per-scene results.
- * RNG identity: the draw of line l is the RNG contract of oracle/scene_oracle.py with (seed, line, scene index) =
- * (seeds[l], line_ids[l], index within scene line_scene[l]), i.e. scene_oracle.build_segment(scene_k, raw, N, r, decay,
- * seeds[l], line_ids[l]).  lrn_scene_segments over the lines of one scene is the case seeds[l] = seed, line_ids[l] = position
- * of l among that scene's lines, and gives the same bits.
+ *   workspace at least lrn_scenes_workspace_bytes(L, K, capacity) bytes, 256-byte aligned; points / context 16-byte aligned
+ * RNG: the draw of line l follows the RNG contract documented in oracle/scene_oracle.py (counter-based hash of seed, line,
+ * scene index; Efraimidis-Spirakis keys; samples in descending key order) with (seed, line, scene index) = (seeds[l],
+ * line_ids[l], index within scene line_scene[l]), i.e. scene_oracle.build_segment(scene_k, raw, N, r, decay, seeds[l],
+ * line_ids[l]): same distribution as the reference's np.random.choice(replace=False, p), reproducible and independent of
+ * thread order and of which lines share the call.
  * One pass: each point is tested only against the lines of its own scene; blocks of scenes without a line exit at once.
  * Launches per call are independent of K.  S_total < 2^31, K <= 65535, L <= 65535, N <= 4096 (else LRN_ERR_BAD_SHAPE). */
 size_t lrn_scenes_workspace_bytes(int L, int K, int64_t capacity);

@@ -16,7 +16,7 @@ CSRC = os.path.join(_HERE, "csrc")
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "lrn_b200.h")
 
 # enums of include/lrn_b200.h
-ABI_VERSION = 3      # LRN_ABI_VERSION
+ABI_VERSION = 4      # LRN_ABI_VERSION
 LRN_OK = 0
 PREC_BF16, PREC_TF32, PREC_FP32X3 = 0, 1, 2
 OUT_POOL, OUT_ARGMAX, OUT_FUSED, OUT_MEMORY, OUT_MEMORY_BF16 = 1, 2, 4, 8, 16
@@ -74,8 +74,6 @@ SIGNATURES = {
     "lrn_ctx_attention": (ci, [vp, vp, i64, vp, i64, ci, ci, ci, vp, ci, vp, vp]),
     "lrn_pos_hidden": (ci, [vp, vp, vp, i64, vp, i64, vp]),
     "lrn_pos_hidden_backward": (ci, [vp, i64, vp, i64, vp, i64, vp, vp, vp]),
-    "lrn_scene_workspace_bytes": (sz, [ci, i64]),
-    "lrn_scene_segments": (ci, [vp, i64, vp, vp, vp, vp, vp, ci, ci, f64, f64, f64, u64, i64, vp, vp, vp, vp, vp, sz, vp]),
     "lrn_scene_resample": (ci, [vp, vp, ci, ci, vp, vp, vp, vp, vp]),
     "lrn_scenes_workspace_bytes": (sz, [ci, ci, i64]),
     "lrn_scenes_segments": (ci, [vp, vp, ci, i64, vp, vp, vp, vp, vp, vp, vp, vp, ci, ci, f64, f64, f64, i64, vp, vp, vp, vp, vp, sz,

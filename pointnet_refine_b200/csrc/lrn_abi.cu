@@ -764,8 +764,8 @@ namespace {
 struct SceneLayout {
   size_t aabb, dense_f, count, fill, imin, imax, offset, cand, keys, first, cursor, order, total;
 };
-// K > 0: the many-scene call's line grouping (first (K+1), cursor (K), order (L) ints) follows the per-line arrays
-SceneLayout scene_layout(int L, int64_t capacity, int K = 0) {
+// the line grouping by scene (first (K+1), cursor (K), order (L) ints) follows the per-line arrays
+SceneLayout scene_layout(int L, int64_t capacity, int K) {
   SceneLayout w{};
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
@@ -778,11 +778,9 @@ SceneLayout scene_layout(int L, int64_t capacity, int K = 0) {
   w.offset = take(size_t(L + 1) * 8);
   w.cand = take(size_t(capacity) * 4);
   w.keys = take(size_t(capacity) * 8);
-  if (K > 0) {
-    w.first = take(size_t(K + 1) * 4);
-    w.cursor = take(size_t(K) * 4);
-    w.order = take(size_t(L) * 4);
-  }
+  w.first = take(size_t(K + 1) * 4);
+  w.cursor = take(size_t(K) * 4);
+  w.order = take(size_t(L) * 4);
   w.total = off;
   return w;
 }
@@ -803,25 +801,30 @@ int lrn_scene_resample(const double* vertices, const int64_t* offsets, int L, in
                 dense200, centers, noisy_centered);
 }
 
-size_t lrn_scene_workspace_bytes(int L, int64_t capacity) {
-  if (L <= 0 || capacity <= 0) return 0;
-  return scene_layout(L, capacity).total;
+size_t lrn_scenes_workspace_bytes(int L, int K, int64_t capacity) {
+  if (L <= 0 || K <= 0 || capacity <= 0) return 0;
+  return scene_layout(L, capacity, K).total;
 }
 
-namespace {
-// Validation shared by both scene entry points, then prep / count / scan / fill / keys / select (grp.first != null: the
-// many-scene crop, after the lines are grouped by scene).
-int scene_pipeline(const float* scene_pts, int64_t S, const float* scene_sorted, const int32_t* perm, const double* dense200,
-                   const double* line32, const double* centers, int L, int N, double crop_radius, double decay_scale,
-                   double coord_extent, int64_t capacity, float* context, int64_t* indices, int32_t* counts, int64_t* status,
-                   void* workspace, size_t workspace_bytes, scene::Lines src, const int32_t* line_scene, lrn_stream_t stream) {
-  const int K = src.K;
+// group / prep / count / scan / fill / keys / select
+int lrn_scenes_segments(const float* points, const int64_t* scene_offsets, int K, int64_t S_total, const float* sorted_points,
+                        const int32_t* perm, const int32_t* line_scene, const double* dense200, const double* line32,
+                        const double* centers, const uint64_t* seeds, const uint32_t* line_ids, int L, int N, double crop_radius,
+                        double decay_scale, double coord_extent, int64_t capacity, float* context, int64_t* indices, int32_t* counts,
+                        int64_t* status, void* workspace, size_t workspace_bytes, lrn_stream_t stream) {
+  if (!points || !scene_offsets || !line_scene || !dense200 || !line32 || !centers || !seeds || !line_ids || !context || !indices ||
+      !counts || !status || !workspace)
+    return fail(LRN_ERR_BAD_ARG, "null pointer");
+  if (S_total <= 0 || S_total >= (int64_t(1) << 31) || K <= 0 || K > 65535 || L <= 0 || L > 65535 || N <= 0 || N > 4096 ||
+      capacity <= 0)
+    return fail(LRN_ERR_BAD_SHAPE, "S_total=%lld K=%d L=%d N=%d capacity=%lld (S_total < 2^31, K <= 65535, L <= 65535, N <= 4096)",
+                (long long)S_total, K, L, N, (long long)capacity);
   if (!(crop_radius > 0) || !(decay_scale > 0) || !(coord_extent >= 0) ||
       (crop_radius + 2.0) / decay_scale > 25.0)
     return fail(LRN_ERR_BAD_ARG, "crop_radius=%g decay_scale=%g: (radius + 2) / decay must stay <= 25 (weights must not underflow)",
                 crop_radius, decay_scale);
-  if (misaligned(16, scene_pts, context) || misaligned(256, workspace))
-    return fail(LRN_ERR_MISALIGNED, "scene / context need 16-byte, workspace 256-byte alignment");
+  if (misaligned(16, points, context) || misaligned(256, workspace))
+    return fail(LRN_ERR_MISALIGNED, "points / context need 16-byte, workspace 256-byte alignment");
   const SceneLayout w = scene_layout(L, capacity, K);
   if (workspace_bytes < w.total) return fail(LRN_ERR_WORKSPACE, "workspace %zu < %zu bytes", workspace_bytes, w.total);
   LRN_DEVICE(dev);
@@ -835,31 +838,31 @@ int scene_pipeline(const float* scene_pts, int64_t S, const float* scene_sorted,
   long long* offset = reinterpret_cast<long long*>(ws + w.offset);
   uint32_t* cand = reinterpret_cast<uint32_t*>(ws + w.cand);
   uint64_t* keys = reinterpret_cast<uint64_t*>(ws + w.keys);
+  int* first = reinterpret_cast<int*>(ws + w.first);
+  int* order = reinterpret_cast<int*>(ws + w.order);
   long long* stat = reinterpret_cast<long long*>(status);
   // fp32 pre-filter: decides `distance < radius` outside a band of +-eps, the band is evaluated in double
   const double eps = 1e-3 + 4e-6 * coord_extent;
   const double rlo = std::max(crop_radius - eps, 0.0), rhi = crop_radius + eps;
   const float r2_lo = float(rlo * rlo * (1.0 - 1e-6)), r2_hi = float(rhi * rhi * (1.0 + 1e-6));
-  const float4* pts = reinterpret_cast<const float4*>(scene_pts);
-  if ((scene_sorted != nullptr) != (perm != nullptr)) return fail(LRN_ERR_BAD_ARG, "scene_sorted and perm come together");
-  if (misaligned(16, scene_sorted)) return fail(LRN_ERR_MISALIGNED, "scene_sorted needs 16-byte alignment");
-  const float4* crop_pts = scene_sorted ? reinterpret_cast<const float4*>(scene_sorted) : pts;
-  scene::Groups grp{};
-  if (K > 0) {
-    grp = scene::Groups{src.scene_off, reinterpret_cast<int*>(ws + w.first), reinterpret_cast<int*>(ws + w.order), K};
-    LRN_TRY(launch(scene::group_kernel, 1, 1024, 0, stream, line_scene, L, K, reinterpret_cast<int*>(ws + w.first),
-                   reinterpret_cast<int*>(ws + w.cursor), reinterpret_cast<int*>(ws + w.order)));
-  }
+  const float4* pts = reinterpret_cast<const float4*>(points);
+  if ((sorted_points != nullptr) != (perm != nullptr)) return fail(LRN_ERR_BAD_ARG, "sorted_points and perm come together");
+  if (misaligned(16, sorted_points)) return fail(LRN_ERR_MISALIGNED, "sorted_points needs 16-byte alignment");
+  const float4* crop_pts = sorted_points ? reinterpret_cast<const float4*>(sorted_points) : pts;
+  const long long* scene_off = reinterpret_cast<const long long*>(scene_offsets);
+  const scene::Lines src{scene_off, line_scene, seeds, line_ids, K};
+  const scene::Groups grp{scene_off, first, order, K};
+  LRN_TRY(launch(scene::group_kernel, 1, 1024, 0, stream, line_scene, L, K, first, reinterpret_cast<int*>(ws + w.cursor), order));
   LRN_TRY(launch(scene::prep_kernel, L, 128, 0, stream, dense200, L, float(rhi * (1.0 + 1e-6)), aabb, dense_f, count, fill, imin,
                  imax));
-  const int grid = int((S + 255) / 256);
+  const int grid = int((S_total + 255) / 256);
   auto crop = [&](auto kernel) {
-    return launch(kernel, grid, 256, 0, stream, crop_pts, S, L, aabb, dense_f, dense200, crop_radius, r2_lo, r2_hi, count, imin,
+    return launch(kernel, grid, 256, 0, stream, crop_pts, S_total, aabb, dense_f, dense200, crop_radius, r2_lo, r2_hi, count, imin,
                   imax, fill, offset, capacity, perm, cand, grp);
   };
-  LRN_TRY(K > 0 ? crop(scene::tube_crop_kernel<false, true>) : crop(scene::tube_crop_kernel<false, false>));
+  LRN_TRY(crop(scene::tube_crop_kernel<false>));
   LRN_TRY(launch(scene::scan_kernel, 1, 1024, 0, stream, count, L, capacity, offset, stat));
-  LRN_TRY(K > 0 ? crop(scene::tube_crop_kernel<true, true>) : crop(scene::tube_crop_kernel<true, false>));
+  LRN_TRY(crop(scene::tube_crop_kernel<true>));
   LRN_TRY(launch(scene::sample_keys_kernel, dim3(32, L), 256, 0, stream, pts, line32, count, offset, imin, imax, N, decay_scale,
                  src, stat, cand, keys));
   const int cap = scene_cap(N);
@@ -868,43 +871,6 @@ int scene_pipeline(const float* scene_pts, int64_t S, const float* scene_sorted,
   LRN_CUDA(cudaFuncSetAttribute(scene::select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   return launch(scene::select_kernel, L, 256, smem, stream, pts, centers, count, offset, N, cap, src, stat, cand, keys, context,
                 reinterpret_cast<long long*>(indices), counts);
-}
-}  // namespace
-
-int lrn_scene_segments(const float* scene_pts, int64_t S, const float* scene_sorted, const int32_t* perm, const double* dense200, const double* line32, const double* centers,
-                       int L, int N, double crop_radius, double decay_scale, double coord_extent, uint64_t seed, int64_t capacity,
-                       float* context, int64_t* indices, int32_t* counts, int64_t* status, void* workspace, size_t workspace_bytes,
-                       lrn_stream_t stream) {
-  if (!scene_pts || !dense200 || !line32 || !centers || !context || !indices || !counts || !status || !workspace)
-    return fail(LRN_ERR_BAD_ARG, "null pointer");
-  if (S <= 0 || S >= (int64_t(1) << 31) || L <= 0 || L > 65535 || N <= 0 || N > 4096 || capacity <= 0)
-    return fail(LRN_ERR_BAD_SHAPE, "S=%lld L=%d N=%d capacity=%lld (S < 2^31, L <= 65535, N <= 4096)", (long long)S, L, N, (long long)capacity);
-  const scene::Lines src{nullptr, nullptr, nullptr, nullptr, seed, 0};
-  return scene_pipeline(scene_pts, S, scene_sorted, perm, dense200, line32, centers, L, N, crop_radius, decay_scale, coord_extent,
-                        capacity, context, indices, counts, status, workspace, workspace_bytes, src, nullptr, stream);
-}
-
-size_t lrn_scenes_workspace_bytes(int L, int K, int64_t capacity) {
-  if (L <= 0 || K <= 0 || capacity <= 0) return 0;
-  return scene_layout(L, capacity, K).total;
-}
-
-int lrn_scenes_segments(const float* points, const int64_t* scene_offsets, int K, int64_t S_total, const float* sorted_points,
-                        const int32_t* perm, const int32_t* line_scene, const double* dense200, const double* line32,
-                        const double* centers, const uint64_t* seeds, const uint32_t* line_ids, int L, int N, double crop_radius,
-                        double decay_scale, double coord_extent, int64_t capacity, float* context, int64_t* indices, int32_t* counts,
-                        int64_t* status, void* workspace, size_t workspace_bytes, lrn_stream_t stream) {
-  if (!points || !scene_offsets || !line_scene || !dense200 || !line32 || !centers || !seeds || !line_ids || !context || !indices ||
-      !counts || !status || !workspace)
-    return fail(LRN_ERR_BAD_ARG, "null pointer");
-  if (S_total <= 0 || S_total >= (int64_t(1) << 31) || K <= 0 || K > 65535 || L <= 0 || L > 65535 || N <= 0 || N > 4096 ||
-      capacity <= 0)
-    return fail(LRN_ERR_BAD_SHAPE, "S_total=%lld K=%d L=%d N=%d capacity=%lld (S_total < 2^31, K <= 65535, L <= 65535, N <= 4096)",
-                (long long)S_total, K, L, N, (long long)capacity);
-  const scene::Lines src{reinterpret_cast<const long long*>(scene_offsets), line_scene, seeds, line_ids, 0, K};
-  return scene_pipeline(points, S_total, sorted_points, perm, dense200, line32, centers, L, N, crop_radius, decay_scale,
-                        coord_extent, capacity, context, indices, counts, status, workspace, workspace_bytes, src, line_scene,
-                        stream);
 }
 
 int lrn_debug_timeline(long long* device_buffer) {

@@ -70,26 +70,23 @@ __device__ __forceinline__ uint64_t double_to_sortable(double d) {
   return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
 
-// ------------------------------------------------------------------------------------------------ one scene or many
-// Where line l's points and RNG identity come from.  lrn_scene_segments: one scene, (seed, l).  lrn_scenes_segments
-// (scene_off != null): the points of scene line_scene[l], starting at scene_off[line_scene[l]], and (seeds[l],
-// line_ids[l]).  Scene indices (candidates, `indices`, the RNG counter) are always within the line's own scene.
+// ------------------------------------------------------------------------------------------------ scenes and lines
+// Where line l's points and RNG identity come from: the points of scene line_scene[l], starting at
+// scene_off[line_scene[l]], and (seeds[l], line_ids[l]).  Scene indices (candidates, `indices`, the RNG counter) are
+// always within the line's own scene.  One scene is the case K = 1.
 struct Lines {
-  const long long* scene_off;  // (K+1) first point of every scene, or null
+  const long long* scene_off;  // (K+1) first point of every scene
   const int* line_scene;       // (L)
   const uint64_t* seeds;       // (L)
   const uint32_t* line_ids;    // (L)
-  uint64_t seed;
   int K;
-  __device__ __forceinline__ bool bad(int l) const {
-    return scene_off && static_cast<unsigned>(line_scene[l]) >= static_cast<unsigned>(K);
-  }
-  __device__ __forceinline__ long long base(int l) const { return scene_off ? scene_off[line_scene[l]] : 0; }
-  __device__ __forceinline__ uint64_t seed_of(int l) const { return scene_off ? seeds[l] : seed; }
-  __device__ __forceinline__ uint64_t id_of(int l) const { return scene_off ? static_cast<uint64_t>(line_ids[l]) : static_cast<uint64_t>(l); }
+  __device__ __forceinline__ bool bad(int l) const { return static_cast<unsigned>(line_scene[l]) >= static_cast<unsigned>(K); }
+  __device__ __forceinline__ long long base(int l) const { return scene_off[line_scene[l]]; }
+  __device__ __forceinline__ uint64_t seed_of(int l) const { return seeds[l]; }
+  __device__ __forceinline__ uint64_t id_of(int l) const { return static_cast<uint64_t>(line_ids[l]); }
 };
 
-// Lines of a many-scene call grouped by scene (group_kernel): order[first[k] .. first[k+1]) are the lines of scene k, in
+// The lines of a call grouped by scene (group_kernel): order[first[k] .. first[k+1]) are the lines of scene k, in
 // no particular order (nothing downstream depends on it: per-line counters, candidates sorted before use).
 struct Groups {
   const long long* scene_off;  // (K+1)
@@ -281,11 +278,11 @@ __global__ void prep_kernel(const double* __restrict__ dense, int L, float grow,
 // pieces whose box contains it, and the exact double evaluation only inside the band where fp32 cannot decide
 // `distance < radius`.
 // FILL = false: count the candidates of every line (+ intensity range).  FILL = true: write their scene indices.
-// MANY = true (lrn_scenes_segments): `pts` holds K scenes back to back (grp.scene_off) and a point is tested only against
-// the lines of its own scene (grp.order[grp.first[k] .. grp.first[k+1])); a block whose scenes have no line in the call
-// exits at once.  The candidate written is the point's index within its scene.
-template <bool FILL, bool MANY>
-__global__ void __launch_bounds__(256) tube_crop_kernel(const float4* __restrict__ pts, long long S, int L,
+// `pts` holds K scenes back to back (grp.scene_off) and a point is tested only against the lines of its own scene
+// (grp.order[grp.first[k] .. grp.first[k+1])); a block whose scenes have no line in the call exits at once.  The
+// candidate written is the point's index within its scene.
+template <bool FILL>
+__global__ void __launch_bounds__(256) tube_crop_kernel(const float4* __restrict__ pts, long long S,
                                                         const float* __restrict__ aabb, const float* __restrict__ dense_f,
                                                         const double* __restrict__ dense, double radius, float r2_lo, float r2_hi,
                                                         int* __restrict__ count, int* __restrict__ imin, int* __restrict__ imax,
@@ -293,50 +290,37 @@ __global__ void __launch_bounds__(256) tube_crop_kernel(const float4* __restrict
                                                         long long capacity, const int* __restrict__ perm,
                                                         uint32_t* __restrict__ cand, Groups grp) {
   __shared__ float box[kLineTile * 6];
-  __shared__ int line_s[MANY ? kLineTile : 1];
+  __shared__ int line_s[kLineTile];
   __shared__ int s_k0, s_k1;
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
   if (i < S) p = pts[i];
   auto inside = [&](const float* b) { return !(p.x < b[0] || p.y < b[1] || p.z < b[2] || p.x > b[3] || p.y > b[4] || p.z > b[5]); };
-  // grouped line positions [g_lo, g_hi) of this block's scenes, [my_lo, my_hi) of this thread's scene
-  int g_lo = 0, g_hi = L, my_lo = 0, my_hi = L;
-  long long base = 0;
-  if constexpr (MANY) {
-    if (threadIdx.x == 0) {
-      const long long b0 = static_cast<long long>(blockIdx.x) * blockDim.x;
-      const long long b1 = min(b0 + static_cast<long long>(blockDim.x), S) - 1;
-      s_k0 = scene_of(grp.scene_off, 0, grp.K - 1, b0);
-      s_k1 = scene_of(grp.scene_off, s_k0, grp.K - 1, b1);
-    }
-    __syncthreads();
-    const int k0 = s_k0, k1 = s_k1;
-    g_lo = grp.first[k0];
-    g_hi = grp.first[k1 + 1];
-    if (g_lo >= g_hi) return;  // no line of the call in this block's scenes (uniform over the block)
-    const int k = (k0 == k1 || i >= S) ? k0 : scene_of(grp.scene_off, k0, k1, i);
-    my_lo = grp.first[k];
-    my_hi = grp.first[k + 1];
-    base = grp.scene_off[k];
+  if (threadIdx.x == 0) {
+    const long long b0 = static_cast<long long>(blockIdx.x) * blockDim.x;
+    const long long b1 = min(b0 + static_cast<long long>(blockDim.x), S) - 1;
+    s_k0 = scene_of(grp.scene_off, 0, grp.K - 1, b0);
+    s_k1 = scene_of(grp.scene_off, s_k0, grp.K - 1, b1);
   }
+  __syncthreads();
+  // grouped line positions [g_lo, g_hi) of this block's scenes, [my_lo, my_hi) of this thread's scene
+  const int k0 = s_k0, k1 = s_k1;
+  const int g_lo = grp.first[k0], g_hi = grp.first[k1 + 1];
+  if (g_lo >= g_hi) return;  // no line of the call in this block's scenes (uniform over the block)
+  const int k = (k0 == k1 || i >= S) ? k0 : scene_of(grp.scene_off, k0, k1, i);
+  const int my_lo = grp.first[k], my_hi = grp.first[k + 1];
+  const long long base = grp.scene_off[k];
   for (int l0 = g_lo; l0 < g_hi; l0 += kLineTile) {
     const int nl = min(kLineTile, g_hi - l0);
     __syncthreads();
-    if constexpr (MANY) {
-      for (int t = threadIdx.x; t < nl; t += blockDim.x) line_s[t] = grp.order[l0 + t];
-      __syncthreads();
-      for (int t = threadIdx.x; t < nl * 6; t += blockDim.x) box[t] = aabb[line_s[t / 6] * kBoxFloats + t % 6];
-    } else {
-      for (int t = threadIdx.x; t < nl * 6; t += blockDim.x) box[t] = aabb[(l0 + t / 6) * kBoxFloats + t % 6];
-    }
+    for (int t = threadIdx.x; t < nl; t += blockDim.x) line_s[t] = grp.order[l0 + t];
+    __syncthreads();
+    for (int t = threadIdx.x; t < nl * 6; t += blockDim.x) box[t] = aabb[line_s[t / 6] * kBoxFloats + t % 6];
     __syncthreads();
     if (i >= S) continue;
-    for (int j = 0; j < nl; ++j) {
-      if constexpr (MANY) {
-        if (l0 + j < my_lo || l0 + j >= my_hi) continue;
-      }
+    for (int j = max(my_lo - l0, 0), j_end = min(my_hi - l0, nl); j < j_end; ++j) {
       if (!inside(box + j * 6)) continue;
-      const int l = MANY ? line_s[j] : l0 + j;
+      const int l = line_s[j];
       const float* sb = aabb + l * kBoxFloats + 6;
       const float* q = dense_f + static_cast<size_t>(l) * kDense * 3;
       float best = 3.4e38f;
@@ -490,7 +474,6 @@ __global__ void __launch_bounds__(256) select_kernel(const float4* __restrict__ 
   }
   if (status[1] & 1) return;  // candidate buffer too small: the host re-runs with status[0] entries
   pts += src.base(l);
-  const uint64_t seed = src.seed_of(l), line = src.id_of(l);
   const long long off = offset[l];
   const double cx = centers[l * 3], cy = centers[l * 3 + 1], cz = centers[l * 3 + 2];
   float* ctx = context + static_cast<size_t>(l) * N * 4;
@@ -507,7 +490,7 @@ __global__ void __launch_bounds__(256) select_kernel(const float4* __restrict__ 
       long long idx = -1;
       float4 p = make_float4(0.f, 0.f, 0.f, 0.f);
       if (n > 0) {
-        const double u = det_uniform(seed, line, (1ull << 40) + j);
+        const double u = det_uniform(src.seed_of(l), src.id_of(l), (1ull << 40) + j);
         long long pick = static_cast<long long>(__dmul_rn(u, static_cast<double>(n)));
         pick = pick < n - 1 ? pick : n - 1;
         idx = sv[pick];

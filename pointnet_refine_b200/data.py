@@ -14,7 +14,8 @@ from typing import Sequence
 import numpy as np
 import torch
 
-from .scene import PreparedScenes, _resample_on_device, default_capacity, prepare_scenes, scenes_segments
+from .scene import (PreparedScenes, _resample_on_device, _seed_bits, _target_offset, default_capacity, prepare_scenes,
+                    scenes_segments)
 
 _MASK64 = (1 << 64) - 1
 
@@ -82,9 +83,7 @@ class SceneTrainingSet:
         self.num_context_points, self.crop_radius, self.decay_scale = int(num_context_points), float(crop_radius), float(decay_scale)
         self.seed, self.epoch = int(seed), 0
         self.line32, self.dense200, self.centers, self.noisy_line, ext_noisy = _resample_on_device([s[1] for s in samples], dev)
-        gt32, _, _, _, _ = _resample_on_device([s[2] for s in samples], dev)
-        center = self.centers[:, None, :]
-        self.target_offset = ((gt32 - center) - (self.line32 - center)).float()    # build_training_batch's rounding
+        self.target_offset = _target_offset([s[2] for s in samples], self.line32, self.centers)
         self.line_scene = torch.from_numpy(scene_idx.astype(np.int32)).to(dev)
         self.extent = max(ext_noisy, float(self.prepared.extents.max()))
         self.capacity = default_capacity(int(self.prepared.offsets_host[-1]), self.batch_size, self.num_context_points)
@@ -103,8 +102,7 @@ class SceneTrainingSet:
         """The batch of the given sample numbers (int64 CUDA tensor) as drawn in `epoch` (default: the current one)."""
         idx = samples.to(self.device, torch.int64)
         B = int(idx.shape[0])
-        s = epoch_seed(self.seed, self.epoch if epoch is None else epoch)
-        seeds = torch.full((B,), s - (1 << 64) if s >= 1 << 63 else s, dtype=torch.int64, device=self.device)   # uint64 bits
+        seeds = _seed_bits(epoch_seed(self.seed, self.epoch if epoch is None else epoch), B, self.device)
         context, _, _, total = scenes_segments(
             self.prepared, self.line_scene[idx], self.dense200[idx], self.line32[idx], self.centers[idx], seeds,
             idx.to(torch.int32), self.num_context_points, self.crop_radius, self.decay_scale, self.extent, self.capacity)

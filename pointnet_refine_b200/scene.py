@@ -3,11 +3,11 @@
 The reference builds the network input for ONE line at a time on the host: KD-tree over a 200-point resampling of the
 line, distance query for every scene point, crop, weighted sampling, centroid normalisation
 (src/dataset.py:78-130,214-237; inference_whole_scene.py:95-121), then a B = 1 forward per line (:124-142).
-`build_segments` does the crop / sampling / normalisation for all lines of a scene in one pass on the device
-(`lrn_scene_segments`, csrc/scene_kernels.cuh) and `refine_scene` runs the lines of a scene as one batch.
-`build_segments_many` / `build_training_batches` / `refine_scenes` do the same for lines of MANY scenes in one device call
-(`lrn_scenes_segments`) over scenes prepared once with `prepare_scenes`; `data.SceneTrainingSet` turns such a set of
-scenes into shuffled training batches.
+`build_segments` does the crop / sampling / normalisation for all lines of a scene in one pass on the device and
+`refine_scene` runs the lines of a scene as one batch.  `build_segments_many` / `build_training_batches` / `refine_scenes`
+do the same for lines of MANY scenes in one device call over scenes prepared once with `prepare_scenes`.  Every build is
+one `lrn_scenes_segments` call (csrc/scene_kernels.cuh); one scene is the case K = 1.  `data.SceneTrainingSet` turns a
+set of scenes into shuffled training batches.
 
 The polyline resampling runs on the device too (`lrn_scene_resample`, bit-equal to the numpy formulation; the host
 `resample_polyline` below is kept for callers and tests).  The draw follows the reproducible RNG contract documented in include/lrn_b200.h (the reference uses the global unseeded
@@ -97,34 +97,15 @@ def build_segments(scene, raw_lines: Sequence, num_context_points: int = 1024, c
                    decay_scale: float = 2.0, seed: int = 0, capacity: int | None = None) -> SceneSegments:
     """scene (S, 4) fp32 CUDA [x, y, z, intensity] or a PreparedScene (several line sets over one scene: sort it once);
     raw_lines: polylines (n_i, 3) in scene coordinates.  Defaults are inference_whole_scene.py's (:21-22,
-    weighted_sampling's decay_scale); LaneRefineDataset uses 2048 / 4.0 / 2.0."""
-    prepared = scene if isinstance(scene, PreparedScene) else prepare_scene(scene)
-    scene = prepared.points
-    S, L, N = scene.shape[0], len(raw_lines), int(num_context_points)
+    weighted_sampling's decay_scale); LaneRefineDataset uses 2048 / 4.0 / 2.0.  Line l is drawn with (seed, l)."""
+    prepared = _one_scene(scene)
+    L = len(raw_lines)
     if L == 0:
         raise ValueError("no lines")
-    dev = scene.device
-    d_line, d_dense, d_cent, noisy, extent_lines = _resample_on_device(raw_lines, dev)
-    extent = max(extent_lines, prepared.extent)
-    context = torch.empty(L, N, 4, dtype=torch.float32, device=dev)
-    indices = torch.empty(L, N, dtype=torch.int64, device=dev)
-    counts = torch.empty(L, dtype=torch.int32, device=dev)
-    status = torch.zeros(2, dtype=torch.int64, device=dev)
-    cap = int(capacity) if capacity else max(1 << 20, min(S * L, 8 * L * N))
-    for _ in range(2):
-        ws = _aligned_bytes(lib.lrn_scene_workspace_bytes(L, cap), dev)
-        _call("lrn_scene_segments", dev, scene, S, prepared.sorted_points, prepared.perm,
-              d_dense, d_line, d_cent, L, N, float(crop_radius), float(decay_scale), extent, int(seed) & (2 ** 64 - 1), cap,
-              context, indices, counts, status, ws, ws.numel())
-        total, flags = (int(v) for v in status.tolist())        # synchronises
-        if flags & 2:
-            raise RuntimeError("lrn_scene_segments: too many candidates tie exactly at a threshold key")
-        if not flags & 1:
-            break
-        cap = total                                                # candidate buffer was too small: exact size now
-    else:
-        raise RuntimeError("lrn_scene_segments: candidate buffer overflow after resizing")
-    return SceneSegments(context, noisy, d_cent.cpu().numpy(), d_line.cpu().numpy(), indices, counts)
+    dev = prepared.points.device
+    return _segments(prepared, raw_lines, torch.zeros(L, dtype=torch.int32, device=dev), _seed_bits(seed, L, dev),
+                     torch.arange(L, dtype=torch.int32, device=dev), num_context_points, crop_radius, decay_scale,
+                     float(prepared.extents[0]), capacity)
 
 
 def build_training_batch(scene, noisy_lines: Sequence, gt_lines: Sequence, num_context_points: int = 2048,
@@ -133,15 +114,8 @@ def build_training_batch(scene, noisy_lines: Sequence, gt_lines: Sequence, num_c
     sample: {'context' (L,N,4), 'noisy_line' (L,32,3), 'target_offset' (L,32,3)} fp32 CUDA, with
     target_offset = (gt32 - center) - (noisy32 - center) in float64, rounded once (src/dataset.py:239-243).
     Defaults are LaneRefineDataset's (num_context_points 2048, crop_radius 4.0, decay_scale 2.0)."""
-    if len(noisy_lines) != len(gt_lines):
-        raise ValueError("one ground-truth polyline per noisy polyline")
-    seg = build_segments(scene, noisy_lines, num_context_points, crop_radius, decay_scale, seed)
-    dev = seg.context.device
-    gt32, _, _, _, _ = _resample_on_device(gt_lines, dev)
-    center = torch.from_numpy(seg.centers).to(dev)[:, None, :]
-    noisy32 = torch.from_numpy(seg.line32).to(dev)
-    target = ((gt32 - center) - (noisy32 - center)).float()
-    return {"context": seg.context, "noisy_line": seg.noisy_line, "target_offset": target}
+    return build_training_batches(_one_scene(scene), noisy_lines, gt_lines, np.zeros(len(noisy_lines), dtype=np.int64),
+                                  num_context_points, crop_radius, decay_scale, seed)
 
 
 @torch.no_grad()
@@ -192,13 +166,14 @@ def prepare_scenes(scenes: Sequence, sort: bool = True) -> PreparedScenes:
     np.cumsum(sizes, out=offsets[1:])
     if offsets[-1] >= 2 ** 31:
         raise ValueError(f"{offsets[-1]} points in all: fewer than 2^31 per PreparedScenes")
-    points = torch.cat([p.points for p in preps])
+    cat = (lambda ts: ts[0]) if len(preps) == 1 else torch.cat      # one scene: its own tensors, not a copy
+    points = cat([p.points for p in preps])
     sorted_points = perm = None
     if sort:
         if any(p.sorted_points is None for p in preps):
             raise ValueError("sort=True needs every PreparedScene to carry its sorted copy")
-        sorted_points = torch.cat([p.sorted_points for p in preps])
-        perm = torch.cat([p.perm for p in preps])
+        sorted_points = cat([p.sorted_points for p in preps])
+        perm = cat([p.perm for p in preps])
     extents = np.array([p.extent for p in preps], dtype=np.float64)
     return PreparedScenes(points, torch.from_numpy(offsets).to(dev), offsets, sorted_points, perm, extents)
 
@@ -225,9 +200,30 @@ def index_within_scene(line_scene) -> np.ndarray:
     return out
 
 
-def _u64_device(values, dev) -> torch.Tensor:
-    """uint64 values as an int64 CUDA tensor holding the same bits (what the C ABI reads as uint64_t)."""
-    return torch.from_numpy(np.ascontiguousarray(np.asarray(values, dtype=np.uint64)).view(np.int64)).to(dev)
+def _one_scene(scene) -> PreparedScenes:
+    """A scene (S, 4) fp32 CUDA, sorted here, or a PreparedScene as a one-scene PreparedScenes over the same tensors."""
+    prep = scene if isinstance(scene, PreparedScene) else prepare_scene(scene)
+    return prepare_scenes([prep], sort=prep.sorted_points is not None)
+
+
+def _seed_bits(seeds, L: int, dev) -> torch.Tensor:
+    """uint64 seeds as an (L,) int64 CUDA tensor holding the same bits (what the C ABI reads as uint64_t): one seed for
+    every line (a device fill) or one per line."""
+    if np.ndim(seeds) == 0:
+        s = int(seeds) & (2 ** 64 - 1)
+        return torch.full((L,), s - 2 ** 64 if s >= 2 ** 63 else s, dtype=torch.int64, device=dev)
+    bits = np.ascontiguousarray(np.asarray(seeds, dtype=np.uint64)).view(np.int64)
+    if bits.shape != (L,):
+        raise ValueError("one seed per line")
+    return torch.from_numpy(bits).to(dev)
+
+
+def _target_offset(gt_lines: Sequence, line32: torch.Tensor, centers: torch.Tensor) -> torch.Tensor:
+    """LaneRefineDataset's target_offset (src/dataset.py:239-243) of every line: (gt32 - center) - (noisy32 - center) in
+    float64, rounded once to fp32; line32 (L,32,3) / centers (L,3) float64 CUDA of the noisy lines."""
+    gt32, _, _, _, _ = _resample_on_device(gt_lines, line32.device)
+    center = centers[:, None, :]
+    return ((gt32 - center) - (line32 - center)).float()
 
 
 def default_capacity(S: int, L: int, N: int) -> int:
@@ -280,19 +276,25 @@ def build_segments_many(prepared, raw_lines: Sequence, line_scene, num_context_p
         raise ValueError("no lines")
     ls = _host_line_scene(line_scene, L, K)
     dev = prepared.points.device
-    seeds = np.full(L, int(seed) & (2 ** 64 - 1), dtype=np.uint64) if seeds is None else np.asarray(seeds, dtype=np.uint64)
     line_ids = index_within_scene(ls) if line_ids is None else np.asarray(line_ids, dtype=np.int64)
-    if seeds.shape != (L,) or line_ids.shape != (L,):
-        raise ValueError("one seed and one line id per line")
+    if line_ids.shape != (L,):
+        raise ValueError("one line id per line")
     if line_ids.min() < 0 or line_ids.max() >= 2 ** 32:
         raise ValueError("line ids are uint32")
-    d_line, d_dense, d_cent, noisy, extent_lines = _resample_on_device(raw_lines, dev)
-    extent = max(extent_lines, float(prepared.extents[np.unique(ls)].max()))
+    return _segments(prepared, raw_lines, torch.from_numpy(ls.astype(np.int32)).to(dev),
+                     _seed_bits(seed if seeds is None else seeds, L, dev),
+                     torch.from_numpy(line_ids.astype(np.uint32).view(np.int32)).to(dev), num_context_points, crop_radius,
+                     decay_scale, float(prepared.extents[np.unique(ls)].max()), capacity)
+
+
+def _segments(prepared: PreparedScenes, raw_lines: Sequence, line_scene, seeds, line_ids, num_context_points, crop_radius,
+              decay_scale, extent: float, capacity) -> SceneSegments:
+    """The lines resampled on the device, then scenes_segments over them; extent: of the scenes the lines lie in."""
+    d_line, d_dense, d_cent, noisy, extent_lines = _resample_on_device(raw_lines, prepared.points.device)
     N = int(num_context_points)
-    cap = int(capacity) if capacity else default_capacity(int(prepared.offsets_host[-1]), L, N)
-    context, indices, counts, _ = scenes_segments(
-        prepared, torch.from_numpy(ls.astype(np.int32)).to(dev), d_dense, d_line, d_cent, _u64_device(seeds, dev),
-        torch.from_numpy(line_ids.astype(np.uint32).view(np.int32)).to(dev), N, crop_radius, decay_scale, extent, cap)
+    cap = int(capacity) if capacity else default_capacity(int(prepared.offsets_host[-1]), len(raw_lines), N)
+    context, indices, counts, _ = scenes_segments(prepared, line_scene, d_dense, d_line, d_cent, seeds, line_ids, N, crop_radius,
+                                                  decay_scale, max(extent, extent_lines), cap)
     return SceneSegments(context, noisy, d_cent.cpu().numpy(), d_line.cpu().numpy(), indices, counts)
 
 
@@ -306,10 +308,7 @@ def build_training_batches(prepared, noisy_lines: Sequence, gt_lines: Sequence, 
     seg = build_segments_many(prepared, noisy_lines, line_scene, num_context_points, crop_radius, decay_scale, seed, seeds,
                               line_ids)
     dev = seg.context.device
-    gt32, _, _, _, _ = _resample_on_device(gt_lines, dev)
-    center = torch.from_numpy(seg.centers).to(dev)[:, None, :]
-    noisy32 = torch.from_numpy(seg.line32).to(dev)
-    target = ((gt32 - center) - (noisy32 - center)).float()
+    target = _target_offset(gt_lines, torch.from_numpy(seg.line32).to(dev), torch.from_numpy(seg.centers).to(dev))
     return {"context": seg.context, "noisy_line": seg.noisy_line, "target_offset": target}
 
 

@@ -16,14 +16,14 @@ from pointnet_refine_b200 import _lib, shard
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_exports_every_declared_symbol_abi_v3():
+def test_library_exports_every_declared_symbol_abi_v4():
     header = open(os.path.join(ROOT, "include", "lrn_b200.h")).read()
     declared = set(re.findall(r"^(?:int|size_t|const char\*) (lrn_[a-z0-9_]+)\(", header, re.M))
     assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 3
+    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 4
     assert _lib.lib.lrn_status_string(3).decode().startswith("unsupported")
     assert _lib.lib.lrn_encoder_packed_bytes(0) > 2 * 2_803_000 - 700      # bf16 blob holds all matrices
     assert _lib.lib.lrn_encoder_packed_bytes(1) > _lib.lib.lrn_encoder_packed_bytes(0)

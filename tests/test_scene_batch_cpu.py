@@ -13,23 +13,24 @@ from pointnet_refine_b200 import _lib, data, scene
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_many_scene_entry_points_are_declared_bound_and_exported():
-    """Added to ABI version 3 without a version change: every earlier entry point is unchanged."""
+def test_scene_entry_points_abi_v4_many_scene_only():
+    """ABI version 4: the many-scene entry points are the only scene builders; the per-scene ones are gone everywhere."""
     header = open(os.path.join(ROOT, "include", "lrn_b200.h")).read()
     declared = set(re.findall(r"^(?:int|size_t|const char\*) (lrn_[a-z0-9_]+)\(", header, re.M))
-    new = {"lrn_scenes_segments", "lrn_scenes_workspace_bytes"}
-    assert new <= declared and new <= set(_lib.EXPORTS)
+    many = {"lrn_scenes_segments", "lrn_scenes_workspace_bytes"}
+    assert many <= declared and many <= set(_lib.SIGNATURES)
     lib = ctypes.CDLL(_lib.LIB_PATH)
-    for name in new:
+    for name in many:
         assert hasattr(lib, name), name
-    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 3
+    for name in ("lrn_scene_segments", "lrn_scene_workspace_bytes"):
+        assert name not in header and name not in _lib.SIGNATURES and not hasattr(lib, name), name
+    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 4
 
 
-def test_scenes_workspace_grows_with_lines_scenes_and_capacity():
+def test_scenes_workspace_bytes_grow_with_lines_scenes_and_capacity():
     ws = _lib.lib.lrn_scenes_workspace_bytes
     assert ws(0, 3, 100) == 0 and ws(4, 0, 100) == 0 and ws(4, 3, 0) == 0
     base = ws(16, 3, 1 << 20)
-    assert base > _lib.lib.lrn_scene_workspace_bytes(16, 1 << 20)          # the grouping arrays come on top
     assert ws(16, 3000, 1 << 20) > base and ws(32, 3, 1 << 20) > base and ws(16, 3, 1 << 21) >= base + 12 * (1 << 20)
 
 
