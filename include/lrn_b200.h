@@ -36,8 +36,11 @@ extern "C" {
  *    so a caller built against an earlier version-3 library runs unchanged, and a caller that needs the additions finds
  *    them missing by name when it loads an older library (pointnet_refine_b200/_lib.py reports which).
  * 4: the per-scene segment builder and its workspace-size function removed: the lines of one scene are the K = 1 case
- *    of lrn_scenes_segments, which gives the same bits. */
-#define LRN_ABI_VERSION 4
+ *    of lrn_scenes_segments, which gives the same bits.
+ * 5: the head gather of attention gradients and the host-counted lrn_adam_step removed: the train attention backward
+ *    writes dK / dV in place in the K / V projections' layout, and every Adam step keeps its step count on the device
+ *    (lrn_adam_step_capturable). */
+#define LRN_ABI_VERSION 5
 
 typedef struct CUstream_st* lrn_stream_t; /* == cudaStream_t */
 
@@ -374,18 +377,12 @@ int lrn_train_attention_backward(const float* q, const void* k, int64_t ld_k, co
  * gradient is bf16 (cols % 64 == 0, ld % 8 == 0, A 16-byte aligned). */
 int lrn_col_sum_bf16(const void* A, int64_t ld, int64_t rows, int64_t cols, float* out, lrn_stream_t stream);
 
-/* src (B, H, N, 32) bf16 contiguous (the dK / dV of one cross-attention layer) -> column block `layer` of the
- * (B, N, L, H, 32) gradient buffer that the K / V projection's dgrad and wgrad GEMMs read. */
-int lrn_gather_heads(const void* src, int B, int H, int N, int layer, int L, void* dst, lrn_stream_t stream);
-
 /* ---- training-loop machinery (SURVEY.md 8f row 4) ----
  * One Adam step over a flat fp32 buffer holding every parameter (train.py:40 optim.Adam(model.parameters(), lr);
- * torch.optim.Adam semantics without amsgrad, weight decay added to the gradient); step counts from 1. */
-int lrn_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
-                  float beta2, float eps, float weight_decay, int64_t step, lrn_stream_t stream);
-/* The same step with the step count kept on the device (torch.optim.Adam(capturable=True) semantics): *step_state is
- * incremented by a one-thread kernel first, the bias corrections are computed from it on the device, so the two launches
- * can be captured in a CUDA graph and replayed (train.py:71 optimizer.step() inside GraphedTrainStep). */
+ * torch.optim.Adam semantics without amsgrad, weight decay added to the gradient), with the step count kept on the
+ * device (torch.optim.Adam(capturable=True) semantics): *step_state (0 before the first step) is incremented by a
+ * one-thread kernel first and the bias corrections are computed from it on the device in double precision, so the two
+ * launches can be captured in a CUDA graph and replayed (train.py:71 optimizer.step() inside GraphedTrainStep). */
 int lrn_adam_step_capturable(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
                              float beta2, float eps, float weight_decay, int64_t* step_state, lrn_stream_t stream);
 /* Deep-supervision loss of train.py:63-69: loss[0] = (1/L) sum_l L1Loss(pred[l], target) for pred (L, n) and target (n)

@@ -16,7 +16,7 @@ CSRC = os.path.join(_HERE, "csrc")
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "lrn_b200.h")
 
 # enums of include/lrn_b200.h
-ABI_VERSION = 4      # LRN_ABI_VERSION
+ABI_VERSION = 5      # LRN_ABI_VERSION
 LRN_OK = 0
 PREC_BF16, PREC_TF32, PREC_FP32X3 = 0, 1, 2
 OUT_POOL, OUT_ARGMAX, OUT_FUSED, OUT_MEMORY, OUT_MEMORY_BF16 = 1, 2, 4, 8, 16
@@ -78,11 +78,9 @@ SIGNATURES = {
     "lrn_scenes_workspace_bytes": (sz, [ci, ci, i64]),
     "lrn_scenes_segments": (ci, [vp, vp, ci, i64, vp, vp, vp, vp, vp, vp, vp, vp, ci, ci, f64, f64, f64, i64, vp, vp, vp, vp, vp, sz,
                                  vp]),
-    "lrn_adam_step": (ci, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, i64, vp]),
     "lrn_adam_step_capturable": (ci, [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, vp, vp]),
     "lrn_l1_deep_supervision": (ci, [vp, vp, ci, i64, vp, vp, vp]),
     "lrn_col_sum_bf16": (ci, [vp, i64, i64, i64, vp, vp]),
-    "lrn_gather_heads": (ci, [vp, ci, ci, ci, ci, ci, vp, vp]),
     "lrn_add_layernorm": (ci, [vp, vp, vp, vp, f32, vp, vp, i64, i64, vp]),
     "lrn_add_layernorm_backward": (ci, [vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, vp]),
     "lrn_self_attention32": (ci, [vp, vp, vp, ci, vp]),

@@ -1239,17 +1239,6 @@ int lrn_encoder_train_backward(const lrn_encoder_params* pr, const float* contex
   return LRN_OK;
 }
 
-int lrn_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
-                  float beta2, float eps, float weight_decay, int64_t step, lrn_stream_t stream) {
-  if (!params || !grads || !exp_avg || !exp_avg_sq) return fail(LRN_ERR_BAD_ARG, "null pointer");
-  if (n <= 0 || step < 1) return fail(LRN_ERR_BAD_SHAPE, "n=%lld step=%lld", (long long)n, (long long)step);
-  LRN_DEVICE(dev);
-  const double bc1 = 1.0 - pow(double(beta1), double(step)), bc2 = 1.0 - pow(double(beta2), double(step));
-  const int grid = int(std::min<int64_t>((n + 255) / 256, int64_t(dev.sms) * 16));
-  return launch(adam_step_kernel, grid, 256, 0, stream, params, grads, exp_avg, exp_avg_sq, n, float(double(lr) / bc1), beta1,
-                beta2, eps, weight_decay, float(1.0 / sqrt(bc2)));
-}
-
 int lrn_adam_step_capturable(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float beta1,
                              float beta2, float eps, float weight_decay, int64_t* step_state, lrn_stream_t stream) {
   if (!params || !grads || !exp_avg || !exp_avg_sq || !step_state) return fail(LRN_ERR_BAD_ARG, "null pointer");
@@ -1437,17 +1426,6 @@ int lrn_col_sum_bf16(const void* A, int64_t ld, int64_t rows, int64_t cols, floa
   LRN_CUDA(cudaMemsetAsync(out, 0, size_t(cols) * 4, stream));
   return launch(col_stats_kernel, stream_grid(col_stats_kernel, int(cols), rows, dev.sms), 256, 0, stream,
                 reinterpret_cast<const __nv_bfloat16*>(A), ld, rows, out, nullptr, 0);
-}
-
-int lrn_gather_heads(const void* src, int B, int H, int N, int layer, int L, void* dst, lrn_stream_t stream) {
-  if (!src || !dst) return fail(LRN_ERR_BAD_ARG, "null pointer");
-  if (B <= 0 || H <= 0 || N <= 0 || L <= 0 || layer < 0 || layer >= L) return fail(LRN_ERR_BAD_SHAPE, "B=%d H=%d N=%d layer=%d L=%d", B, H, N, layer, L);
-  if (misaligned(16, src, dst)) return fail(LRN_ERR_MISALIGNED, "16-byte alignment");
-  LRN_DEVICE(dev);
-  const long long groups = static_cast<long long>(B) * H * ((N + 7) / 8);
-  const int grid = int(std::min<long long>((groups + 7) / 8, static_cast<long long>(dev.sms) * 16));
-  return launch(gather_heads_kernel, grid, 256, 0, stream, reinterpret_cast<const uint4*>(src), B, H, N, layer, L,
-                reinterpret_cast<uint4*>(dst));
 }
 
 }  // extern "C"

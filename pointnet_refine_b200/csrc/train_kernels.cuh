@@ -602,52 +602,13 @@ __global__ void copy_submatrix_kernel(const float* __restrict__ src, long long l
   }
 }
 
-// Attention gradients back into the projection layout: src (B, H, N, 32) bf16 contiguous (what scaled_dot_product_attention
-// returns for dK / dV of one layer) -> dst[b][n][layer][h][0:32] of a (B, N, L, H, 32) buffer, i.e. the column block of
-// that layer in the (B*N, L*H*32) gradient matrix the dgrad / wgrad GEMMs read.  One warp moves 8 points of one head per
-// step: 512 contiguous bytes in, eight 64-byte pieces out.
-__global__ void __launch_bounds__(256)
-gather_heads_kernel(const uint4* __restrict__ src, int B, int H, int N, int layer, int L, uint4* __restrict__ dst) {
-  const int lane = threadIdx.x & 31;
-  const long long warps = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
-  const long long groups = static_cast<long long>(B) * H * ((N + 7) / 8);
-  const int per = (N + 7) / 8;
-  for (long long gidx = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; gidx < groups; gidx += warps) {
-    const int n0 = static_cast<int>(gidx % per) * 8;
-    const long long bh = gidx / per;
-    const int h = static_cast<int>(bh % H);
-    const long long b = bh / H;
-    const int n = n0 + (lane >> 2), piece = lane & 3;   // 4 x 16 bytes = one point's 32 bf16
-    if (n < N) {
-      const uint4 v = src[((b * H + h) * N + n) * 4 + piece];
-      dst[(((b * N + n) * L + layer) * H + h) * 4 + piece] = v;
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
 // Training-loop machinery (SURVEY.md 8f row 4): Adam over one flat parameter buffer and the L1 deep-supervision loss.
 // ---------------------------------------------------------------------------------------------
 // torch.optim.Adam (train.py:40, no amsgrad), same operation order as its single-tensor path:
 //   g += wd * p;  m = m + (1 - b1) (g - m);  v = b2 v + (1 - b2) g g;  p -= (lr / bc1) * m / (sqrt(v) / sqrt(bc2) + eps)
-__global__ void __launch_bounds__(256)
-adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
-                 float step_size, float b1, float b2, float eps, float wd, float inv_bc2_sqrt) {
-  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
-  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride) {
-    float gi = g[i];
-    const float pi = p[i];
-    if (wd != 0.f) gi = fmaf(wd, pi, gi);
-    const float mi = fmaf(1.f - b1, gi - m[i], m[i]);
-    const float vi = fmaf(1.f - b2, gi * gi, b2 * v[i]);
-    m[i] = mi;
-    v[i] = vi;
-    p[i] = pi - step_size * (mi / (sqrtf(vi) * inv_bc2_sqrt + eps));
-  }
-}
-
-// The same step with the step count in device memory (torch.optim.Adam(capturable=True)): a captured CUDA graph replays
-// it with the right bias corrections.  adam_bump_step_kernel runs first in the stream (step += 1).
+// The step count is in device memory (torch.optim.Adam(capturable=True)), so a captured CUDA graph replays the step with
+// the right bias corrections.  adam_bump_step_kernel runs first in the stream (step += 1).
 __global__ void adam_bump_step_kernel(long long* step) { *step += 1; }
 
 __global__ void __launch_bounds__(256)

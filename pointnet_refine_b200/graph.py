@@ -56,7 +56,7 @@ class GraphedTrainStep:
 
     What capture needs, and how the pieces provide it:
     * static shapes: `context` (B, N, 4), `noisy_line` (B, M, 3), `target` (B, M, 3) are copied into static buffers;
-    * the optimizer's step count on the device: `FlatAdam(capturable=True)` (lrn_adam_step_capturable);
+    * the optimizer's step count on the device: `FlatAdam` keeps it there (lrn_adam_step_capturable);
     * dropout that changes from replay to replay with frozen launch arguments: the train attention kernels add a device
       word to their seed (train_ops.DropoutSeedState), advanced inside the graph; torch's own dropout kernels take their
       Philox offsets from the graph-registered generator;
@@ -78,8 +78,8 @@ class GraphedTrainStep:
     def __init__(self, net, optimizer, context, noisy_line, target, loss_fn=None, warmup: int = 2):
         from . import train_ops
         from .optim import FlatAdam, deep_supervision_l1
-        if not isinstance(optimizer, FlatAdam) or not optimizer.capturable:
-            raise TypeError("GraphedTrainStep needs FlatAdam(..., capturable=True): the step count must live on the device")
+        if not isinstance(optimizer, FlatAdam):
+            raise TypeError("GraphedTrainStep needs FlatAdam: the step count must live on the device")
         model = getattr(net, "module", net)
         if not model.training:
             raise RuntimeError("GraphedTrainStep captures a training step: call model.train() first")
@@ -92,7 +92,7 @@ class GraphedTrainStep:
         self._side = torch.cuda.Stream(device=dev)
         # ---- eager warm-up on the capture stream (lazy handles, kernel attributes, allocator), state put back afterwards
         keep = [optimizer._flat, optimizer._m, optimizer._v, optimizer._step_dev] + [b for b in model.buffers()]
-        saved, host_step = [t.clone() for t in keep], optimizer._step
+        saved = [t.clone() for t in keep]
         self._side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(self._side):
             for _ in range(warmup):
@@ -100,7 +100,6 @@ class GraphedTrainStep:
             with torch.no_grad():
                 for t, s in zip(keep, saved):
                     t.copy_(s)
-        optimizer._step = host_step
         torch.cuda.current_stream(dev).wait_stream(self._side)
         # ---- capture
         self.graph = torch.cuda.CUDAGraph()
@@ -119,7 +118,6 @@ class GraphedTrainStep:
             raise
         finally:
             train_ops.DropoutSeedState.word = None
-        optimizer._step = host_step                        # the capture executed nothing
         self.loss, self.pred = loss.detach(), pred.detach()
         self.replays = 0
 
@@ -161,7 +159,6 @@ class GraphedTrainStep:
         self.tgt.copy_(target, non_blocking=True)
         self.graph.replay()
         self.replays += 1
-        self.opt._step += 1
         # the replayed kernels wrote the parameters through raw pointers: the weight-folding caches of the eval path
         # fingerprint (data_ptr, _version)
         torch.autograd.graph.increment_version(self._params)

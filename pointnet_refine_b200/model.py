@@ -13,8 +13,9 @@ What runs where
   * train mode (batch-statistic BatchNorm, autograd): by default the stock PyTorch fp32 formulation, i.e. exactly
     the reference's numerics (a bf16 forward flips the ReLU mask of a few per mille of the activations, which is
     within tolerance for inference but changes gradients -- the caller decides).  `native_training = True` /
-    LRN_NATIVE_TRAIN=1 (bf16 tier) switches the encoder, context_proj and the decoder's linears to the sm_100a
-    train path (train_ops.py: batch-stat BN forward and a hand-written backward on the tcgen05 GEMMs).
+    LRN_NATIVE_TRAIN=1 (bf16 tier) switches the encoder, and with M = 32 also context_proj and the decoder's linears and
+    attention, to the sm_100a train path (train_ops.py: batch-stat BN forward and a hand-written backward on the tcgen05
+    GEMMs).
   * CPU tensors: not supported -- there is no CPU path in the product (the oracle lives in oracle/).
 """
 from __future__ import annotations
@@ -26,7 +27,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import ops
+from . import ops, train_ops
 
 _DEFAULT_PRECISION = os.environ.get("LRN_PRECISION", "bf16")
 
@@ -131,10 +132,8 @@ class MultiScalePointNetEncoder(nn.Module):
 
     def forward(self, x):
         _require_cuda(x, "MultiScalePointNetEncoder")
-        if self.training and self.native_training and self.precision == "bf16":
-            from .train_ops import encoder_train_forward, native_train_supported   # batch-stat BN forward + hand-written backward
-            if native_train_supported(self):
-                return encoder_train_forward(self, x.transpose(2, 1))
+        if train_ops.native_train_supported(self):   # batch-stat BN forward + hand-written backward
+            return train_ops.encoder_train_forward(self, x.transpose(2, 1))
         if not _use_native(self, x):
             return self._forward_torch(x)
         out = self.run_native(x.transpose(2, 1), pool=True, fused=True)
@@ -420,15 +419,15 @@ class LineRefineNet(nn.Module):
         return cross_attention
 
     def _refine_fast_train(self, context, noisy_line, fused_pm):
-        """Autograd-capable decoder of model.train() on the native encoder: context_proj, the memory positional embedding
-        and the K / V projections of all six cross-attention layers run as differentiable bf16 tensor-core linears
-        (train_ops.linear_bf16: tcgen05 forward, dgrad and wgrad), the cross attention through
-        scaled_dot_product_attention with the reference's dropout rate on the attention weights
-        (src/model.py:84, nn.MultiheadAttention(dropout=0.1)); the query-side linears (self-attention projections,
-        FFN, pos_emb layer 2, cross-attention q / out_proj) take the same bf16 tensor-core linear when the batch has
-        >= 256 query rows; the 32 x 32 self attention, LayerNorms, dropouts and heads are stock ops.  Same parameters
-        as DetrTransformerDecoderLayer; dropout draws differ from the reference's RNG stream (they would from run to
-        run there, too)."""
+        """Autograd-capable decoder of model.train() on the native encoder, for M = 32 polyline points: context_proj, the
+        memory positional embedding and the K / V projections of all six cross-attention layers run as differentiable bf16
+        tensor-core linears (train_ops.linear_bf16 / kv_proj: tcgen05 forward, dgrad and wgrad); the self attention of
+        the 32 points and the cross attention run on lrn_train_attention_* with the reference's dropout rate on the
+        attention weights (src/model.py:84, nn.MultiheadAttention(dropout=0.1)); the query-side linears (self-attention
+        projections, FFN, pos_emb layer 2, cross-attention q / out_proj) take the same bf16 tensor-core linear when the
+        batch has >= 256 query rows; residual + LayerNorm is lrn_add_layernorm; point_mlp, dropouts and heads are stock
+        ops.  Same parameters as DetrTransformerDecoderLayer; dropout draws differ from the reference's RNG stream (they
+        would from run to run there, too)."""
         from .train_ops import (KVGradShare, add_layernorm, cross_attention_train, kv_proj, linear_bf16, pos_hidden_train,
                                 self_attention_train, thin_linear)
         B, N, _ = context.shape
@@ -441,11 +440,11 @@ class LineRefineNet(nn.Module):
         h = pos_hidden_train(context, self.pos_emb.mlp[0].weight, self.pos_emb.mlp[0].bias)    # (B,N,256) bf16
         posm = linear_bf16(h, self.pos_emb.mlp[2].weight, self.pos_emb.mlp[2].bias)
         share = KVGradShare()                           # the attention backward writes dK / dV of all layers in place
-        k_l = kv_proj(mem + posm, wk, bk, 6, H, share, zero_bias_grad=True)  # six (B, H, N, 32) views of one (B, N, 6, H, 32) GEMM result
-        v_l = kv_proj(mem, wv, bv, 6, H, share)
-        native_ca = noisy_line.shape[1] == 32           # 32 queries per segment: lrn_train_attention_* (else SDPA)
+        k_l = kv_proj(mem + posm, wk, bk, 6, H, share, key=True)  # six (B, H, N, 32) views of one (B, N, 6, H, 32) GEMM result
+        v_l = kv_proj(mem, wv, bv, 6, H, share, key=False)
         rows = B * noisy_line.shape[1]
         tc = rows >= 256 and rows % 64 == 0   # query-side linears on the bf16 tensor-core path (fwd, dgrad, wgrad)
+        lin16 = linear_bf16 if tc else F.linear   # self attention's [q | k] and v stay bf16 where the tensor-core linear produced them
 
         def lin(x, w, b):
             return linear_bf16(x, w, b, torch.float32) if tc else F.linear(x, w, b)
@@ -456,29 +455,14 @@ class LineRefineNet(nn.Module):
         outs = []
         for i, (layer, head) in enumerate(zip(self.decoder_layers, self.reg_branches)):
             qpos = lin(F.relu(thin_linear(current, pe0.weight, pe0.bias)), pe2.weight, pe2.bias)
-            q = tgt + qpos
             sa = layer.self_attn
-            if native_ca:     # [q | k] and v stay bf16 where the tensor-core linear produced them; attention on lrn_train_attention_*
-                lin16 = linear_bf16 if tc else F.linear
-                att = self_attention_train(lin16(q, sa.in_proj_weight[:2 * d], sa.in_proj_bias[:2 * d]),
-                                           lin16(tgt, sa.in_proj_weight[2 * d:], sa.in_proj_bias[2 * d:]),
-                                           sa.dropout if self.training else 0.0)
-            else:
-                qk = lin(q, sa.in_proj_weight[:2 * d], sa.in_proj_bias[:2 * d]).view(B, -1, 2, H, d // H)
-                v = lin(tgt, sa.in_proj_weight[2 * d:], sa.in_proj_bias[2 * d:]).view(B, -1, H, d // H)
-                att = F.scaled_dot_product_attention(qk[:, :, 0].transpose(1, 2), qk[:, :, 1].transpose(1, 2), v.transpose(1, 2),
-                                                     dropout_p=sa.dropout if self.training else 0.0)
-                att = att.transpose(1, 2).reshape(B, -1, d)
+            att = self_attention_train(lin16(tgt + qpos, sa.in_proj_weight[:2 * d], sa.in_proj_bias[:2 * d]),
+                                       lin16(tgt, sa.in_proj_weight[2 * d:], sa.in_proj_bias[2 * d:]), sa.dropout)
             att = lin(att, sa.out_proj.weight, sa.out_proj.bias)
             tgt = add_layernorm(tgt, layer.dropout1(att), layer.norm1)
             ca = layer.cross_attn
             qh = lin(tgt + qpos, ca.in_proj_weight[:d], ca.in_proj_bias[:d])
-            if native_ca:
-                att = cross_attention_train(qh, k_l[i], v_l[i], ca.dropout if self.training else 0.0, share, i)
-            else:
-                att = F.scaled_dot_product_attention(qh.view(B, -1, H, d // H).transpose(1, 2).bfloat16(), k_l[i], v_l[i],
-                                                     dropout_p=ca.dropout if self.training else 0.0)
-                att = att.transpose(1, 2).reshape(B, -1, d).float()
+            att = cross_attention_train(qh, k_l[i], v_l[i], ca.dropout, share, i)
             tgt = add_layernorm(tgt, layer.dropout2(lin(att, ca.out_proj.weight, ca.out_proj.bias)), layer.norm2)
             ffn = lin(layer.dropout(F.relu(lin(tgt, layer.linear1.weight, layer.linear1.bias))), layer.linear2.weight, layer.linear2.bias)
             tgt = add_layernorm(tgt, layer.dropout3(ffn), layer.norm3)
@@ -492,12 +476,11 @@ class LineRefineNet(nn.Module):
                 or noisy_line.shape[-1] != 3:
             raise ValueError(f"expected context (B,N,4) and noisy_line (B,M,3), got {tuple(context.shape)} and {tuple(noisy_line.shape)}")
         if not _use_native(self, context, noisy_line):
-            from .train_ops import encoder_train_forward, native_train_supported
             enc = self.context_encoder
-            if self.training and self.precision == "bf16" and enc.native_training and native_train_supported(enc):
-                _, fused_pm = encoder_train_forward(enc, context, point_major=True)
+            if self.training and noisy_line.shape[1] == 32 and train_ops.native_train_supported(enc):
+                _, fused_pm = train_ops.encoder_train_forward(enc, context, point_major=True)
                 return self._refine_fast_train(context, noisy_line, fused_pm)
-            _, fused = enc(context.transpose(2, 1))   # train mode: native fwd/bwd (bf16 tier)
+            _, fused = enc(context.transpose(2, 1))   # with native training on (M != 32): the channel-major native encoder
             memory = self.context_proj(fused.transpose(2, 1))
             return self._refine(context, noisy_line, memory, native_heads=False)
         B, N = context.shape[:2]

@@ -2,7 +2,7 @@
 
 `FlatAdam` is a drop-in for `optim.Adam(model.parameters(), lr=LR)` (reference train.py:40, train_dist.py:149): every
 parameter becomes a view of ONE flat fp32 buffer (and its `.grad` a view of one flat gradient buffer), so a step is one
-`lrn_adam_step` launch instead of a multi-tensor sweep, and `zero_grad` is one memset.
+`lrn_adam_step_capturable` call instead of a multi-tensor sweep, and `zero_grad` is one memset.
 `deep_supervision_l1` is the loss of train.py:63-69 (mean over decoder layers of L1Loss) as one fused forward+backward
 kernel."""
 from __future__ import annotations
@@ -28,15 +28,14 @@ class FlatAdam(torch.optim.Optimizer):
         self._m = torch.zeros_like(self._flat)
         self._v = torch.zeros_like(self._flat)
         self._views = list(zip(self._fp.params, self._fp.grad_views))
-        self._step = 0
-        # capturable (torch.optim.Adam's flag of the same name): the step count lives on the device and the bias
-        # corrections are computed there, so step() can be captured in a CUDA graph and replayed (graph.GraphedTrainStep)
-        self.capturable = bool(capturable)
-        self._step_dev = torch.zeros(1, dtype=torch.int64, device=self._flat.device) if capturable else None
+        # the step count lives on the device and the bias corrections are computed there, so step() can be captured in a
+        # CUDA graph and replayed (graph.GraphedTrainStep).  `capturable` (torch.optim.Adam's flag of the same name) is
+        # accepted for drop-in use and has no effect: every step is capturable.
+        self._step_dev = torch.zeros(1, dtype=torch.int64, device=self._flat.device)
 
     @property
     def steps_taken(self) -> int:
-        return int(self._step_dev.item()) if self.capturable else self._step
+        return int(self._step_dev.item())
 
     def _attach(self, keep_foreign: bool = True):
         """Make every parameter's .grad the view of the flat gradient buffer.  A gradient some other code bound to
@@ -68,9 +67,7 @@ class FlatAdam(torch.optim.Optimizer):
                 raise ValueError("FlatAdam.load_state_dict: checkpoint belongs to a different parameter list")
             self._m.copy_(flat["exp_avg"])
             self._v.copy_(flat["exp_avg_sq"])
-            self._step = int(flat["step"])
-            if self.capturable:
-                self._step_dev.fill_(self._step)
+            self._step_dev.fill_(int(flat["step"]))
 
     @torch.no_grad()
     def step(self, closure=None):
@@ -80,15 +77,9 @@ class FlatAdam(torch.optim.Optimizer):
                 loss = closure()
         self._attach()
         g = self.param_groups[0]
-        self._step += 1
         hyper = (float(g["lr"]), float(g["betas"][0]), float(g["betas"][1]), float(g["eps"]), float(g["weight_decay"]))
-        if self.capturable:
-            _call("lrn_adam_step_capturable", self._flat.device, self._flat, self._grad, self._m, self._v, self._flat.numel(),
-                  *hyper, self._step_dev)
-            torch.autograd.graph.increment_version([p for p, _ in self._views])
-            return loss
-        _call("lrn_adam_step", self._flat.device, self._flat, self._grad, self._m, self._v, self._flat.numel(), *hyper,
-              self._step)
+        _call("lrn_adam_step_capturable", self._flat.device, self._flat, self._grad, self._m, self._v, self._flat.numel(),
+              *hyper, self._step_dev)
         # the kernel wrote through raw pointers: tell autograd / the weight-folding caches (data_ptr + _version
         # fingerprints in model.py) that every parameter changed
         torch.autograd.graph.increment_version([p for p, _ in self._views])

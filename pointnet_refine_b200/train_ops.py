@@ -99,9 +99,13 @@ def _encoder_bns(module):
 
 
 def native_train_supported(module) -> bool:
-    """The native train path implements torch.nn.BatchNorm1d's default training behaviour: every BatchNorm of the encoder
-    in training mode with running statistics, an exponential momentum and one common eps.  Anything else (frozen /
-    .eval()'d BatchNorm layers, momentum=None cumulative averaging, track_running_stats=False) runs the stock ops."""
+    """Whether the encoder `module` trains on the native path: it is in train mode, opted in (`native_training`), in the
+    bf16 tier, and its BatchNorms behave as torch.nn.BatchNorm1d does by default in training, which is what the native
+    path implements: every one in training mode with running statistics, an exponential momentum and one common eps.
+    Anything else (frozen / .eval()'d BatchNorm layers, momentum=None cumulative averaging, track_running_stats=False)
+    runs the stock ops."""
+    if not (module.training and module.native_training and module.precision == "bf16"):
+        return False
     bns = _encoder_bns(module)
     return all(b.training and b.track_running_stats and b.momentum is not None and b.affine and b.eps == bns[0].eps
                and b.momentum == bns[0].momentum for b in bns)
@@ -185,16 +189,16 @@ class KVGradShare:
 
 class KVProjFn(torch.autograd.Function):
     """K (or V) projections of all L cross-attention layers as ONE bf16 tensor-core linear over the context points,
-    handed to the attention as L views (B, H, N, hd) of the (B, N, L, H, hd) result.  The backward takes the L attention
-    gradients in that same layout: when they are the views of a KVGradShare buffer that CrossAttnTrainFn filled in place
-    there is nothing to move; otherwise each is gathered into its column block (one strided copy), then dgrad / wgrad run
-    like LinearBf16Fn.  x (B, N, K) bf16 or fp32, weight (L*H*hd, K) fp32, bias fp32."""
+    handed to the attention as L views (B, H, N, hd) of the (B, N, L, H, hd) result.  The backward reads the L attention
+    gradients from the matching KVGradShare buffer (dK for the K projection, dV for V), where CrossAttnTrainFn wrote
+    them in place, then dgrad / wgrad run like LinearBf16Fn.  x (B, N, K) bf16 or fp32, weight (L*H*hd, K) fp32,
+    bias fp32."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, L, H, share, zero_bias_grad=False):
+    def forward(ctx, x, weight, bias, L, H, share, key):
         from . import ops
         B, N, K = x.shape
-        ctx.zero_bias_grad = bool(zero_bias_grad)
+        ctx.key = bool(key)
         xb = x.detach().to(torch.bfloat16).contiguous().view(B * N, K)
         wb = weight.detach().to(torch.bfloat16).contiguous()
         ctx.save_for_backward(xb, wb)
@@ -209,23 +213,14 @@ class KVProjFn(torch.autograd.Function):
         from . import ops
         xb, wb = ctx.saved_tensors
         B, N, K, L, H, x_dtype = ctx.meta
-        hd = wb.shape[0] // (L * H)
-        dy = None
-        if ctx.share is not None and ctx.share.dk is not None and all(g is not None for g in grads):
-            for base in (ctx.share.dk, ctx.share.dv):      # every gradient is the layer's column block of ONE shared buffer
-                if all(g.dtype == torch.bfloat16 and g.data_ptr() == base.data_ptr() + 2 * i * H * hd
-                       and tuple(g.stride()) == (N * L * H * hd, hd, L * H * hd, 1) for i, g in enumerate(grads)):
-                    dy = base
-        if dy is None:
-            dy = torch.empty(B, N, L, H, hd, dtype=torch.bfloat16, device=xb.device)
-            for i, g in enumerate(grads):
-                if g is None:
-                    dy[:, :, i].zero_()
-                elif hd == 32 and g.dtype == torch.bfloat16 and g.is_contiguous():
-                    # (B,H,N,32) as SDPA returns it -> its column block, one pass
-                    _call("lrn_gather_heads", g.device, g, B, H, N, i, L, dy)
-                else:
-                    dy[:, :, i].copy_(g.transpose(1, 2))
+        dk, dv = ctx.share.buffers(B, N, L, xb.device)
+        dy = dk if ctx.key else dv
+        for i, g in enumerate(grads):
+            block = dy[:, :, i]
+            if g.data_ptr() != block.data_ptr():
+                # autograd materialised this gradient (zeros): the layer's output is not on the loss's graph, so its
+                # attention backward never wrote the block
+                block.copy_(g.transpose(1, 2))
         dyb = dy.view(B * N, -1)
         need_x, need_w, need_b = ctx.needs
         dx = dw = db = None
@@ -237,14 +232,14 @@ class KVProjFn(torch.autograd.Function):
             # K projection: a key bias shifts every score of a query by the same amount, which softmax ignores, so its
             # gradient sum_n dK[n] vanishes identically (rows of the score gradient sum to zero, with or without dropout);
             # the reference produces fp32 rounding noise there, a bf16 column sum would produce more - write the exact zero
-            db = torch.zeros(wb.shape[0], dtype=torch.float32, device=xb.device) if ctx.zero_bias_grad else _col_sum(dyb)
+            db = torch.zeros(wb.shape[0], dtype=torch.float32, device=xb.device) if ctx.key else _col_sum(dyb)
         return dx, dw, db, None, None, None, None
 
 
-def kv_proj(x, weight, bias, layers: int, heads: int, share: KVGradShare | None = None, zero_bias_grad: bool = False):
-    """(B, N, K) -> tuple of `layers` tensors (B, heads, N, hd), see KVProjFn.  zero_bias_grad: the K projection (its
-    bias gradient is identically zero)."""
-    return KVProjFn.apply(x, weight, bias, layers, heads, share, zero_bias_grad)
+def kv_proj(x, weight, bias, layers: int, heads: int, share: KVGradShare, key: bool):
+    """(B, N, K) -> tuple of `layers` tensors (B, heads, N, hd), see KVProjFn.  key: the K projection (its gradients
+    come from share.dk and its bias gradient is identically zero), else the V projection (share.dv)."""
+    return KVProjFn.apply(x, weight, bias, layers, heads, share, key)
 
 
 class DropoutSeedState:

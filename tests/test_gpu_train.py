@@ -355,8 +355,81 @@ def test_train_native_decoder_close_to_stock(dev, B):
         assert cos >= 0.9, (n, cos)
 
 
+def test_train_native_at_m16_runs_stock_decoder(dev):
+    """native_training with M = 16 polyline points: the train decoder is the stock one (channel-major native encoder,
+    context_proj, _refine(native_heads=False)), never _refine_fast_train, which is for M = 32; loss and gradients match
+    that arm run explicitly, within the thresholds of test_train_native_decoder_close_to_stock."""
+    import pointnet_refine_b200 as prb
+    m = prb.LineRefineNet().to(dev)
+    m.load_state_dict(synth.to_torch(synth.make_state_dict(2)), strict=True)
+    m.train()
+    m.context_encoder.native_training = True
+    _no_dropout(m)
+    fast_calls = []
+    fast = m._refine_fast_train
+    m._refine_fast_train = lambda *a: fast_calls.append(1) or fast(*a)
+    B = 8
+    ctx, line = (torch.from_numpy(a).to(dev) for a in synth.make_inputs(B, 512, M=16, seed=11))
+    tgt = 0.1 * torch.randn(B, 16, 3, device=dev, generator=torch.Generator(device=dev).manual_seed(1))
+    res = {}
+    for forward in (True, False):
+        m.zero_grad()
+        if forward:
+            out = m(ctx, line)
+        else:
+            _, fused = m.context_encoder(ctx.transpose(2, 1))
+            out = m._refine(ctx, line, m.context_proj(fused.transpose(2, 1)), native_heads=False)
+        loss = sum(torch.nn.functional.l1_loss(out[l], tgt) for l in range(6)) / 6
+        loss.backward()
+        res[forward] = (float(loss.detach()), {n: p.grad.clone() for n, p in m.named_parameters()})
+    assert not fast_calls
+    assert abs(res[True][0] - res[False][0]) <= 2e-2 * abs(res[False][0])
+    for n in ("context_proj.weight", "pos_emb.mlp.2.weight", "decoder_layers.0.cross_attn.in_proj_weight",
+              "decoder_layers.5.linear1.weight", "reg_branches.5.0.weight"):
+        a, b = res[True][1][n].flatten().double(), res[False][1][n].flatten().double()
+        cos = float(torch.dot(a, b) / (a.norm() * b.norm()))
+        assert cos >= 0.9, (n, cos)
+
+
+def test_kv_proj_unused_layers_get_zero_gradient(dev):
+    """kv_proj feeding cross_attention_train for layer 0 only: autograd materialises the gradients of layers 1..5 (their
+    attention backward never runs) and KVProjFn writes them into their column blocks of the shared dK / dV buffers, which
+    start as NaN here.  The weight and bias rows of layers 1..5 get exactly zero; layer 0's rows and dx match fp64
+    autograd on the same bf16-rounded operands."""
+    from pointnet_refine_b200.train_ops import KVGradShare, cross_attention_train, kv_proj
+    g = torch.Generator(device=dev).manual_seed(5)
+    B, N, L, d = 2, 333, 6, 256
+    xk, xv = (torch.randn(B, N, d, device=dev, generator=g).requires_grad_() for _ in range(2))
+    wk, wv = ((torch.randn(L * d, d, device=dev, generator=g) / 16).requires_grad_() for _ in range(2))
+    bk, bv = ((torch.randn(L * d, device=dev, generator=g) / 4).requires_grad_() for _ in range(2))
+    q = torch.randn(B, 32, d, device=dev, generator=g)
+    r = torch.randn(B, 32, d, device=dev, generator=g)
+    share = KVGradShare()
+    for t in share.buffers(B, N, L, dev):
+        t.fill_(float("nan"))
+    k_l = kv_proj(xk, wk, bk, L, 8, share, key=True)
+    v_l = kv_proj(xv, wv, bv, L, 8, share, key=False)
+    (cross_attention_train(q, k_l[0], v_l[0], 0.0, share, 0) * r).sum().backward()
+    rd = lambda t: t.detach().bfloat16().double().requires_grad_()
+    xkd, xvd, wkd, wvd = rd(xk), rd(xv), rd(wk), rd(wv)
+    bkd, bvd = bk.detach().double(), bv.detach().double().requires_grad_()
+    heads0 = lambda t: t.view(B, N, L, 8, 32)[:, :, 0].transpose(1, 2)            # layer 0, (B, 8, N, 32)
+    kd, vd = heads0(xkd @ wkd.t() + bkd), heads0(xvd @ wvd.t() + bvd)
+    qd = q.double().view(B, 32, 8, 32).transpose(1, 2)
+    ref = (torch.softmax(qd @ kd.transpose(2, 3) / 32 ** 0.5, dim=-1) @ vd).transpose(1, 2).reshape(B, 32, d)
+    (ref * r.double()).sum().backward()
+    rel = lambda a, b: float((a.detach().double() - b).norm() / b.norm())
+    for w, wref in ((wk, wkd), (wv, wvd)):
+        assert torch.equal(w.grad[d:], torch.zeros_like(w.grad[d:]))
+        assert rel(w.grad[:d], wref.grad[:d]) <= 2e-2
+    assert torch.equal(bk.grad, torch.zeros_like(bk.grad))      # the K bias gradient is identically zero in every layer
+    assert torch.equal(bv.grad[d:], torch.zeros_like(bv.grad[d:]))
+    assert rel(bv.grad[:d], bvd.grad[:d]) <= 2e-2
+    assert rel(xk.grad, xkd.grad) <= 2e-2 and rel(xv.grad, xvd.grad) <= 2e-2
+
+
 def test_flat_adam_and_fused_l1_match_torch(dev):
-    """FlatAdam (one lrn_adam_step launch over a flat buffer) and deep_supervision_l1 against torch.optim.Adam and the
+    """FlatAdam (one lrn_adam_step_capturable call over a flat buffer) and deep_supervision_l1 against torch.optim.Adam and the
     reference's loss loop (train.py:40,63-72) over several steps of the same small model."""
     import copy
     import pointnet_refine_b200 as prb
@@ -563,24 +636,20 @@ def test_train_attention_seed_state_word(dev):
     assert rel(outs[2][0], ref) > 0.1                                # another word -> another mask
 
 
-def test_flat_adam_capturable_matches_host_step(dev):
-    """FlatAdam(capturable=True): the step count and bias corrections live on the device (lrn_adam_step_capturable);
-    same trajectory as the host-counted step, and the count round-trips through state_dict."""
+def test_flat_adam_step_count_on_device(dev):
+    """FlatAdam keeps the step count and computes the bias corrections on the device (lrn_adam_step_capturable): the
+    count advances once per step and round-trips through state_dict."""
     from pointnet_refine_b200.optim import FlatAdam
     torch.manual_seed(0)
     net_a = torch.nn.Linear(96, 64).to(dev)
-    net_b = copy.deepcopy(net_a)
-    opt_a, opt_b = FlatAdam(net_a.parameters(), lr=1e-3, capturable=True), FlatAdam(net_b.parameters(), lr=1e-3)
+    opt_a = FlatAdam(net_a.parameters(), lr=1e-3)
     x = torch.randn(16, 96, device=dev)
     for _ in range(7):
-        for net, opt in ((net_a, opt_a), (net_b, opt_b)):
-            opt.zero_grad()
-            net(x).square().mean().backward()
-            opt.step()
-    for pa, pb in zip(net_a.parameters(), net_b.parameters()):
-        assert float((pa - pb).detach().abs().max()) <= 1e-6
+        opt_a.zero_grad()
+        net_a(x).square().mean().backward()
+        opt_a.step()
     assert opt_a.steps_taken == 7 and opt_a.state_dict()["flat_adam"]["step"] == 7
-    opt_c = FlatAdam(copy.deepcopy(net_a).parameters(), lr=1e-3, capturable=True)
+    opt_c = FlatAdam(copy.deepcopy(net_a).parameters(), lr=1e-3)
     opt_c.load_state_dict(opt_a.state_dict())
     assert opt_c.steps_taken == 7
 

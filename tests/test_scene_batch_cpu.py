@@ -13,8 +13,8 @@ from pointnet_refine_b200 import _lib, data, scene
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_scene_entry_points_abi_v4_many_scene_only():
-    """ABI version 4: the many-scene entry points are the only scene builders; the per-scene ones are gone everywhere."""
+def test_scene_entry_points_abi_v5_many_scene_only():
+    """ABI version 5 (since 4): the many-scene entry points are the only scene builders; the per-scene ones are gone everywhere."""
     header = open(os.path.join(ROOT, "include", "lrn_b200.h")).read()
     declared = set(re.findall(r"^(?:int|size_t|const char\*) (lrn_[a-z0-9_]+)\(", header, re.M))
     many = {"lrn_scenes_segments", "lrn_scenes_workspace_bytes"}
@@ -24,7 +24,7 @@ def test_scene_entry_points_abi_v4_many_scene_only():
         assert hasattr(lib, name), name
     for name in ("lrn_scene_segments", "lrn_scene_workspace_bytes"):
         assert name not in header and name not in _lib.SIGNATURES and not hasattr(lib, name), name
-    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 4
+    assert lib.lrn_abi_version() == _lib.ABI_VERSION == 5
 
 
 def test_scenes_workspace_bytes_grow_with_lines_scenes_and_capacity():
