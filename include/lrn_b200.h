@@ -39,7 +39,10 @@ extern "C" {
  *    of lrn_scenes_segments, which gives the same bits.
  * 5: the head gather of attention gradients and the host-counted lrn_adam_step removed: the train attention backward
  *    writes dK / dV in place in the K / V projections' layout, and every Adam step keeps its step count on the device
- *    (lrn_adam_step_capturable). */
+ *    (lrn_adam_step_capturable).  Later, without a version change, the output flag LRN_OUT_FUSED_BF16 of
+ *    lrn_encoder_forward: an addition only; every flag combination that existed keeps its workspace size, its launches
+ *    and its results.  A library built before it ignores the bit, so a call that requests nothing else fails there
+ *    with LRN_ERR_BAD_ARG (no output requested). */
 #define LRN_ABI_VERSION 5
 
 typedef struct CUstream_st* lrn_stream_t; /* == cudaStream_t */
@@ -71,6 +74,11 @@ enum lrn_encoder_flags {
   LRN_OUT_MEMORY = 8, /* memory fp32 (B,N,256) = context_proj(fused^T) src/model.py:194   */
   LRN_OUT_MEMORY_BF16 = 16, /* with LRN_OUT_MEMORY (bf16 tier): memory is written as bf16 into rows of pitch 512
                                elements, columns [0,256); columns [256,512) are left to the caller (lrn_pos_hidden) */
+  LRN_OUT_FUSED_BF16 = 32,  /* bf16 tier only, not with LRN_OUT_FUSED (both write through `fused`): fused as bf16 in
+                               point-major order (B*N, 1024), the layout lrn_encoder_train_forward writes with
+                               fused_point_major = 1 and context_proj consumes; each element is the bf16 rounding (to
+                               nearest even) of the fp32 value LRN_OUT_FUSED writes.  On its own it launches no
+                               context_proj GEMM, reads no proj_w and needs no workspace beyond the operand rows. */
 };
 
 /* Raw fp32 parameters of the reference module, exactly as they sit in its state_dict
@@ -125,6 +133,7 @@ int lrn_encoder_fold(const lrn_encoder_params* params, int precision, void* pack
  *                  called with at src/model.py:192-193 is a transpose of this buffer)
  *   global_feat  : (B, 2048) fp32               required iff LRN_OUT_POOL or LRN_OUT_ARGMAX
  *   fused        : (B, 1024, N) fp32            required iff LRN_OUT_FUSED
+ *                  ((B*N, 1024) bf16, 16-byte aligned, with LRN_OUT_FUSED_BF16; rows from B*N on are not written)
  *   argmax       : (B, 1024) int64              required iff LRN_OUT_ARGMAX
  *   memory       : (B, N, 256) fp32             required iff LRN_OUT_MEMORY  ((B, N, 512) bf16 with LRN_OUT_MEMORY_BF16)
  *   chunk_rows   : points processed per wave (0 = library default); a tuning knob only.

@@ -19,7 +19,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "lrn_b200.h")
 ABI_VERSION = 5      # LRN_ABI_VERSION
 LRN_OK = 0
 PREC_BF16, PREC_TF32, PREC_FP32X3 = 0, 1, 2
-OUT_POOL, OUT_ARGMAX, OUT_FUSED, OUT_MEMORY, OUT_MEMORY_BF16 = 1, 2, 4, 8, 16
+OUT_POOL, OUT_ARGMAX, OUT_FUSED, OUT_MEMORY, OUT_MEMORY_BF16, OUT_FUSED_BF16 = 1, 2, 4, 8, 16, 32
 PRECISIONS = {"bf16": PREC_BF16, "tf32": PREC_TF32, "fp32x3": PREC_FP32X3}
 STAGES = ["embed", "conv2", "conv3", "conv4", "conv5", "fusion", "proj"]
 

@@ -451,17 +451,21 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
   if (bad_precision(precision)) return fail(LRN_ERR_BAD_ARG, "bad precision %d", precision);
   if ((flags & LRN_OUT_MEMORY_BF16) && (precision != LRN_PREC_BF16 || !(flags & LRN_OUT_MEMORY)))
     return fail(LRN_ERR_BAD_ARG, "LRN_OUT_MEMORY_BF16 needs LRN_OUT_MEMORY and the bf16 tier");
+  if ((flags & LRN_OUT_FUSED_BF16) && (precision != LRN_PREC_BF16 || (flags & LRN_OUT_FUSED)))
+    return fail(LRN_ERR_BAD_ARG, "LRN_OUT_FUSED_BF16 needs the bf16 tier and excludes LRN_OUT_FUSED");
   if (B <= 0 || N <= 0) return fail(LRN_ERR_BAD_SHAPE, "empty input B=%lld N=%lld", (long long)B, (long long)N);
   if (B * N >= (int64_t(1) << 31) - 128) return fail(LRN_ERR_BAD_SHAPE, "B*N = %lld must be < 2^31", (long long)(B * N));
   if (!packed || !context || !workspace) return fail(LRN_ERR_BAD_ARG, "null packed/context/workspace");
-  if (!(flags & (LRN_OUT_POOL | LRN_OUT_ARGMAX | LRN_OUT_FUSED | LRN_OUT_MEMORY)))
+  if (!(flags & (LRN_OUT_POOL | LRN_OUT_ARGMAX | LRN_OUT_FUSED | LRN_OUT_MEMORY | LRN_OUT_FUSED_BF16)))
     return fail(LRN_ERR_BAD_ARG, "no output requested");
   if ((flags & (LRN_OUT_POOL | LRN_OUT_ARGMAX)) && !global_feat) return fail(LRN_ERR_BAD_ARG, "global_feat is null");
   if ((flags & LRN_OUT_ARGMAX) && !argmax) return fail(LRN_ERR_BAD_ARG, "argmax is null");
-  if ((flags & LRN_OUT_FUSED) && !fused) return fail(LRN_ERR_BAD_ARG, "fused is null");
+  if ((flags & (LRN_OUT_FUSED | LRN_OUT_FUSED_BF16)) && !fused) return fail(LRN_ERR_BAD_ARG, "fused is null");
   if ((flags & LRN_OUT_MEMORY) && !memory) return fail(LRN_ERR_BAD_ARG, "memory is null");
   if (misaligned(16, context, memory, global_feat) || misaligned(1024, workspace, packed))
     return fail(LRN_ERR_MISALIGNED, "context/memory/global_feat need 16-byte, packed/workspace 1024-byte alignment");
+  if ((flags & LRN_OUT_FUSED_BF16) && misaligned(16, fused))
+    return fail(LRN_ERR_MISALIGNED, "LRN_OUT_FUSED_BF16: fused needs 16-byte alignment");
   LRN_DEVICE(dev);
 
   const bool tf32 = precision != LRN_PREC_BF16;      // fp32 operands on the kind::tf32 tensor-core path
@@ -475,7 +479,7 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
   const uint8_t* pk = static_cast<const uint8_t*>(packed);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   void* cat = ws + W.cat;
-  void* fused_pm = ws + W.fused_pm;
+  const bool fused_bf16 = flags & LRN_OUT_FUSED_BF16;
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + W.keys);
   const int64_t P = B * N;
 
@@ -506,6 +510,9 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
 
   for (int64_t r0 = 0; r0 < P; r0 += W.chunk) {
     const int64_t rows = std::min<int64_t>(W.chunk, P - r0);
+    // point-major fused rows of this wave: the caller's (B*N, 1024) bf16 buffer at row r0 (LRN_OUT_FUSED_BF16; the fusion
+    // kernel writes only rows < p.M = rows of it), else the workspace block the projection reads
+    void* fused_pm = fused_bf16 ? static_cast<void*>(reinterpret_cast<uint16_t*>(fused) + r0 * 1024) : ws + W.fused_pm;
     auto m_tiles_of = [&](const GemmPlan& g) { return int((rows + g.m_rows - 1) / g.m_rows); };
     CUtensorMap ta, tpm;
     LRN_TRY(make_tmap(&ta, precision, cat, rows, kCat * wm, kCat * wm, BM));
@@ -547,6 +554,8 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
       // A second operand buffer would not let chain(w) start sooner: its CTA needs the SM that fusion(w - 1)'s CTA holds.
       // The first chain kernel of a call is an ordinary launch: it follows the memsets and whatever the caller enqueued.
       // (With LRN_OUT_MEMORY the projection, an ordinary launch, sits between fusion(w - 1) and chain(w).)
+      // With LRN_OUT_FUSED_BF16 fusion(w) also stores into the caller's `fused` rows [r0, r0 + rows), after the wait like
+      // every output store; no kernel of the call reads them (with LRN_OUT_MEMORY the projection does, an ordinary launch).
       LRN_TRY(launch_programmatic(r0 > 0, chain_pair_kernel, grid, kPairThreads, ChainSmem::kDynamic, stream, tw_chain[0],
                                   tw_chain[1], tw_chain[2], tw_chain[3], ta, cp));
     } else {  // layer 1 (+ gate layer 1): raw points -> operand columns
@@ -604,7 +613,7 @@ int lrn_encoder_forward(const void* packed, int precision, const float* context,
       p.npts = int(N);
       p.inv_npts = 1.0f / float(N);
       p.flags = ((flags & LRN_OUT_ARGMAX) ? (FUSE_ARGMAX | FUSE_POOL) : (flags & LRN_OUT_POOL) ? FUSE_POOL : 0) |
-                ((flags & LRN_OUT_FUSED) ? FUSE_STORE_CN : 0) | ((flags & LRN_OUT_MEMORY) ? FUSE_STORE_PM : 0);
+                ((flags & LRN_OUT_FUSED) ? FUSE_STORE_CN : 0) | ((flags & (LRN_OUT_MEMORY | LRN_OUT_FUSED_BF16)) ? FUSE_STORE_PM : 0);
       p.global_feat = global_feat;
       p.pool_key = keys;
       p.fused_cn = fused;

@@ -61,6 +61,9 @@ class GraphedTrainStep:
       word to their seed (train_ops.DropoutSeedState), advanced inside the graph; torch's own dropout kernels take their
       Philox offsets from the graph-registered generator;
     * no host synchronisation anywhere in the step (there is none: the loss stays on the device).
+    A frozen context encoder (`context_encoder.eval().requires_grad_(False)` with the native-training opt-in, FlatAdam over
+    the trainable parameters only) runs as its eval forward inside the graph; the wrapper keeps the fold blob and scratch
+    buffer that forward reads alive.
     Launch arguments are frozen at capture: the optimizer's lr / betas / eps / weight decay, the dropout rates and the batch
     shape are the ones in force when the step was built (the reference trains at a constant lr, train.py:21,40); build a
     new GraphedTrainStep to change them.
@@ -76,7 +79,7 @@ class GraphedTrainStep:
     last batch of an epoch) runs the same step eagerly (`eager`)."""
 
     def __init__(self, net, optimizer, context, noisy_line, target, loss_fn=None, warmup: int = 2):
-        from . import train_ops
+        from . import ops, train_ops
         from .optim import FlatAdam, deep_supervision_l1
         if not isinstance(optimizer, FlatAdam):
             raise TypeError("GraphedTrainStep needs FlatAdam: the step count must live on the device")
@@ -99,7 +102,8 @@ class GraphedTrainStep:
                 self._step_body()
             with torch.no_grad():
                 for t, s in zip(keep, saved):
-                    t.copy_(s)
+                    if not torch.equal(t, s):   # what the step left alone (a frozen encoder's BatchNorm statistics) keeps
+                        t.copy_(s)              # its version, so its prepared weights (encoder fold) are not rebuilt in the capture
         torch.cuda.current_stream(dev).wait_stream(self._side)
         # ---- capture
         self.graph = torch.cuda.CUDAGraph()
@@ -119,6 +123,9 @@ class GraphedTrainStep:
         finally:
             train_ops.DropoutSeedState.word = None
         self.loss, self.pred = loss.detach(), pred.detach()
+        # what the captured kernels point at outside the graph's memory pool (a frozen encoder's eval forward: its fold blob
+        # and scratch buffer), kept alive whatever later eager calls or invalidate() do to the caches
+        self._keep = (ops.workspaces_of(dev), dict(model._prepared))
         self.replays = 0
 
     def close(self):

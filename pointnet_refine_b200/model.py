@@ -15,7 +15,9 @@ What runs where
     within tolerance for inference but changes gradients -- the caller decides).  `native_training = True` /
     LRN_NATIVE_TRAIN=1 (bf16 tier) switches the encoder, and with M = 32 also context_proj and the decoder's linears and
     attention, to the sm_100a train path (train_ops.py: batch-stat BN forward and a hand-written backward on the tcgen05
-    GEMMs).
+    GEMMs).  With the opt-in, a frozen encoder (transfer learning: `context_encoder.eval().requires_grad_(False)`, see
+    train_ops.native_frozen_encoder) at M = 32 runs as the eval encoder, whose point-major bf16 `fused` feeds the same
+    native train decoder; trainable encoder weights under frozen BatchNorm, and M != 32, stay on the stock ops.
   * CPU tensors: not supported -- there is no CPU path in the product (the oracle lives in oracle/).
 """
 from __future__ import annotations
@@ -94,20 +96,24 @@ class MultiScalePointNetEncoder(nn.Module):
         self._prepared = {}                     # prepared weights (_prepared); never in the state_dict
         self._proj = None                       # optional nn.Linear(1024,256) folded alongside (set by LineRefineNet)
 
-    def folded(self) -> ops.FoldedEncoder:
+    def folded(self, proj: bool = True) -> ops.FoldedEncoder:
         """BN-folded operand blob for the current parameters; re-folded whenever a parameter or
-        running statistic changes (optimizer step, load_state_dict, .to())."""
+        running statistic changes (optimizer step, load_state_dict, .to()).  proj=False: the blob without context_proj,
+        cached apart and fingerprinted on the encoder's own parameters and buffers only, so that training context_proj
+        (frozen-encoder steps) does not re-fold the encoder every step."""
+        name = "fold" if proj else "fold_encoder"
+        proj = proj and self._proj is not None
         ts = list(self.parameters()) + list(self.buffers())
-        if self._proj is not None:
+        if proj:
             ts += list(self._proj[0].parameters())
 
         def fold():
             tensors = {k: v for k, v in self.state_dict().items() if v.is_floating_point()}
-            if self._proj is not None:
+            if proj:
                 tensors["context_proj.weight"] = self._proj[0].weight
                 tensors["context_proj.bias"] = self._proj[0].bias
             return ops.FoldedEncoder(tensors, self.precision, bn_eps=self.bn1.eps)
-        return _prepared(self._prepared, "fold", ts, fold, key=(self.precision,))
+        return _prepared(self._prepared, name, ts, fold, key=(self.precision,))
 
     def invalidate(self):
         """Drop the prepared weights.  They are keyed on (data_ptr, _version) of every parameter and buffer, which
@@ -477,9 +483,16 @@ class LineRefineNet(nn.Module):
             raise ValueError(f"expected context (B,N,4) and noisy_line (B,M,3), got {tuple(context.shape)} and {tuple(noisy_line.shape)}")
         if not _use_native(self, context, noisy_line):
             enc = self.context_encoder
-            if self.training and noisy_line.shape[1] == 32 and train_ops.native_train_supported(enc):
-                _, fused_pm = train_ops.encoder_train_forward(enc, context, point_major=True)
-                return self._refine_fast_train(context, noisy_line, fused_pm)
+            if self.training and noisy_line.shape[1] == 32:
+                if train_ops.native_train_supported(enc):
+                    _, fused_pm = train_ops.encoder_train_forward(enc, context, point_major=True)
+                    return self._refine_fast_train(context, noisy_line, fused_pm)
+                if train_ops.native_frozen_encoder(enc):
+                    # frozen encoder (transfer learning): its eval function, point-major bf16 `fused` straight from the
+                    # fusion kernel, no autograd node, no running-statistic update; the blob leaves out context_proj, which trains
+                    fused_pm = ops.encoder_forward(enc.folded(proj=False), context, pool=False, fused_bf16=True,
+                                                   chunk_rows=enc.chunk_rows)["fused_pm"]
+                    return self._refine_fast_train(context, noisy_line, fused_pm)
             _, fused = enc(context.transpose(2, 1))   # with native training on (M != 32): the channel-major native encoder
             memory = self.context_proj(fused.transpose(2, 1))
             return self._refine(context, noisy_line, memory, native_heads=False)

@@ -7,7 +7,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import OUT_ARGMAX, OUT_FUSED, OUT_MEMORY, OUT_MEMORY_BF16, OUT_POOL, PRECISIONS, lib
+from ._lib import OUT_ARGMAX, OUT_FUSED, OUT_FUSED_BF16, OUT_MEMORY, OUT_MEMORY_BF16, OUT_POOL, PRECISIONS, lib
 
 DEFAULT_CHUNK_ROWS = 148 * 128 * 16   # keep in sync with kDefaultChunkRows (csrc/lrn_abi.cu)
 
@@ -93,11 +93,13 @@ def workspaces_of(device) -> list:
 
 
 def encoder_forward(folded: FoldedEncoder, context: torch.Tensor, *, pool=True, argmax=False, fused=False,
-                    memory=False, memory_bf16=False, chunk_rows: int = 0):
+                    memory=False, memory_bf16=False, fused_bf16=False, chunk_rows: int = 0):
     """Run the fused encoder on context (B, N, 4) float32 CUDA.  Returns a dict with the requested
     outputs: global_feat (B,2048), argmax (B,1024) int64, fused (B,1024,N), memory (B,N,256).
     memory_bf16 (bf16 tier): memory is returned as a (B,N,512) bfloat16 buffer whose columns [0,256) hold it and
-    whose columns [256,512) are uninitialised (filled by pos_hidden for the decoder's context side)."""
+    whose columns [256,512) are uninitialised (filled by pos_hidden for the decoder's context side).
+    fused_bf16 (bf16 tier, not with fused): fused_pm (B,N,1024) bfloat16, point-major, the bf16 rounding of `fused`:
+    the layout context_proj consumes (LRN_OUT_FUSED_BF16)."""
     if context.dim() != 3 or context.shape[-1] != 4:
         raise ValueError(f"context must be (B, N, 4), got {tuple(context.shape)}")
     context = _f32c(context)
@@ -106,7 +108,8 @@ def encoder_forward(folded: FoldedEncoder, context: torch.Tensor, *, pool=True, 
         raise ValueError("empty context (the reference's torch.max over an empty dimension raises too)")
     dev = context.device
     flags = (OUT_POOL if pool else 0) | (OUT_ARGMAX if argmax else 0) | (OUT_FUSED if fused else 0) | \
-            (OUT_MEMORY if memory else 0) | (OUT_MEMORY_BF16 if memory and memory_bf16 else 0)
+            (OUT_MEMORY if memory else 0) | (OUT_MEMORY_BF16 if memory and memory_bf16 else 0) | \
+            (OUT_FUSED_BF16 if fused_bf16 else 0)
     if memory and not folded.has_proj:
         raise ValueError("memory output needs context_proj weights in the folded blob")
     out = {}
@@ -117,6 +120,8 @@ def encoder_forward(folded: FoldedEncoder, context: torch.Tensor, *, pool=True, 
         out["argmax"] = am = torch.empty(B, 1024, dtype=torch.int64, device=dev)
     if fused:
         out["fused"] = fz = torch.empty(B, 1024, N, dtype=torch.float32, device=dev)
+    if fused_bf16:
+        out["fused_pm"] = fz = torch.empty(B, N, 1024, dtype=torch.bfloat16, device=dev)
     if memory:
         out["memory"] = mem = (torch.empty(B, N, 512, dtype=torch.bfloat16, device=dev) if memory_bf16 else
                                torch.empty(B, N, 256, dtype=torch.float32, device=dev))

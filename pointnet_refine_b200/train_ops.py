@@ -111,6 +111,21 @@ def native_train_supported(module) -> bool:
                and b.momentum == bns[0].momentum for b in bns)
 
 
+def native_frozen_encoder(module) -> bool:
+    """Whether the encoder `module` is frozen in a way that lets a train step run it as its eval function on the native
+    path (transfer learning: `module.eval().requires_grad_(False)` with the `native_training` opt-in, bf16 tier): every
+    BatchNorm in eval mode with running statistics and one common eps, and no parameter requiring grad.  Then the encoder
+    is exactly its eval-mode forward and autograd needs nothing from it; LineRefineNet feeds the native train decoder from
+    the eval encoder's point-major bf16 `fused`.  Trainable weights under frozen BatchNorm stay on the stock ops."""
+    if not (module.native_training and module.precision == "bf16"):
+        return False
+    if any(p.requires_grad for p in module.parameters()):
+        return False
+    bns = _encoder_bns(module)
+    return all(not b.training and b.track_running_stats and b.running_mean is not None and b.affine and b.eps == bns[0].eps
+               for b in bns)
+
+
 def encoder_train_forward(module, context, point_major=False):
     """module: MultiScalePointNetEncoder in train mode; context (B,N,4).  Returns (global_feat, fused) with
     autograd through the native backward; updates running statistics / num_batches_tracked like PyTorch.
